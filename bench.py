@@ -1,13 +1,14 @@
 #!/usr/bin/env python
 """Benchmark of the GNN branching-score hot path: subdomains scored per second on a B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload base|wide|deep] [--domains B_per_gpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload base|wide|deep] [--domains B_per_gpu] [--dump-outputs DIR]
     python bench.py --impl reference ...      # the reference algorithm on the host CPU (oracle port)
 
 One step = one pass of the hot path over one frontier of synthetic subdomains (SURVEY §8d generator):
 at N = 1 the workload is BASELINE.json configs[1], cifar_base_kw x 1 024 subdomains; at N > 1 every rank scores
 the same number of subdomains (weak scaling, no data-path collective) and the per-subdomain winners are
-all-gathered with NCCL inside the timed region.  Prints ONE JSON line (rank 0).
+all-gathered with NCCL inside the timed region.  Prints ONE JSON line (rank 0).  The frontiers are seeded, so two runs
+with the same arguments score the same inputs: --dump-outputs lets two builds be compared winner for winner.
 """
 import argparse
 import json
@@ -48,7 +49,14 @@ def parse():
     ap.add_argument('--no-step', action='store_true', help='skip the device-resident branch-and-bound step (pick, bound, score, add)')
     ap.add_argument('--no-secondary', action='store_true', help='skip the wide / deep x 4096 secondary objects of the default line')
     ap.add_argument('--opt', action='append', default=[], help='library option key=value (e.g. fuse=0, prop_share=40)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the winners of the last timed step (what the caller receives) as DIR/<name>.npy')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
+    return args
 
 
 def load_problem(workload):
@@ -164,12 +172,14 @@ def run_timed(step, local_step, K, barrier, record0, record1, clock_samples, syn
     """The timed region: barrier, K steps between the two event records, barrier.  `step` may contain collectives (every
     rank calls it exactly K times); afterwards the identical load is kept running with `local_step` — rank-LOCAL work only,
     because every rank runs a different number of these — until the clock sampler has `min_samples` samples under load
-    (a K x 5 ms region can end before NVML has answered a handful of times)."""
+    (a K x 5 ms region can end before NVML has answered a handful of times).  What the last timed step returned is kept in
+    `run_timed.last`."""
     barrier()
     record0()
     for i in range(K):
-        step(i)
+        out = step(i)
     record1()
+    run_timed.last = out
     barrier()
     extra = 0
     while clock_samples() < min_samples and extra < max_extra:
@@ -183,6 +193,7 @@ def run_timed(step, local_step, K, barrier, record0, record1, clock_samples, syn
 
 
 run_timed.extra = 0
+run_timed.last = None
 
 
 def _run_ref_runner(device, workload, weights, batches, reps, warmup=1, timeout=900):
@@ -381,6 +392,7 @@ def measure_device(scorer, fronts, B, K, W, world, dev, local, gather):
         run_timed(step, lambda i: score(fronts[i % len(fronts)]), K, barrier, ev0.record, ev1.record, clk.count, torch.cuda.synchronize)
         launches = (scorer.launches - launches0) * K // (K + run_timed.extra)      # every step issues the same launches
     scorer.check()
+    outputs = tuple(t.clone() for t in run_timed.last)          # the gather writes a persistent buffer the passes below reuse
     ms = ev0.elapsed_time(ev1)
     # per-kernel-class durations: a second pass of K identical steps with CUDA events around every launch (on the launching
     # stream).  The events serialise consecutive launches (no programmatic overlap of a kernel's prologue with its
@@ -396,7 +408,29 @@ def measure_device(scorer, fronts, B, K, W, world, dev, local, gather):
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
-    return {'value': B * world * K / (ms * 1e-3), 'ms': ms, 'launches': launches, 'prof': prof, 'clocks': clk.summary()}
+    return {'value': B * world * K / (ms * 1e-3), 'ms': ms, 'launches': launches, 'prof': prof, 'clocks': clk.summary(),
+            'outputs': outputs}
+
+
+DUMP_LIMIT = 64 * 10 ** 6      # bytes written by --dump-outputs
+
+
+def dump_outputs(out_dir, best, idx):
+    """The winners of the last timed step as DIR/best_score.npy (float32) and DIR/best_index.npy (float64: flat index of the
+    chosen ReLU over all hidden layers, -1 where a subdomain has no candidate).  Past DUMP_LIMIT bytes, a fixed seeded sample
+    of subdomains is written, their positions in DIR/sample_rows.npy."""
+    import numpy as np
+    best, idx = best.cpu().numpy().astype(np.float32), idx.cpu().numpy().astype(np.float64)
+    n, headers = best.shape[0], 4096          # 4096: room for the .npy headers
+    arrays = {'best_score': best, 'best_index': idx}
+    # 12 bytes per subdomain: a 65 536-subdomain frontier writes 0.8 MB, so only very large --domains x --gpus runs sample;
+    # a sampled row costs 20 bytes (its position in sample_rows.npy included)
+    if n * (4 + 8) + headers > DUMP_LIMIT:
+        rows = np.sort(np.random.default_rng(0).choice(n, (DUMP_LIMIT - headers) // (4 + 8 + 8), replace=False))
+        arrays = {'best_score': best[rows], 'best_index': idx[rows], 'sample_rows': rows.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def measure_e2e(model, host_fronts, B, K, W, world, dev, gather):
@@ -629,6 +663,8 @@ def main():
 
     m = measure_device(scorer, fronts, B, K, W, world, dev, local, gather_winner_records)
     value, ms, launches, clocks = m['value'], m['ms'], m['launches'], m['clocks']
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *m['outputs'])
 
     # ---- end to end through the public API with pinned HOST buffers (copies inside the timed region) ----
     e2e = None
