@@ -32,7 +32,6 @@ struct gnnb_ctx {
     int chunk = 0;
     int snapshot = 0;
     int fuse = 1;                   // propagation + node update of a layer in one launch, nb handed over in tensor memory (k_tc_fused); 0 = two launches
-    int gather_prefetch = 0;        // stand-alone propagation kernel variants that fetch the gather indices one chunk ahead (bit-identical, off)
     // GNN parameters
     bool have_gnn = false;
     float* d_gnn = nullptr;
@@ -354,7 +353,7 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
                          ctx->mu[k], nullptr, M(k), 0, 0, rows, ctx->d_nan, ctx->snapshot ? ctx->nb : nullptr, false, st, lc);
             } else {
                 ProfScope ps(ctx, GNNB_K_PROP_FWD, nodes, st);
-                if (tc) prop_tc_run(ctx->plan_fwd[k - 1], ctx->mu[k - 1], ctx->nb, Bc, st, lc, ctx->gather_prefetch);
+                if (tc) prop_tc_run(ctx->plan_fwd[k - 1], ctx->mu[k - 1], ctx->nb, Bc, st, lc);
                 else prop_forward(ctx->layers[k - 1], ctx->mu[k - 1], ctx->nb, Bc, st, lc);
             }
             TRY(snap_img(ctx, name("t%d_fwd_nb%d", t, k), ctx->nb, k, Bc, true, st));
@@ -386,7 +385,7 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
                 ProfScope ps(ctx, GNNB_K_PROP_BWD, nodes, st);
                 if (k == L && tc) prop_tc_property_backward(in.wp, ctx->mu[L + 1], ctx->nb, ctx->n[L], ctx->rowmap[L].nslots, Bc, st, lc);
                 else if (k == L) prop_property_backward(in.wp, ctx->mu[L + 1], ctx->nb, ctx->n[L], Bc, st, lc);
-                else if (tc) prop_tc_run(ctx->plan_bwd[k], ctx->mu[k + 1], ctx->nb, Bc, st, lc, ctx->gather_prefetch);
+                else if (tc) prop_tc_run(ctx->plan_bwd[k], ctx->mu[k + 1], ctx->nb, Bc, st, lc);
                 else prop_backward(ctx->layers[k], ctx->mu[k + 1], ctx->nb, Bc, true, st, lc);
             }
             TRY(snap_img(ctx, name("t%d_bwd_nb%d", t, k), ctx->nb, k, Bc, true, st));
@@ -406,7 +405,7 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
         } else if (!last) {
             {
                 ProfScope ps(ctx, GNNB_K_PROP_BWD, (int64_t)Bc * ctx->n[0], st);
-                if (tc) prop_tc_run(ctx->plan_bwd[0], ctx->mu[1], ctx->nb, Bc, st, lc, ctx->gather_prefetch);
+                if (tc) prop_tc_run(ctx->plan_bwd[0], ctx->mu[1], ctx->nb, Bc, st, lc);
                 else prop_backward(ctx->layers[0], ctx->mu[1], ctx->nb, Bc, false, st, lc);
             }
             {
@@ -795,11 +794,6 @@ int gnnb_set_option(gnnb_ctx* ctx, const char* key, int64_t value) {
         ctx->chunk = (int)value;
     } else if (k == "fuse") {
         ctx->fuse = value ? 1 : 0;
-    } else if (k == "gather_prefetch") {
-        if (value < 0 || value > 2) return fail(ctx, GNNB_ERR_INVALID, "gather_prefetch is 0, 1 or 2");
-        ctx->gather_prefetch = (int)value;
-    } else if (k.rfind("fused_", 0) == 0) {       // experiment knobs of k_tc_fused (process-wide)
-        tc_fused_tune(k.c_str() + 6, (int)value);
     } else if (k == "snapshot") {
         ctx->snapshot = value ? 1 : 0;
     } else if (k == "profile") {
@@ -817,7 +811,6 @@ int64_t gnnb_get_option(gnnb_ctx* ctx, const char* key) {
     if (k == "chunk") return ctx->chunk;
     if (k == "snapshot") return ctx->snapshot;
     if (k == "fuse") return ctx->fuse;
-    if (k == "gather_prefetch") return ctx->gather_prefetch;
     if (k == "profile") return ctx->profile;
     if (k == "n_hidden") return ctx->n_hidden;
     if (k == "workspace_domains") return ctx->ws_cap;

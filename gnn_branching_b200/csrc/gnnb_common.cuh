@@ -126,7 +126,6 @@ void tc_update(const GnnParams& g, bool backward, const float* lb, const float* 
 // to the update chain through tensor memory and are never written (k_tc_fused); nb_dbg: the nb tile images for snapshots, or null;
 // input_layer: the chain is the input-layer update (lb / ub = input bounds; backward, relax, amb_base, scores unused)
 struct PropPlan;
-void tc_fused_tune(const char* key, int value);
 void tc_fused(const GnnParams& g, const PropPlan* plan, const float* mu_in, bool backward, const float* lb, const float* ub,
               const float* relax, const int32_t* amb_base, float* mu_out, float* scores, RowMap map, int64_t score_stride, int64_t score_off,
               int64_t rows, unsigned long long* nan_count, float* nb_dbg, bool input_layer, cudaStream_t st, int64_t* launches);
@@ -178,8 +177,7 @@ PropPlan* prop_plan_build(const LayerDev& L, const float* host_weight, bool back
                           const LayerTiling& in);
 void prop_plan_free(PropPlan* p);
 double prop_plan_density(const PropPlan* p);
-void prop_tc_run(const PropPlan* plan, const float* mu_in, float* nb_img, int Bc, cudaStream_t st, int64_t* launches,
-                 int gather_prefetch = 0);
+void prop_tc_run(const PropPlan* plan, const float* mu_in, float* nb_img, int Bc, cudaStream_t st, int64_t* launches);
 void prop_tc_property_backward(const float* wp, const float* mu_out, float* nb_img, int nL, int nslots, int Bc, cudaStream_t st, int64_t* launches);
 
 // BaBSR / KW heuristic (gnnb_babsr.cu); every pointer is a device pointer; returns -1 when the network does not fit

@@ -1,19 +1,14 @@
-// Device side of the stand-alone tensor-core propagation (gather-GEMM, gnnb_prop_tc.cu) and the plan format it shares with
-// the fused propagation + node-update kernel (gnnb_tc.cu, k_tc_fused).
+// The block plan of one edge set (gnnb_prop_tc.cu builds it) as the tensor-core propagation kernels read it: the stand-alone
+// gather-GEMM k_tc_prop (gnnb_prop_tc.cu) and the fused propagation + node-update kernel k_tc_fused (gnnb_tc.cu).
 #pragma once
 
-#include "gnnb_umma.cuh"
+#include "gnnb_common.cuh"
 
 namespace gnnb {
 
-using namespace tcx;
-
+// A tile's K dimension (the sorted input slots its 128 output rows touch) is cut into K steps of 16 rows; a tile has at
+// least one step.  The steps of a tile are contiguous in ks_rows and ks_w.
 struct PropPlanDev {
-    const int32_t* in_rows;       // [nchunks][64] input slot of each K row, -1 = zero row
-    const uint16_t* a_planes;     // [nchunks][2][128 * 64] hi plane then lo plane, 32 KB per chunk
-    const int32_t* tile_chunk0;   // [ntiles + 1] first chunk of each tile
-    const int32_t* ksteps;        // [nchunks] K = 16 steps that hold data (1..4)
-    // the same plan per K step (16 input rows), for the fused kernel (gnnb_tc.cu, k_tc_fused): the steps that hold data only
     const int32_t* tile_ks0;      // [ntiles + 1] first K step of each tile
     const int32_t* ks_rows;       // [nksteps][16] input slot of each K row, -1 = zero row
     const uint16_t* ks_w;         // [nksteps] 8 KB weight blocks: [hi plane 4 KB][lo plane 4 KB], each 128 x 16 fp16 K-major without
@@ -22,321 +17,8 @@ struct PropPlanDev {
     int nslots_in, nslots_out;    // rows per subdomain of the input / output layer (slot order, gnnb_common.cuh)
 };
 
-
 struct PropPlan;
 const PropPlanDev& prop_plan_dev(const PropPlan* p);
-double prop_plan_chunks_per_tile(const PropPlan* p);
 double prop_plan_ksteps_per_tile(const PropPlan* p);
 
-namespace prop {
-
-// ---- the gather-GEMM kernel ---------------------------------------------------------------------------------
-// A persistent CTA (1 per SM) walks items = (tile of 128 output nodes, group of PD = 4 subdomains); per K chunk
-//   D[128 nodes x (4 subdomains x 64 channels)] += Wblock[128 x 64] * Mu[64 input nodes x (4 x 64)]
-// as tcgen05.mma M = 128, N = 256, K = 16, three passes for the fp16 hi/lo split (Wh Mh + Wl Mh + Wh Ml).
-// Warp roles (14 warps), decoupled by mbarrier rings:
-//   warp 0      TMA: the chunk's 32 KB weight block (hi, lo plane; K-major SWIZZLE_128B)      -> W ring, 3 stages
-//   warp 1      MMA issue + tcgen05.commit (frees ring stages, publishes accumulators): all 32 lanes walk the loop with
-//               uniform operands, one elected lane issues (6 back-to-back UTCHMMA per half chunk)
-//   warps 2-5   gather, one subdomain each: the chunk's input-node rows are copied with 16-byte cp.async straight
-//               from the mu tile images (already fp16 hi/lo, scaled) into the MN-major SWIZZLE_128B B operand — no
-//               registers, no conversion; half a chunk (32 rows x 4 subdomains x 2 planes = 32 KB) per stage, 4 stages
-//   warps 6-13  two epilogue warpgroups, alternating items on a double-buffered accumulator (2 x 256 TMEM columns):
-//               tcgen05.ld -> fp16 hi/lo split -> piece-major nb tile image (consecutive rows = consecutive 16 bytes)
-constexpr int PD = 4;
-constexpr int W_STAGES = 3, B_STAGES = 4;
-constexpr uint32_t W_STAGE_BYTES = 2 * APLANE;            // 32 KB
-constexpr uint32_t B_ROWS = 32;                           // input nodes per B stage (half a chunk = 2 K steps)
-constexpr uint32_t B_DOM_BYTES = B_ROWS * 128;            // 4 KB: one plane of one subdomain
-constexpr uint32_t B_PLANE_BYTES = PD * B_DOM_BYTES;      // 16 KB
-constexpr uint32_t B_STAGE_BYTES = 2 * B_PLANE_BYTES;     // 32 KB
-constexpr int PROP_WARPS = 14, PROP_THREADS = PROP_WARPS * 32;
-constexpr int GATHER_WARP0 = 2, EPI_WARP0 = 6;
-
-template <int WS, int BS>
-struct PropTailT {
-    uint64_t w_full[WS], w_empty[WS], b_full[BS], b_empty[BS], acc_full[2], acc_empty[2];
-    uint32_t tmem_slot;
-};
-using PropTail = PropTailT<W_STAGES, B_STAGES>;
-static_assert(sizeof(PropTailT<2, 5>) == sizeof(PropTail), "the 2 + 5 stage variant uses the same shared memory");
-constexpr size_t PROP_SMEM = 1024 + W_STAGES * W_STAGE_BYTES + B_STAGES * B_STAGE_BYTES + sizeof(PropTail);
-
-// One CTA's share of a propagation launch: items rank, rank + nranks, ...  All threads of the block must call it (block-wide
-// barriers).
-template <bool GATHER_PREFETCH = false, int WS = W_STAGES, int BS = B_STAGES>
-__device__ __forceinline__ void prop_body(const PropPlanDev& plan, const uint16_t* __restrict__ mu_img, uint16_t* __restrict__ nb_img,
-                                          int Bc, unsigned char* smem_raw, int rank, int nranks, bool pdl = false) {
-    unsigned char* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // keeps the shared address space
-    const uint32_t w_ring = smem_u32(base), b_ring = w_ring + WS * W_STAGE_BYTES;
-    using Tail = PropTailT<WS, BS>;
-    Tail* tail = reinterpret_cast<Tail*>(base + WS * W_STAGE_BYTES + BS * B_STAGE_BYTES);
-    const int warp = uniform((int)(threadIdx.x >> 5)), lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < WS; ++i) { mbar_init(smem_u32(&tail->w_full[i]), 1); mbar_init(smem_u32(&tail->w_empty[i]), 1); }
-        for (int i = 0; i < BS; ++i) { mbar_init(smem_u32(&tail->b_full[i]), PD * 32); mbar_init(smem_u32(&tail->b_empty[i]), 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(smem_u32(&tail->acc_full[i]), 1); mbar_init(smem_u32(&tail->acc_empty[i]), 128); }
-        fence_mbar_init();
-    }
-    __syncwarp();
-    if (warp == 0) tmem_alloc(smem_u32(&tail->tmem_slot), 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = tail->tmem_slot;
-    if (pdl) { pdl_trigger(); pdl_wait(); }     // prologue done; the mu images are the predecessor's output
-
-    const int ngroups = (Bc + PD - 1) / PD;
-    const int64_t nitems = (int64_t)plan.ntiles * ngroups;       // item = group * ntiles + tile
-
-    if (warp == 0) {
-        // ---- weight blocks ----
-        if (lane == 0) {
-            uint32_t ws = 0, wph = 0;
-            for (int64_t item = rank; item < nitems; item += nranks) {
-                const int tile = (int)(item % plan.ntiles);
-                const int ch0 = plan.tile_chunk0[tile], ch1 = plan.tile_chunk0[tile + 1];
-                for (int ch = ch0; ch < ch1; ++ch) {
-                    mbar_wait(smem_u32(&tail->w_empty[ws]), wph ^ 1u);
-                    const uint32_t full = smem_u32(&tail->w_full[ws]);
-                    mbar_expect_tx(full, W_STAGE_BYTES);
-                    bulk_g2s(w_ring + ws * W_STAGE_BYTES, plan.a_planes + (size_t)ch * (W_STAGE_BYTES / 2), W_STAGE_BYTES, full);
-                    if (++ws == WS) { ws = 0; wph ^= 1u; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ---- MMA issue: the whole warp walks the loop (uniform control and operands), one elected lane issues ----
-        // D fp32, A fp16 K-major, B fp16 MN-major (bit 16), M = 128, N = 256
-        const uint32_t idesc = (1u << 4) | (1u << 16) | ((uint32_t)(PD * 64 >> 3) << 17) | ((uint32_t)(TILE >> 4) << 24);
-        uint32_t ws = 0, wph = 0, bs = 0, bph = 0, it = 0;
-#ifdef GNNB_TRACE
-        long long t_acc = 0, t_w = 0, t_b = 0, t_all = clock64(), t0_;
-        int n_chunks = 0;
-#define PTR_BEGIN() t0_ = clock64()
-#define PTR_END(x) x += clock64() - t0_
-#else
-#define PTR_BEGIN()
-#define PTR_END(x)
-#endif
-        for (int64_t item = rank; item < nitems; item += nranks, ++it) {
-            const int tile = (int)(item % plan.ntiles);
-            const int ch0 = uniform(plan.tile_chunk0[tile]), ch1 = uniform(plan.tile_chunk0[tile + 1]);
-            const uint32_t a = it & 1u, aph = (it >> 1) & 1u;
-            PTR_BEGIN();
-            mbar_wait(smem_u32(&tail->acc_empty[a]), aph ^ 1u);      // the epilogue has drained this accumulator
-            PTR_END(t_acc);
-            tc_fence_after();
-            const uint32_t d = (tmem_base & 0x0000FFFFu) + a * 256u;
-            uint32_t accum = 0;
-            for (int ch = ch0; ch < ch1; ++ch) {
-                PTR_BEGIN();
-                mbar_wait(smem_u32(&tail->w_full[ws]), wph);
-                PTR_END(t_w);
-                const int nks = uniform(plan.ksteps[ch]);
-                const uint32_t wa = w_ring + ws * W_STAGE_BYTES;
-                const uint64_t a_hi = make_desc(wa), a_lo = make_desc(wa + APLANE);
-                for (int h = 0; 2 * h < nks; ++h) {
-                    PTR_BEGIN();
-                    mbar_wait(smem_u32(&tail->b_full[bs]), bph);
-                    PTR_END(t_b);
-                    tc_fence_after();
-                    const uint32_t ba = b_ring + bs * B_STAGE_BYTES;
-                    const uint64_t b_hi = make_desc_mn(ba, B_DOM_BYTES), b_lo = make_desc_mn(ba + B_PLANE_BYTES, B_DOM_BYTES);
-                    const bool two = nks - 2 * h >= 2;             // K steps of this half chunk that hold data: 1 or 2
-                    const uint64_t ah0 = a_hi + (uint64_t)(4 * h), al0 = a_lo + (uint64_t)(4 * h);
-                    if (elect_one()) {
-                        umma(d, ah0, b_hi, idesc, accum);                      // Wh Mh
-                        if (two) umma(d, ah0 + 2, b_hi + 128, idesc, 1u);
-                        umma(d, al0, b_hi, idesc, 1u);                         // Wl Mh
-                        if (two) umma(d, al0 + 2, b_hi + 128, idesc, 1u);
-                        umma(d, ah0, b_lo, idesc, 1u);                         // Wh Ml
-                        if (two) umma(d, ah0 + 2, b_lo + 128, idesc, 1u);
-                        umma_commit(smem_u32(&tail->b_empty[bs]));
-                    }
-                    __syncwarp();
-                    accum = 1u;
-                    if (++bs == BS) { bs = 0; bph ^= 1u; }
-                }
-                if (elect_one()) umma_commit(smem_u32(&tail->w_empty[ws]));
-                __syncwarp();
-                if (++ws == WS) { ws = 0; wph ^= 1u; }
-            }
-            if (elect_one()) umma_commit(smem_u32(&tail->acc_full[a]));
-            __syncwarp();
-#ifdef GNNB_TRACE
-            n_chunks += ch1 - ch0;
-#endif
-        }
-#ifdef GNNB_TRACE
-        if (rank == 1 && lane == 0) printf("TRACE prop-mma: items %u chunks %d total %lld | wait acc_empty %lld, w_full %lld, b_full %lld\n", it, n_chunks,
-                                           clock64() - t_all, t_acc, t_w, t_b);
-#endif
-    } else if (warp < EPI_WARP0 && GATHER_PREFETCH) {
-        // ---- gather with the row indices fetched one chunk ahead (option "gather_prefetch"; NOT the default yet) ----
-        // ncu's source page puts 57 % of the gather warps' samples on the first shuffle of `idx` below, i.e. on the latency of
-        // the index load that precedes every stage (profiles/r01s, DESIGN §7): here the 64 indices and the K-step count of
-        // the next chunk (of this item or of the CTA's next item) are in registers before the current chunk is copied.
-        const int g = warp - GATHER_WARP0;
-        const unsigned char* mu_bytes = reinterpret_cast<const unsigned char*>(mu_img);
-        uint32_t bs = 0, bph = 0;
-        int64_t item = rank;
-        if (item < nitems) {
-            int ch = plan.tile_chunk0[(int)(item % plan.ntiles)], ch1 = plan.tile_chunk0[(int)(item % plan.ntiles) + 1];
-            int i0 = __ldg(plan.in_rows + (size_t)ch * 64 + lane), i1 = __ldg(plan.in_rows + (size_t)ch * 64 + B_ROWS + lane);
-            int nks = __ldg(plan.ksteps + ch);
-            while (true) {
-                int64_t nitem = item;
-                int nch = ch + 1, nch1 = ch1;
-                if (nch >= ch1) {
-                    nitem = item + nranks;
-                    if (nitem < nitems) {
-                        const int nt = (int)(nitem % plan.ntiles);
-                        nch = plan.tile_chunk0[nt]; nch1 = plan.tile_chunk0[nt + 1];
-                    }
-                }
-                const bool has_next = nitem < nitems;
-                int n0 = -1, n1 = -1, nnks = 0;
-                if (has_next) {
-                    n0 = __ldg(plan.in_rows + (size_t)nch * 64 + lane); n1 = __ldg(plan.in_rows + (size_t)nch * 64 + B_ROWS + lane);
-                    nnks = __ldg(plan.ksteps + nch);
-                }
-                const int d = (int)(item / plan.ntiles) * PD + g;
-                const bool dom_ok = d < Bc;
-                const int64_t drow = (int64_t)d * plan.nslots_in;
-                for (int h = 0; 2 * h < nks; ++h) {
-                    const int idx = h ? i1 : i0;
-                    mbar_wait(smem_u32(&tail->b_empty[bs]), bph ^ 1u);
-                    const uint32_t dst0 = b_ring + bs * B_STAGE_BYTES + (uint32_t)g * B_DOM_BYTES;
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const int k = i * 4 + (lane >> 3);
-                        const int node = __shfl_sync(0xffffffffu, idx, k);
-                        const bool ok = dom_ok && node >= 0;
-                        const int64_t grow = ok ? drow + node : 0;
-                        const uint32_t r = (uint32_t)(grow & (TILE - 1));
-                        const uint32_t jp = (uint32_t)(lane & 7);
-                        const unsigned char* src = mu_bytes + (grow >> 7) * (int64_t)ABUF + (r >> 3) * 1024u + (r & 7u) * 128u + jp * 16u;
-                        const uint32_t dst = dst0 + swz((uint32_t)k, jp ^ (r & 7u));
-                        cp_async16(dst, src, ok);
-                        cp_async16(dst + B_PLANE_BYTES, src + APLANE, ok);
-                    }
-                    cp_async_arrive(smem_u32(&tail->b_full[bs]));
-                    if (++bs == BS) { bs = 0; bph ^= 1u; }
-                }
-                if (!has_next) break;
-                item = nitem; ch = nch; ch1 = nch1; i0 = n0; i1 = n1; nks = nnks;
-            }
-        }
-    } else if (warp < EPI_WARP0) {
-        // ---- gather: warp g copies the rows of subdomain d0 + g ----
-        const int g = warp - GATHER_WARP0;
-        const unsigned char* mu_bytes = reinterpret_cast<const unsigned char*>(mu_img);
-        uint32_t bs = 0, bph = 0;
-#ifdef GNNB_TRACE
-        long long g_wait = 0, g_all = clock64(), g0_;
-#endif
-        for (int64_t item = rank; item < nitems; item += nranks) {
-            const int tile = (int)(item % plan.ntiles);
-            const int d = (int)(item / plan.ntiles) * PD + g;
-            const bool dom_ok = d < Bc;
-            const int64_t drow = (int64_t)d * plan.nslots_in;
-            const int ch0 = plan.tile_chunk0[tile], ch1 = plan.tile_chunk0[tile + 1];
-            for (int ch = ch0; ch < ch1; ++ch) {
-                const int nks = plan.ksteps[ch];
-                for (int h = 0; 2 * h < nks; ++h) {
-                    const int idx = __ldg(plan.in_rows + (size_t)ch * 64 + h * B_ROWS + lane);
-#ifdef GNNB_TRACE
-                    g0_ = clock64();
-#endif
-                    mbar_wait(smem_u32(&tail->b_empty[bs]), bph ^ 1u);
-#ifdef GNNB_TRACE
-                    g_wait += clock64() - g0_;
-#endif
-                    const uint32_t dst0 = b_ring + bs * B_STAGE_BYTES + (uint32_t)g * B_DOM_BYTES;
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const int k = i * 4 + (lane >> 3);               // row of the stage: 4 rows x 8 chunks per instruction
-                        const int node = __shfl_sync(0xffffffffu, idx, k);
-                        const bool ok = dom_ok && node >= 0;
-                        const int64_t grow = ok ? drow + node : 0;
-                        const uint32_t r = (uint32_t)(grow & (TILE - 1));
-                        const uint32_t jp = (uint32_t)(lane & 7);       // physical 16-byte chunk of the row in the mu image
-                        const unsigned char* src = mu_bytes + (grow >> 7) * (int64_t)ABUF + (r >> 3) * 1024u + (r & 7u) * 128u + jp * 16u;
-                        const uint32_t dst = dst0 + swz((uint32_t)k, jp ^ (r & 7u));   // logical chunk = physical ^ (row & 7)
-                        cp_async16(dst, src, ok);
-                        cp_async16(dst + B_PLANE_BYTES, src + APLANE, ok);
-                    }
-                    cp_async_arrive(smem_u32(&tail->b_full[bs]));
-                    if (++bs == BS) { bs = 0; bph ^= 1u; }
-                }
-            }
-        }
-#ifdef GNNB_TRACE
-        if (rank == 1 && g == 0 && lane == 0) printf("TRACE prop-gather: total %lld, wait b_empty %lld\n", clock64() - g_all, g_wait);
-#endif
-    } else if (warp < EPI_WARP0 + 8) {
-        // ---- epilogue: warpgroup ew takes the items it & 1 == ew ----
-        const int ew = (warp - EPI_WARP0) >> 2;
-        const int m = (warp & 3) * 32 + lane;                      // TMEM lane = tile row (a warp reaches lanes 32 * (warp % 4) ..)
-        const uint32_t tmem = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)ew * 256u;
-        const uint32_t full = smem_u32(&tail->acc_full[ew]), empty = smem_u32(&tail->acc_empty[ew]);
-        uint32_t aph = 0, it = 0;
-#ifdef GNNB_TRACE
-        long long e_wait = 0, e_work = 0, e0_;
-#endif
-        for (int64_t item = rank; item < nitems; item += nranks, ++it) {
-            if ((int)(it & 1u) != ew) continue;
-            const int tile = (int)(item % plan.ntiles);
-            const int d0 = (int)(item / plan.ntiles) * PD;
-#ifdef GNNB_TRACE
-            e0_ = clock64();
-#endif
-            mbar_wait(full, aph);
-            aph ^= 1u;
-            tc_fence_after();
-#ifdef GNNB_TRACE
-            e_wait += clock64() - e0_; e0_ = clock64();
-#endif
-#pragma unroll 1
-            for (int dom = 0; dom < PD; ++dom) {
-                if (d0 + dom >= Bc) break;
-                // slot order: the tile's 128 rows are one tile image of the output layer; thread = row, so a warp's store
-                // instruction writes 512 contiguous bytes of a piece
-                unsigned char* img = reinterpret_cast<unsigned char*>(nb_img) +
-                                     ((int64_t)(d0 + dom) * plan.ntiles + tile) * (int64_t)ABUF + (uint32_t)m * 16u;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    float x[16];
-                    tmem_ld16_sync(tmem + (uint32_t)(dom * 64 + q * 16), x);
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        uint4 hi, lo;
-                        split2(x[h * 8 + 0], x[h * 8 + 1], hi.x, lo.x);
-                        split2(x[h * 8 + 2], x[h * 8 + 3], hi.y, lo.y);
-                        split2(x[h * 8 + 4], x[h * 8 + 5], hi.z, lo.z);
-                        split2(x[h * 8 + 6], x[h * 8 + 7], hi.w, lo.w);
-                        const uint32_t off = (uint32_t)(q * 2 + h) * NB_PIECE;
-                        *reinterpret_cast<uint4*>(img + off) = hi;
-                        *reinterpret_cast<uint4*>(img + APLANE + off) = lo;
-                    }
-                }
-            }
-            tc_fence_before();
-            mbar_arrive(empty);
-#ifdef GNNB_TRACE
-            e_work += clock64() - e0_;
-#endif
-        }
-#ifdef GNNB_TRACE
-        if (rank == 1 && m == 0) printf("TRACE prop-epi wg %d: wait acc_full %lld, work %lld\n", ew, e_wait, e_work);
-#endif
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem_base, 512);
-}
-
-
-}  // namespace prop
 }  // namespace gnnb

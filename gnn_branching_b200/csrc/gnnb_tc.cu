@@ -46,6 +46,7 @@
 //   mu       per tile [hi plane][lo plane] K-major SWIZZLE_128B (a row's 64 channels = 128 contiguous bytes), bulk-stored;
 //   relax'   ambiguous rows only, compacted in row order: [tile][16 channel quads][128 slots][4] fp32 (scaled domain).
 #include "gnnb_prop_body.cuh"
+#include "gnnb_umma.cuh"
 
 namespace gnnb {
 namespace {
@@ -1653,17 +1654,6 @@ void tc_update(const GnnParams& g, bool backward, const float* lb, const float* 
     ++*launches;
 }
 
-// process-wide experiment knobs of the fused kernel (gnnb_set_option "fused_mma_group")
-static int env_int(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : dflt;
-}
-static struct { int mma_group = env_int("GNNB_FUSED_MMA_GROUP", 0); } g_fused_tune;
-void tc_fused_tune(const char* key, int value) {
-    const std::string k(key);
-    if (k == "mma_group") g_fused_tune.mma_group = value;
-}
-
 void tc_fused(const GnnParams& g, const PropPlan* plan, const float* mu_in, bool backward, const float* lb, const float* ub,
               const float* relax, const int32_t* amb_base, float* mu_out, float* scores, RowMap map, int64_t score_stride, int64_t score_off,
               int64_t rows, unsigned long long* nan_count, float* nb_dbg, bool input_layer, cudaStream_t st, int64_t* launches) {
@@ -1681,7 +1671,6 @@ void tc_fused(const GnnParams& g, const PropPlan* plan, const float* mu_in, bool
     // behind whatever the propagation has issued: groups of 4 K steps for the former, pairs of steps for the latter
     // (a chain takes ~11 000 cycles per item, a K step 192 cycles of tensor time: only K loops of 48+ steps outlast the chains)
     fa.mma_group = prop_plan_ksteps_per_tile(plan) >= 48.0 ? 4 : 2;      // (2 instead of 1 for the short loops: +1 % on the base step)
-    if (g_fused_tune.mma_group > 0) fa.mma_group = g_fused_tune.mma_group;
     if (fa.mma_group > fa.n_stages / 2) fa.mma_group = fa.n_stages / 2;
     const int64_t nitems = (int64_t)fa.plan.ntiles * ((fa.u.Bc + fz::PD - 1) / fz::PD);
     launch_pdl(input_layer ? k_tc_fused_input : k_tc_fused, (int)(nitems < 1 ? 1 : (nitems < 148 ? nitems : 148)), fz::THREADS,

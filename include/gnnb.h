@@ -105,12 +105,13 @@ int gnnb_set_gnn_weights(gnnb_ctx* ctx, const float* const* tensors, const int64
  * (graph_conv.py:107-137, 222-249). */
 int gnnb_set_network(gnnb_ctx* ctx, const gnnb_layer_desc* layers, int n_layers, int c0, int h0, int w0);
 
-/* Options: "math" (gnnb_math_mode), "chunk" (subdomains per wave; 0 = auto), "gather_prefetch" (0/1/2, default 0: propagation
- * kernel variants that fetch their gather indices one chunk ahead; 2 also trades one weight stage for a gather stage), "fuse" (0/1, default 0: propagation and
- * node update of a layer in one launch, tensor-core mode), "prop_share" (0 = cost model, else the percentage of the
- * CTAs of a fused launch that run the propagation), "snapshot" (0/1: keep
- * per-stage copies for gnnb_debug_snapshot; debugging only), "profile" (0/1: time every stage launch with
- * CUDA events for gnnb_profile_read). */
+/* Options: "math" (gnnb_math_mode), "chunk" (subdomains per wave; 0 = auto), "fuse" (0/1, default 1: propagation and
+ * node update of a layer in one launch, tensor-core mode; 0 = two launches), "snapshot" (0/1: keep per-stage copies
+ * for gnnb_debug_snapshot; debugging only), "profile" (0/1: time every stage launch with CUDA events for
+ * gnnb_profile_read).  Any other key of gnnb_set_option fails with GNNB_ERR_INVALID.
+ * gnnb_get_option also reads these, and "n_hidden" (hidden ReLUs of the network), "workspace_domains" (subdomains the
+ * workspace holds) and "plan_density_pct_f<k>" / "plan_density_pct_b<k>" (percentage of the MACs issued by forward /
+ * backward propagation plan k that are useful); it returns -1 for an unknown key. */
 int gnnb_set_option(gnnb_ctx* ctx, const char* key, int64_t value);
 int64_t gnnb_get_option(gnnb_ctx* ctx, const char* key);
 

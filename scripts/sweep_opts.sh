@@ -1,5 +1,5 @@
 #!/bin/bash
-# bench.py over a list of library option sets: bash scripts/sweep_opts.sh <workload> "fuse=1 prop_share=30" "fuse=0" ...
+# bench.py over a list of library option sets: bash scripts/sweep_opts.sh <workload> "fuse=1" "fuse=0 chunk=512" ...
 W=$1; shift
 for o in "$@"; do
   args=""; for kv in $o; do args="$args --opt $kv"; done

@@ -14,24 +14,6 @@ from golden_io import load_case, load_gnn, load_root             # noqa: E402
 from gnn_branching_b200 import GraphNet, synthetic_frontier      # noqa: E402
 
 
-def check_gather_prefetch(arch):
-    """The propagation kernel variants k_tc_prop_pf (option value 1) and k_tc_prop_pf25 (2) must give bit-identical scores,
-    winners and indices."""
-    fr, _ = load_case(arch, 'fr')
-    model = GraphNet(2, 64, math='tc')
-    model.load_state_dict(load_gnn('random'))
-    model = model.eval().cuda()
-    model.scorer(0).set_option('fuse', 0)          # the variants belong to the stand-alone propagation kernel
-    for f in (fr.to('cuda'), synthetic_frontier(*load_root(arch), 37, seed=5, device='cuda')):
-        model.scorer(0).set_option('gather_prefetch', 0)
-        b0, i0, s0 = model.score_frontier(f)
-        for variant in (1, 2):
-            model.scorer(0).set_option('gather_prefetch', variant)
-            b1, i1, s1 = model.score_frontier(f)
-            torch.cuda.synchronize()
-            assert torch.equal(s0, s1) and torch.equal(i0, i1) and torch.equal(b0, b1), f'gather_prefetch={variant} changes the results'
-
-
 def check_fused(arch):
     """k_tc_fused (default) against the two-launch path: both split the same fp32 propagation accumulator into the same fp16
     hi / lo operand, but the first chain GEMM reads it from tensor memory instead of shared memory and the hardware's
@@ -324,6 +306,6 @@ def check_frontier_step(arch):
 
 
 if __name__ == '__main__':
-    {'gather_prefetch': check_gather_prefetch, 'frontier_step': check_frontier_step, 'kw_bounds': check_kw_bounds, 'fused': check_fused,
+    {'frontier_step': check_frontier_step, 'kw_bounds': check_kw_bounds, 'fused': check_fused,
      'child_bounds': check_child_bounds, 'child_bounds_shapes': check_child_bounds_shapes}[sys.argv[1]](sys.argv[2])
     print('ok')

@@ -638,11 +638,6 @@ def _run_isolated(what, arg, timeout=120, env=None):
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-2000:])
 
 
-@pytest.mark.parametrize('arch', ARCHS)
-def test_gather_prefetch_variant_is_bit_identical(arch):
-    _run_isolated('gather_prefetch', arch)
-
-
 @pytest.mark.parametrize('math', ['0', '1'])
 @pytest.mark.parametrize('arch', ARCHS)
 def test_kw_bounds_match_reference(arch, math):
