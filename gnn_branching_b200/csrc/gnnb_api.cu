@@ -32,6 +32,8 @@ struct gnnb_ctx {
     int chunk = 0;
     int snapshot = 0;
     int fuse = 1;                   // propagation + node update of a layer in one launch, nb handed over in tensor memory (k_tc_fused); 0 = two launches
+    int rescore = 0;                // score the subdomains whose tensor-core pass met a NaN again in exact fp32 (rescore_flagged)
+    int64_t rescored = 0;           // subdomains the last scoring call scored again
     // GNN parameters
     bool have_gnn = false;
     float* d_gnn = nullptr;
@@ -94,6 +96,12 @@ struct gnnb_ctx {
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr};
     unsigned long long* d_nan = nullptr;
+    // option "rescore": NanDoms of a call, [count | flags [resc_cap] | list [resc_cap]] (grow-only; count and flags are 0 between
+    // calls), and the gather table of the re-score pass (grow-only)
+    int32_t* d_resc = nullptr;
+    int resc_cap = 0;
+    RowGather* d_gather = nullptr;
+    size_t gather_cap = 0;
     // debugging snapshots
     std::map<std::string, std::pair<float*, int64_t>> snaps;
     // per-kernel-class device timing (option "profile")
@@ -213,8 +221,8 @@ int ensure_workspace(gnnb_ctx* ctx, int Bc, bool host_staging) {
 
 #define TRY_(expr) do { int s__ = (expr); if (s__ != GNNB_OK) return s__; } while (0)
 
-int snap(gnnb_ctx* ctx, const std::string& name, const float* src, int64_t numel, cudaStream_t st) {
-    if (!ctx->snapshot) return GNNB_OK;
+int snap(gnnb_ctx* ctx, bool on, const std::string& name, const float* src, int64_t numel, cudaStream_t st) {
+    if (!on) return GNNB_OK;
     auto it = ctx->snaps.find(name);
     if (it == ctx->snaps.end() || it->second.second < numel) {
         if (it != ctx->snaps.end()) cudaFree(it->second.first);
@@ -264,11 +272,11 @@ int prof_collect(gnnb_ctx* ctx) {
 }
 
 // mu and nb are fp16 tile images in tensor-core mode (mu swizzled, nb piece-major): unpack them into the snapshot
-int snap_img(gnnb_ctx* ctx, const std::string& name, const float* img, int k, int Bc, bool piece_major, cudaStream_t st) {
-    if (!ctx->snapshot) return GNNB_OK;
+int snap_img(gnnb_ctx* ctx, bool on, const std::string& name, const float* img, int k, int Bc, bool piece_major, cudaStream_t st) {
+    if (!on) return GNNB_OK;
     const int64_t numel = (int64_t)Bc * ctx->n[k] * P;                     // snapshots are in node order in both modes
-    if (ctx->math != GNNB_MATH_TC_FP16X3) return snap(ctx, name, img, numel, st);
-    TRY_(snap(ctx, name, img, numel, st));          // allocates / sizes the snapshot buffer
+    if (ctx->math != GNNB_MATH_TC_FP16X3) return snap(ctx, on, name, img, numel, st);
+    TRY_(snap(ctx, on, name, img, numel, st));      // allocates / sizes the snapshot buffer
     tc_unpack_tile_image(img, ctx->snaps[name].first, ctx->rowmap[k], (int64_t)Bc * ctx->rowmap[k].nslots, piece_major, st);
     return GNNB_OK;
 }
@@ -280,12 +288,14 @@ struct ChunkPtrs {
 
 #define TRY(expr) do { int s__ = (expr); if (s__ != GNNB_OK) return s__; } while (0)
 
-// the stage schedule for one chunk; every pointer is a device pointer
-int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* best_score, int32_t* best_idx,
+// the stage schedule for one chunk in arithmetic `math`; every pointer is a device pointer; nd: where the tensor-core NaN watch
+// records the subdomains it flags (nd.flag = null: nowhere)
+int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, int math, const NanDoms& nd, float* scores, float* best_score, int32_t* best_idx,
               gnnb_winner* winners, cudaStream_t st) {
     const int L = (int)ctx->layers.size();
     const GnnParams& g = ctx->gp;
-    const bool tc = ctx->math == GNNB_MATH_TC_FP16X3;
+    const bool tc = math == GNNB_MATH_TC_FP16X3;
+    const bool snaps = ctx->snapshot && math == ctx->math;        // an fp32 re-score pass leaves the tensor-core pass's snapshots
     int64_t* lc = &ctx->launches;
     auto name = [](const char* fmt, int a, int b) { char buf[64]; snprintf(buf, sizeof buf, fmt, a, b); return std::string(buf); };
 
@@ -331,8 +341,8 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
                 simt_relax(g, nis[k], ctx->relax_f[k], ctx->relax_b[k], st, lc);
             }
             // tensor-core mode stores relax' (pre-multiplied by fc4 / bc4's relax half, compacted, tile-transposed): not comparable 1:1
-            TRY(snap(ctx, name(tc ? "relaxp_f%d" : "relax_f%d", k, 0), ctx->relax_f[k], (int64_t)Bc * ctx->n[k] * P, st));
-            TRY(snap(ctx, name(tc ? "relaxp_b%d" : "relax_b%d", k, 0), ctx->relax_b[k], (int64_t)Bc * ctx->n[k] * P, st));
+            TRY(snap(ctx, snaps, name(tc ? "relaxp_f%d" : "relax_f%d", k, 0), ctx->relax_f[k], (int64_t)Bc * ctx->n[k] * P, st));
+            TRY(snap(ctx, snaps, name(tc ? "relaxp_b%d" : "relax_b%d", k, 0), ctx->relax_b[k], (int64_t)Bc * ctx->n[k] * P, st));
         }
     }
     {
@@ -340,7 +350,7 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
         if (tc) tc_input_embed(g, in.lb[0], in.pin, in.ub[0], ctx->mu[0], M(0), R(0), st, lc);
         else simt_input_embed(g, in.lb[0], in.pin, in.ub[0], ctx->mu[0], R(0), st, lc);
     }
-    TRY(snap_img(ctx, "mu0_embed", ctx->mu[0], 0, Bc, false, st));
+    TRY(snap_img(ctx, snaps, "mu0_embed", ctx->mu[0], 0, Bc, false, st));
 
     for (int t = 0; t < g.T; ++t) {
         const bool last = (t == g.T - 1);
@@ -350,26 +360,26 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
             if (fused) {
                 ProfScope ps(ctx, GNNB_K_LAYER_FWD, nodes, st);
                 tc_fused(g, ctx->plan_fwd[k - 1], ctx->mu[k - 1], false, in.lb[k], in.ub[k], ctx->relax_f[k], ctx->amb_base[k],
-                         ctx->mu[k], nullptr, M(k), 0, 0, rows, ctx->d_nan, ctx->snapshot ? ctx->nb : nullptr, false, st, lc);
+                         ctx->mu[k], nullptr, M(k), 0, 0, rows, ctx->d_nan, nd, ctx->snapshot ? ctx->nb : nullptr, false, st, lc);
             } else {
                 ProfScope ps(ctx, GNNB_K_PROP_FWD, nodes, st);
                 if (tc) prop_tc_run(ctx->plan_fwd[k - 1], ctx->mu[k - 1], ctx->nb, Bc, st, lc);
                 else prop_forward(ctx->layers[k - 1], ctx->mu[k - 1], ctx->nb, Bc, st, lc);
             }
-            TRY(snap_img(ctx, name("t%d_fwd_nb%d", t, k), ctx->nb, k, Bc, true, st));
+            TRY(snap_img(ctx, snaps, name("t%d_fwd_nb%d", t, k), ctx->nb, k, Bc, true, st));
             if (!fused) {
                 ProfScope ps(ctx, GNNB_K_UPDATE_FWD, nodes, st);
-                if (tc) tc_update(g, false, in.lb[k], in.ub[k], ctx->nb, ctx->relax_f[k], ctx->amb_base[k], ctx->mu[k], nullptr, M(k), 0, 0, rows, ctx->d_nan, st, lc);
+                if (tc) tc_update(g, false, in.lb[k], in.ub[k], ctx->nb, ctx->relax_f[k], ctx->amb_base[k], ctx->mu[k], nullptr, M(k), 0, 0, rows, ctx->d_nan, nd, st, lc);
                 else simt_update(g, false, in.lb[k], in.ub[k], ctx->nb, ctx->relax_f[k], ctx->mu[k], nullptr, ctx->n[k], 0, 0, rows, ctx->d_nan, st, lc);
             }
-            TRY(snap_img(ctx, name("t%d_fwd_mu%d", t, k), ctx->mu[k], k, Bc, false, st));
+            TRY(snap_img(ctx, snaps, name("t%d_fwd_mu%d", t, k), ctx->mu[k], k, Bc, false, st));
         }
         {
             ProfScope ps(ctx, GNNB_K_OUTPUT, Bc, st);
             output_node(g, in.wp, in.bp, ctx->mu[L], tc, tc ? ctx->rowmap[L].nslots : ctx->n[L], in.lb[L + 1], in.ub[L + 1], in.pout,
                         ctx->mu[L + 1], ctx->n[L], Bc, st, lc);
         }
-        TRY(snap(ctx, name("t%d_mu_out", t, 0), ctx->mu[L + 1], (int64_t)Bc * P, st));
+        TRY(snap(ctx, snaps, name("t%d_mu_out", t, 0), ctx->mu[L + 1], (int64_t)Bc * P, st));
         // backward sweep
         for (int k = L; k >= 1; --k) {
             const int64_t rows = R(k), nodes = (int64_t)Bc * ctx->n[k];
@@ -380,7 +390,7 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
             if (fused_k) {
                 ProfScope ps(ctx, last ? GNNB_K_LAYER_BWD_SCORE : GNNB_K_LAYER_BWD, nodes, st);
                 tc_fused(g, ctx->plan_bwd[k], ctx->mu[k + 1], true, in.lb[k], in.ub[k], ctx->relax_b[k], ctx->amb_base[k],
-                         mu_k, sc, M(k), ctx->n_hidden, ctx->hidden_off[k], rows, ctx->d_nan, ctx->snapshot ? ctx->nb : nullptr, false, st, lc);
+                         mu_k, sc, M(k), ctx->n_hidden, ctx->hidden_off[k], rows, ctx->d_nan, nd, ctx->snapshot ? ctx->nb : nullptr, false, st, lc);
             } else {
                 ProfScope ps(ctx, GNNB_K_PROP_BWD, nodes, st);
                 if (k == L && tc) prop_tc_property_backward(in.wp, ctx->mu[L + 1], ctx->nb, ctx->n[L], ctx->rowmap[L].nslots, Bc, st, lc);
@@ -388,20 +398,20 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
                 else if (tc) prop_tc_run(ctx->plan_bwd[k], ctx->mu[k + 1], ctx->nb, Bc, st, lc);
                 else prop_backward(ctx->layers[k], ctx->mu[k + 1], ctx->nb, Bc, true, st, lc);
             }
-            TRY(snap_img(ctx, name("t%d_bwd_nb%d", t, k), ctx->nb, k, Bc, true, st));
+            TRY(snap_img(ctx, snaps, name("t%d_bwd_nb%d", t, k), ctx->nb, k, Bc, true, st));
             if (!fused_k) {
                 ProfScope ps(ctx, last ? GNNB_K_UPDATE_BWD_SCORE : GNNB_K_UPDATE_BWD, nodes, st);
-                if (tc) tc_update(g, true, in.lb[k], in.ub[k], ctx->nb, ctx->relax_b[k], ctx->amb_base[k], mu_k, sc, M(k), ctx->n_hidden, ctx->hidden_off[k], rows, ctx->d_nan, st, lc);
+                if (tc) tc_update(g, true, in.lb[k], in.ub[k], ctx->nb, ctx->relax_b[k], ctx->amb_base[k], mu_k, sc, M(k), ctx->n_hidden, ctx->hidden_off[k], rows, ctx->d_nan, nd, st, lc);
                 else simt_update(g, true, in.lb[k], in.ub[k], ctx->nb, ctx->relax_b[k], ctx->mu[k], sc, ctx->n[k], ctx->n_hidden, ctx->hidden_off[k], rows, ctx->d_nan, st, lc);
             }
-            TRY(snap_img(ctx, name("t%d_bwd_mu%d", t, k), ctx->mu[k], k, Bc, false, st));
+            TRY(snap_img(ctx, snaps, name("t%d_bwd_mu%d", t, k), ctx->mu[k], k, Bc, false, st));
         }
         // input layer: feeds the next round only (dead on the last round, SURVEY §8a fact 2)
         if (!last && fused) {
             ProfScope ps(ctx, GNNB_K_INPUT_UPDATE, (int64_t)Bc * ctx->n[0], st);
             tc_fused(g, ctx->plan_bwd[0], ctx->mu[1], true, in.lb[0], in.ub[0], nullptr, nullptr, ctx->mu[0], nullptr, M(0), 0, 0, R(0),
-                     ctx->d_nan, nullptr, true, st, lc);
-            TRY(snap_img(ctx, name("t%d_mu0", t, 0), ctx->mu[0], 0, Bc, false, st));
+                     ctx->d_nan, nd, nullptr, true, st, lc);
+            TRY(snap_img(ctx, snaps, name("t%d_mu0", t, 0), ctx->mu[0], 0, Bc, false, st));
         } else if (!last) {
             {
                 ProfScope ps(ctx, GNNB_K_PROP_BWD, (int64_t)Bc * ctx->n[0], st);
@@ -413,13 +423,103 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, float* scores, float* 
                 if (tc) tc_input_update(g, in.lb[0], in.ub[0], ctx->nb, ctx->mu[0], M(0), R(0), st, lc);
                 else simt_input_update(g, in.lb[0], in.ub[0], ctx->nb, ctx->mu[0], R(0), st, lc);
             }
-            TRY(snap_img(ctx, name("t%d_mu0", t, 0), ctx->mu[0], 0, Bc, false, st));
+            TRY(snap_img(ctx, snaps, name("t%d_mu0", t, 0), ctx->mu[0], 0, Bc, false, st));
         }
     }
     {
         ProfScope ps(ctx, GNNB_K_ARGMAX, Bc, st);
         masked_argmax(scores, in.mask, ctx->n_hidden, Bc, best_score, best_idx, winners, st, lc);
     }
+    CU(cudaGetLastError());
+    return GNNB_OK;
+}
+
+// grow-only NanDoms buffer of option "rescore" for calls of up to B subdomains (zeroed when it is allocated)
+int ensure_nan_doms(gnnb_ctx* ctx, int B) {
+    if (ctx->resc_cap >= B) return GNNB_OK;
+    if (ctx->d_resc) { cudaFree(ctx->d_resc); ctx->d_resc = nullptr; ctx->resc_cap = 0; }
+    CU(cudaMalloc(&ctx->d_resc, (1 + 2 * (size_t)B) * sizeof(int32_t)));
+    CU(cudaMemset(ctx->d_resc, 0, (1 + 2 * (size_t)B) * sizeof(int32_t)));
+    ctx->resc_cap = B;
+    return GNNB_OK;
+}
+
+NanDoms nan_doms(gnnb_ctx* ctx) { return NanDoms{ctx->d_resc, ctx->d_resc + 1, ctx->d_resc + 1 + ctx->resc_cap, 0}; }
+
+// after a call that failed part-way: no subdomain may stay flagged for the next call
+void reset_nan_doms(gnnb_ctx* ctx, cudaStream_t st) {
+    cudaStreamSynchronize(st);
+    cudaMemset(ctx->d_resc, 0, (1 + 2 * (size_t)ctx->resc_cap) * sizeof(int32_t));
+}
+
+// Option "rescore", after the tensor-core pass of a call: read how many subdomains its NaN watch flagged (one device -> host copy
+// and one synchronise of `st`; nothing else when there are none), then score those again with the exact-fp32 schedule, in waves
+// of up to `chunk` gathered into staging set 0, and write their results over the tensor-core ones.  best / idx or winners:
+// device arrays of the whole call; scores: the caller's dense scores (in->mem) or null.  The NaN count is reset first, so that
+// afterwards it counts the fp32 pass only.
+int rescore_flagged(gnnb_ctx* ctx, const gnnb_frontier* in, int chunk, float* best, int32_t* idx, gnnb_winner* winners, float* scores,
+                    cudaStream_t st) {
+    const bool host = in->mem == GNNB_MEM_HOST;
+    const int L = (int)ctx->layers.size(), nh = ctx->n_hidden;
+    const std::vector<int>& n = ctx->n;
+    const NanDoms nd = nan_doms(ctx);
+    int32_t count = 0;
+    CU(cudaMemcpyAsync(&count, nd.count, sizeof count, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    ctx->rescored = count;
+    if (count == 0) return GNNB_OK;
+    std::vector<int32_t> rows;                    // host frontier: the flagged rows are copied from the caller's arrays one by one
+    if (host) {
+        rows.resize(count);
+        CU(cudaMemcpyAsync(rows.data(), nd.list, (size_t)count * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+    }
+    CU(cudaMemsetAsync(nd.count, 0, sizeof(int32_t), st));             // the scatter kernel clears the flags
+    CU(cudaMemsetAsync(ctx->d_nan, 0, sizeof(unsigned long long), st));
+    gnnb_ctx::Staging& sg = ctx->stg[0];
+    std::vector<RowGather> tab;
+    ChunkPtrs cp;
+    auto add = [&](const float* src, float* dst, int64_t per) { tab.push_back(RowGather{src, dst, per}); return dst; };
+    cp.lb.resize(L + 2); cp.ub.resize(L + 2); cp.dual.resize(L); cp.pre.resize(L); cp.post.resize(L);
+    for (int k = 0; k <= L + 1; ++k) { cp.lb[k] = add(in->lb[k], sg.lb[k], n[k]); cp.ub[k] = add(in->ub[k], sg.ub[k], n[k]); }
+    for (int k = 0; k < L; ++k) {
+        cp.dual[k] = add(in->dual[k], sg.dual[k], (int64_t)n[k + 1] * 3);
+        cp.pre[k] = add(in->prim_pre[k], sg.pre[k], n[k + 1]);
+        cp.post[k] = add(in->prim_post[k], sg.post[k], n[k + 1]);
+    }
+    cp.pout = add(in->prim_out, sg.pout, 1);
+    cp.pin = add(in->primal_input, sg.pin, n[0]);
+    cp.wp = add(in->wp, sg.wp, n[L]);
+    cp.bp = add(in->bp, sg.bp, 1);
+    cp.mask = add(in->mask, sg.mask, nh);
+    if (!host) {
+        if (ctx->gather_cap < tab.size()) {
+            if (ctx->d_gather) cudaFree(ctx->d_gather);
+            ctx->d_gather = nullptr; ctx->gather_cap = 0;
+            CU(cudaMalloc(&ctx->d_gather, tab.size() * sizeof(RowGather)));
+            ctx->gather_cap = tab.size();
+        }
+        // a stream-ordered copy from pageable memory returns after the source has been read: `tab` may go out of scope
+        CU(cudaMemcpyAsync(ctx->d_gather, tab.data(), tab.size() * sizeof(RowGather), cudaMemcpyHostToDevice, st));
+    }
+    for (int s0 = 0, Bs = 0; s0 < count; s0 += Bs) {
+        Bs = (count - s0) < chunk ? (count - s0) : chunk;
+        if (host) {
+            for (int i = 0; i < Bs; ++i)
+                for (const RowGather& t : tab)
+                    CU(cudaMemcpyAsync(t.dst + i * t.per, t.src + rows[s0 + i] * t.per, t.per * sizeof(float), cudaMemcpyHostToDevice, st));
+        } else {
+            gather_rows(ctx->d_gather, (int)tab.size(), nd.list + s0, Bs, st, &ctx->launches);
+        }
+        TRY(run_chunk(ctx, cp, Bs, GNNB_MATH_SIMT_FP32, NanDoms{nullptr, nullptr, nullptr, 0}, sg.scores, sg.best, sg.idx, nullptr, st));
+        scatter_rescored(nd.list + s0, Bs, sg.best, sg.idx, sg.scores, nh, best, idx, winners, host ? nullptr : scores, nd.flag, st,
+                         &ctx->launches);
+        if (host && scores)
+            for (int i = 0; i < Bs; ++i)
+                CU(cudaMemcpyAsync(scores + (size_t)rows[s0 + i] * nh, sg.scores + (size_t)i * nh, (size_t)nh * sizeof(float),
+                                   cudaMemcpyDeviceToHost, st));
+    }
+    CU(cudaEventRecord(ctx->ev_free[0], st));       // the next host-buffer wave that stages into set 0 waits for this pass
     CU(cudaGetLastError());
     return GNNB_OK;
 }
@@ -604,6 +704,8 @@ void gnnb_destroy(gnnb_ctx* ctx) {
     if (ctx->d_random_order) cudaFree(ctx->d_random_order);
     if (ctx->d_ptrs) cudaFree(ctx->d_ptrs);
     if (ctx->d_nan) cudaFree(ctx->d_nan);
+    if (ctx->d_resc) cudaFree(ctx->d_resc);
+    if (ctx->d_gather) cudaFree(ctx->d_gather);
     for (PropPlan* p : ctx->plan_fwd) prop_plan_free(p);
     for (PropPlan* p : ctx->plan_bwd) prop_plan_free(p);
     for (PropPlan* p : ctx->plan_kw_own) prop_plan_free(p);
@@ -798,6 +900,8 @@ int gnnb_set_option(gnnb_ctx* ctx, const char* key, int64_t value) {
         ctx->snapshot = value ? 1 : 0;
     } else if (k == "profile") {
         ctx->profile = value ? 1 : 0;
+    } else if (k == "rescore") {
+        ctx->rescore = value ? 1 : 0;
     } else {
         return fail(ctx, GNNB_ERR_INVALID, "unknown option " + k);
     }
@@ -812,6 +916,8 @@ int64_t gnnb_get_option(gnnb_ctx* ctx, const char* key) {
     if (k == "snapshot") return ctx->snapshot;
     if (k == "fuse") return ctx->fuse;
     if (k == "profile") return ctx->profile;
+    if (k == "rescore") return ctx->rescore;
+    if (k == "rescored") return ctx->rescored;
     if (k == "n_hidden") return ctx->n_hidden;
     if (k == "workspace_domains") return ctx->ws_cap;
     if (k.rfind("plan_density_pct_", 0) == 0) {      // e.g. plan_density_pct_f0 / plan_density_pct_b1
@@ -828,6 +934,7 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
     if (!ctx || !in || ((!best_score || !best_idx) && !winners)) return fail(ctx, GNNB_ERR_INVALID, "null argument");
     if (!ctx->have_gnn || !ctx->have_net) return fail(ctx, GNNB_ERR_STATE, "gnnb_set_gnn_weights and gnnb_set_network must be called first");
     if (in->B < 0) return fail(ctx, GNNB_ERR_INVALID, "negative batch");
+    ctx->rescored = 0;
     if (in->B == 0) return GNNB_OK;
     if (!in->lb || !in->ub || !in->dual || !in->prim_pre || !in->prim_post || !in->prim_out || !in->primal_input || !in->wp ||
         !in->bp || !in->mask)
@@ -845,7 +952,13 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
     // wave i + 1 (copy stream, second staging set) run under the kernels of wave i
     int chunk = ctx->chunk > 0 ? ctx->chunk : 1024;
     if (chunk > in->B) chunk = in->B;
-    TRY(ensure_workspace(ctx, chunk, host));
+    const bool resc = ctx->rescore && ctx->math == GNNB_MATH_TC_FP16X3;
+    TRY(ensure_workspace(ctx, chunk, host || resc));        // the re-score pass gathers its sub-frontier into a staging set
+    NanDoms nd{nullptr, nullptr, nullptr, 0};
+    if (resc) {
+        TRY(ensure_nan_doms(ctx, in->B));
+        nd = nan_doms(ctx);
+    }
     const std::vector<int>& n = ctx->n;
     if (host && !winners && ctx->res_cap < in->B) {
         if (ctx->res_best) cudaFree(ctx->res_best);
@@ -903,10 +1016,12 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
         float* d_best = winners ? nullptr : (host ? ctx->res_best + c0 : best_score + c0);
         int32_t* d_idx = winners ? nullptr : (host ? ctx->res_idx + c0 : best_idx + c0);
         {
-            const int rc = run_chunk(ctx, cp, Bc, d_scores, d_best, d_idx, winners ? winners + c0 : nullptr, st);
+            nd.dom0 = c0;
+            const int rc = run_chunk(ctx, cp, Bc, ctx->math, nd, d_scores, d_best, d_idx, winners ? winners + c0 : nullptr, st);
             if (rc != GNNB_OK) {      // nothing of this call may still be touching the caller's buffers or the staging sets
                 if (host) cudaStreamSynchronize(ctx->copy_stream);
                 cudaStreamSynchronize(st);
+                if (resc) reset_nan_doms(ctx, st);
                 return rc;
             }
         }
@@ -915,6 +1030,14 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
                 CU(cudaMemcpyAsync(scores + (size_t)c0 * ctx->n_hidden, d_scores, (size_t)Bc * ctx->n_hidden * sizeof(float),
                                    cudaMemcpyDeviceToHost, st));
             CU(cudaEventRecord(ctx->ev_free[wave & 1], st));
+        }
+    }
+    if (resc) {
+        const int rc = rescore_flagged(ctx, in, chunk, winners ? nullptr : (host ? ctx->res_best : best_score),
+                                       winners ? nullptr : (host ? ctx->res_idx : best_idx), winners, scores, st);
+        if (rc != GNNB_OK) {
+            reset_nan_doms(ctx, st);
+            return rc;
         }
     }
     if (host) {

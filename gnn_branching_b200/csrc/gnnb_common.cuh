@@ -102,6 +102,15 @@ struct NodeInputs {
     RowMap map;
 };
 
+// Subdomains in which the tensor-core pass of one scoring call met a NaN (option "rescore"), filled by the NaN watch of the
+// tensor-core update kernels.  Subdomain numbers are indices into the call's frontier.  flag == null: not recorded.
+struct NanDoms {
+    int32_t* count;           // [1] entries of `list`
+    int32_t* flag;            // [B] 1 once the subdomain is on the list (all 0 between calls)
+    int32_t* list;            // [B] flagged subdomains, in the order the kernels found them
+    int dom0;                 // first subdomain of the wave being scored
+};
+
 // ---- launchers (each enqueues on `st` and bumps *launches) -------------------------------------
 // SIMT fp32 node kernels (gnnb_simt.cu)
 void simt_relax(const GnnParams& g, const NodeInputs& in, float* relax_f, float* relax_b, cudaStream_t st, int64_t* launches);
@@ -121,14 +130,15 @@ void tc_relax(const GnnParams& g, const NodeInputs* in, float* const* relax_f, f
               int64_t* launches);
 void tc_update(const GnnParams& g, bool backward, const float* lb, const float* ub, const float* nb, const float* relax,
                const int32_t* amb_base, float* mu_out, float* scores, RowMap map, int64_t score_stride, int64_t score_off, int64_t rows,
-               unsigned long long* nan_count, cudaStream_t st, int64_t* launches);
+               unsigned long long* nan_count, const NanDoms& nan_doms, cudaStream_t st, int64_t* launches);
 // propagation (plan) + node update of one layer in ONE launch: the neighbour embeddings go from the propagation accumulator
 // to the update chain through tensor memory and are never written (k_tc_fused); nb_dbg: the nb tile images for snapshots, or null;
 // input_layer: the chain is the input-layer update (lb / ub = input bounds; backward, relax, amb_base, scores unused)
 struct PropPlan;
 void tc_fused(const GnnParams& g, const PropPlan* plan, const float* mu_in, bool backward, const float* lb, const float* ub,
               const float* relax, const int32_t* amb_base, float* mu_out, float* scores, RowMap map, int64_t score_stride, int64_t score_off,
-              int64_t rows, unsigned long long* nan_count, float* nb_dbg, bool input_layer, cudaStream_t st, int64_t* launches);
+              int64_t rows, unsigned long long* nan_count, const NanDoms& nan_doms, float* nb_dbg, bool input_layer, cudaStream_t st,
+              int64_t* launches);
 // slot of every ambiguous row of a layer, in row order: amb_base[tile] (+ the rank inside the tile), amb_rows[slot] = row;
 // cnt is scratch of ntiles + 1 ints (three small launches: count per tile, scan, fill)
 void amb_compact(const float* lb, const float* ub, RowMap map, int64_t rows, int32_t* cnt, int32_t* amb_base, int32_t* amb_rows,
@@ -169,6 +179,14 @@ void output_node(const GnnParams& g, const float* wp, const float* bp, const flo
 // best_score / best_idx (both or neither) and / or packed winner records
 void masked_argmax(const float* scores, const float* mask, int n_hidden, int Bc, float* best_score, int32_t* best_idx,
                    gnnb_winner* winners, cudaStream_t st, int64_t* launches);
+// re-score pass of option "rescore": one launch copies row rows[i] of every array of `tab` (floats per row = per) to row i of
+// its destination, i < n; the second writes the results of those n rows back to rows rows[i] of the call's outputs (best / idx
+// or winner records, and the dense score rows when `scores` is not null) and clears their flags
+struct RowGather { const float* src; float* dst; int64_t per; };
+void gather_rows(const RowGather* tab, int n_arrays, const int32_t* rows, int n, cudaStream_t st, int64_t* launches);
+void scatter_rescored(const int32_t* rows, int n, const float* sub_best, const int32_t* sub_idx, const float* sub_scores, int n_hidden,
+                      float* best_score, int32_t* best_idx, gnnb_winner* winners, float* scores, int32_t* flag, cudaStream_t st,
+                      int64_t* launches);
 
 // tensor-core propagation (gnnb_prop_tc.cu): block plans built once per network, gather-GEMM kernel
 struct PropPlan;

@@ -10,6 +10,7 @@
 //   prop_property_backward   nb[b,n,:] = Wp[b,n] * mu[L+1][b,:]   (graph_conv.py:324-326, rank-1)
 //   output_node    graph_conv.py:196-210
 //   masked_argmax  torch.max over the candidate rows + index mapping (graph_score.py:41-47)
+//   gather_rows / scatter_rescored   the sub-frontier of option "rescore" in, its results out
 #include <cuda_fp16.h>
 #include <math.h>
 
@@ -280,6 +281,34 @@ __global__ void __launch_bounds__(256) k_masked_argmax(const float* __restrict__
     }
 }
 
+// block (i, a): row rows[i] of array a -> row i of its destination
+__global__ void __launch_bounds__(256) k_gather_rows(const RowGather* __restrict__ tab, const int32_t* __restrict__ rows) {
+    const RowGather t = tab[blockIdx.y];
+    const float* src = t.src + (int64_t)rows[blockIdx.x] * t.per;
+    float* dst = t.dst + (int64_t)blockIdx.x * t.per;
+    for (int64_t j = threadIdx.x; j < t.per; j += blockDim.x) dst[j] = src[j];
+}
+
+// block i: the re-scored results of sub-frontier row i -> row rows[i] of the call's outputs
+__global__ void __launch_bounds__(256) k_scatter_rescored(const int32_t* __restrict__ rows, const float* __restrict__ sub_best,
+                                                          const int32_t* __restrict__ sub_idx, const float* __restrict__ sub_scores,
+                                                          int n_hidden, float* __restrict__ best_score, int32_t* __restrict__ best_idx,
+                                                          gnnb_winner* __restrict__ winners, float* __restrict__ scores,
+                                                          int32_t* __restrict__ flag) {
+    const int i = blockIdx.x;
+    const int64_t b = rows[i];
+    if (threadIdx.x == 0) {
+        if (best_score != nullptr) { best_score[b] = sub_best[i]; best_idx[b] = sub_idx[i]; }
+        if (winners != nullptr) {
+            gnnb_winner w; w.score = sub_best[i]; w.index = sub_idx[i];
+            winners[b] = w;
+        }
+        flag[b] = 0;
+    }
+    if (scores != nullptr)
+        for (int j = threadIdx.x; j < n_hidden; j += blockDim.x) scores[b * n_hidden + j] = sub_scores[(int64_t)i * n_hidden + j];
+}
+
 int capped_grid(int64_t blocks) {
     const int64_t cap = 148 * 16;
     return (int)(blocks < 1 ? 1 : (blocks < cap ? blocks : cap));
@@ -333,6 +362,18 @@ void output_node(const GnnParams& g, const float* wp, const float* bp, const flo
 void masked_argmax(const float* scores, const float* mask, int n_hidden, int Bc, float* best_score, int32_t* best_idx,
                    gnnb_winner* winners, cudaStream_t st, int64_t* launches) {
     k_masked_argmax<<<Bc, 256, 0, st>>>(scores, mask, n_hidden, best_score, best_idx, winners);
+    ++*launches;
+}
+
+void gather_rows(const RowGather* tab, int n_arrays, const int32_t* rows, int n, cudaStream_t st, int64_t* launches) {
+    k_gather_rows<<<dim3((unsigned)n, (unsigned)n_arrays), 256, 0, st>>>(tab, rows);
+    ++*launches;
+}
+
+void scatter_rescored(const int32_t* rows, int n, const float* sub_best, const int32_t* sub_idx, const float* sub_scores, int n_hidden,
+                      float* best_score, int32_t* best_idx, gnnb_winner* winners, float* scores, int32_t* flag, cudaStream_t st,
+                      int64_t* launches) {
+    k_scatter_rescored<<<n, 256, 0, st>>>(rows, sub_best, sub_idx, sub_scores, n_hidden, best_score, best_idx, winners, scores, flag);
     ++*launches;
 }
 

@@ -373,7 +373,15 @@ struct UpdArgs {
     int64_t score_stride, score_off;
     int Bc;
     unsigned long long* nan_count;
+    NanDoms nan_doms;
 };
+
+// NaN watch of a row of subdomain `dom` (of the wave): with option "rescore" the subdomain's first NaN puts it on the call's
+// list of subdomains that are scored again in exact fp32.  Rows of a tile all belong to one subdomain.
+__device__ __forceinline__ bool nan_watch(const NanDoms& nd, int dom, bool nan_row) {
+    if (nan_row && nd.flag != nullptr && atomicExch(nd.flag + nd.dom0 + dom, 1) == 0) nd.list[atomicAdd(nd.count, 1)] = nd.dom0 + dom;
+    return nan_row;
+}
 
 // One CTA's share of a node-update launch.  Work items are the propagation's: item = group of 4 subdomains x tile, taken
 // rank, rank + nranks, ...; warpgroup w updates the tile of subdomain 4 * group + w.
@@ -507,10 +515,10 @@ __device__ __forceinline__ void update_body(const UpdArgs& a, unsigned char* sme
         gemm_ts(c, W + UPD_W42, W + UPD_W42 + WPLANE, 64, DCOL);
         GNNB_TR(5);
         if (scores == nullptr) {
-            bad |= epilogue_to_mu<false>(c, DCOL, tl.bias[2], gate, nrow >= 0);
+            bad |= nan_watch(a.nan_doms, dom, epilogue_to_mu<false>(c, DCOL, tl.bias[2], gate, nrow >= 0));
             commit_tile(c, mu_out + (size_t)tile * (ABUF / 2));
         } else {      // score head on the new embeddings (graph_conv.py:448-449)
-            bad |= epilogue_to_mu<true>(c, DCOL, tl.bias[2], gate, nrow >= 0, mu_out != nullptr);
+            bad |= nan_watch(a.nan_doms, dom, epilogue_to_mu<true>(c, DCOL, tl.bias[2], gate, nrow >= 0, mu_out != nullptr));
             // mu_out == null: nothing reads these embeddings (first hidden layer on the last backward sweep: its only
             // consumer would be the input-layer update, which is dead on the last round) — the scores are all that is kept
             if (mu_out != nullptr) commit_tile(c, mu_out + (size_t)tile * (ABUF / 2));
@@ -1135,7 +1143,7 @@ __device__ __forceinline__ void fused_body(const FusedArgs& fa) {
                 gemm_ts_start(c, W + INF_B22, W + INF_B22 + WPLANE, 64, D);
                 gemm_finish(c);
                 CTR(3);
-                bad |= epilogue_to_mu_pair<false>(c, h, pair_bar, D, tl->bias[1], 1.0f, node >= 0, img, stage, advance);
+                bad |= nan_watch(a.nan_doms, dom, epilogue_to_mu_pair<false>(c, h, pair_bar, D, tl->bias[1], 1.0f, node >= 0, img, stage, advance));
                 CTR(6);
                 continue;
             }
@@ -1204,9 +1212,9 @@ __device__ __forceinline__ void fused_body(const FusedArgs& fa) {
             gemm_finish(c);
             CTR(5);
             if (!with_score) {
-                bad |= epilogue_to_mu_pair<false>(c, h, pair_bar, D, tl->bias[2], gate, node >= 0, img, stage, advance);
+                bad |= nan_watch(a.nan_doms, dom, epilogue_to_mu_pair<false>(c, h, pair_bar, D, tl->bias[2], gate, node >= 0, img, stage, advance));
             } else {      // score head on the new embeddings (graph_conv.py:448-449)
-                bad |= epilogue_to_mu_pair<true>(c, h, pair_bar, D, tl->bias[2], gate, node >= 0, img, stage);
+                bad |= nan_watch(a.nan_doms, dom, epilogue_to_mu_pair<true>(c, h, pair_bar, D, tl->bias[2], gate, node >= 0, img, stage));
                 gemm_ts_start(c, W + UPD_FN, W + UPD_FN + WPLANE, 64, D);
                 gemm_finish(c);
                 float sc = 0.f;
@@ -1636,19 +1644,21 @@ void tc_relax(const GnnParams& g, const NodeInputs* in, float* const* relax_f, f
 namespace {
 UpdArgs make_upd_args(const GnnParams& g, bool backward, const float* lb, const float* ub, const float* nb, const float* relax,
                       const int32_t* amb_base, float* mu_out, float* scores, RowMap map, int64_t score_stride, int64_t score_off,
-                      int64_t rows, unsigned long long* nan_count) {
+                      int64_t rows, unsigned long long* nan_count, const NanDoms& nan_doms) {
     UpdArgs a;
     a.g = g; a.backward = backward ? 1 : 0; a.lb = lb; a.ub = ub; a.nb_img = reinterpret_cast<const uint16_t*>(nb); a.rlx = relax;
     a.amb_base = amb_base; a.mu_out = reinterpret_cast<uint16_t*>(mu_out); a.scores = scores; a.map = map;
     a.score_stride = score_stride; a.score_off = score_off; a.Bc = (int)(rows / map.nslots); a.nan_count = nan_count;
+    a.nan_doms = nan_doms;
     return a;
 }
 }  // namespace
 
 void tc_update(const GnnParams& g, bool backward, const float* lb, const float* ub, const float* nb, const float* relax,
                const int32_t* amb_base, float* mu_out, float* scores, RowMap map, int64_t score_stride, int64_t score_off, int64_t rows,
-               unsigned long long* nan_count, cudaStream_t st, int64_t* launches) {
-    const UpdArgs a = make_upd_args(g, backward, lb, ub, nb, relax, amb_base, mu_out, scores, map, score_stride, score_off, rows, nan_count);
+               unsigned long long* nan_count, const NanDoms& nan_doms, cudaStream_t st, int64_t* launches) {
+    const UpdArgs a = make_upd_args(g, backward, lb, ub, nb, relax, amb_base, mu_out, scores, map, score_stride, score_off, rows, nan_count,
+                                    nan_doms);
     const int64_t nitems = (int64_t)(map.nslots / TILE) * ((a.Bc + NWG - 1) / NWG);
     launch_pdl(k_tc_update, (int)(nitems < 1 ? 1 : (nitems < 148 ? nitems : 148)), 128 * NWG, smem_bytes(UPD_WBYTES, true), st, a);
     ++*launches;
@@ -1656,10 +1666,12 @@ void tc_update(const GnnParams& g, bool backward, const float* lb, const float* 
 
 void tc_fused(const GnnParams& g, const PropPlan* plan, const float* mu_in, bool backward, const float* lb, const float* ub,
               const float* relax, const int32_t* amb_base, float* mu_out, float* scores, RowMap map, int64_t score_stride, int64_t score_off,
-              int64_t rows, unsigned long long* nan_count, float* nb_dbg, bool input_layer, cudaStream_t st, int64_t* launches) {
+              int64_t rows, unsigned long long* nan_count, const NanDoms& nan_doms, float* nb_dbg, bool input_layer, cudaStream_t st,
+              int64_t* launches) {
     FusedArgs fa;
     fa.input_layer = input_layer ? 1 : 0;
-    fa.u = make_upd_args(g, backward, lb, ub, nullptr, relax, amb_base, mu_out, scores, map, score_stride, score_off, rows, nan_count);
+    fa.u = make_upd_args(g, backward, lb, ub, nullptr, relax, amb_base, mu_out, scores, map, score_stride, score_off, rows, nan_count,
+                         nan_doms);
     fa.plan = prop_plan_dev(plan);
     fa.mu_in = reinterpret_cast<const uint16_t*>(mu_in);
     fa.nb_dbg = reinterpret_cast<uint16_t*>(nb_dbg);

@@ -27,7 +27,8 @@ __host__ __device__ inline uint32_t swz(uint32_t row, uint32_t chunk) {
 // scores only ~1.5x inside the 1e-4 parity bound).  fp16's narrow exponent is handled by keeping every activation
 // operand scaled by ASCALE: ReLU and the linears are positively homogeneous, so the whole chain runs in the scaled
 // domain with pre-scaled biases, and results are multiplied by AINV when they leave for global memory.
-// |activation| >= 65504 / ASCALE = 524 288 overflows to inf -> NaN -> GNNB_ERR_NAN (never silent).
+// |activation| >= 65504 / ASCALE = 524 288 overflows to inf -> NaN -> GNNB_ERR_NAN (never silent), or, with option "rescore",
+// the subdomain is scored again in exact fp32 (gnnb_api.cu rescore_flagged).
 constexpr float ASCALE = 0.125f;
 constexpr float AINV = 8.0f;
 

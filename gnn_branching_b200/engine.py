@@ -26,9 +26,12 @@ _LIN_OUT = [64] * 25 + [1]
 
 
 class Scorer:
-    """One libgnnb context bound to one CUDA device."""
+    """One libgnnb context bound to one CUDA device.
 
-    def __init__(self, device: int = 0, math: Optional[str] = None, chunk: int = 0):
+    ``rescore``: in tensor-core mode, score the subdomains whose activations left the fp16 operand range (a NaN in an
+    embedding) again in exact fp32 on the same GPU instead of failing the call (option "rescore" of include/gnnb.h)."""
+
+    def __init__(self, device: int = 0, math: Optional[str] = None, chunk: int = 0, rescore: bool = False):
         if not torch.cuda.is_available():
             raise RuntimeError('gnn_branching_b200 needs a CUDA device (sm_100a); there is no CPU path')
         self.lib = _lib.load()
@@ -45,6 +48,8 @@ class Scorer:
             self.set_option('math', _MATH[math])
         if chunk:
             self.set_option('chunk', chunk)
+        if rescore:
+            self.set_option('rescore', 1)
 
     def __del__(self):
         h, self.h = getattr(self, 'h', None), None
@@ -73,6 +78,11 @@ class Scorer:
     @property
     def launches(self) -> int:
         return int(self.lib.gnnb_launch_count(self.h))
+
+    @property
+    def rescored(self) -> int:
+        """Subdomains the last scoring call scored again in exact fp32 (option ``rescore``)."""
+        return self.get_option('rescored')
 
     # ---- parameters ----
     def set_gnn(self, state_dict: Dict[str, torch.Tensor], T: int = 2, p: int = 64, key=None, force: bool = False):

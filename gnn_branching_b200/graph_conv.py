@@ -66,14 +66,14 @@ class ComputeFinalScore(nn.Module):
 class GraphNet(nn.Module):
     """Drop-in for graphnet.graph_conv.GraphNet (graph_conv.py:473-483)."""
 
-    def __init__(self, T, p, math: Optional[str] = None, chunk: int = 0):
+    def __init__(self, T, p, math: Optional[str] = None, chunk: int = 0, rescore: bool = False):
         super().__init__()
         if p != 64:
             raise NotImplementedError('the CUDA kernels are specialised for p = 64 (graph_score.py:9)')
         self.T, self.p = T, p
         self.EmbedUpdates = EmbedUpdates(T, p)
         self.ComputeFinalScore = ComputeFinalScore(p)
-        self._math, self._chunk = math, chunk
+        self._math, self._chunk, self._rescore = math, chunk, rescore
         self._scorer: Optional[Scorer] = None
 
     # ---- engine plumbing ----
@@ -82,7 +82,7 @@ class GraphNet(nn.Module):
             q = next(self.parameters())
             device_index = q.device.index if q.device.type == 'cuda' else torch.cuda.current_device()
         if self._scorer is None or self._scorer.device != device_index:
-            self._scorer = Scorer(device_index, math=self._math, chunk=self._chunk)
+            self._scorer = Scorer(device_index, math=self._math, chunk=self._chunk, rescore=self._rescore)
         key = tuple((q.data_ptr(), q._version) for q in self.parameters())
         if self._scorer._gnn_key != key:          # state_dict() costs ~0.2 ms: only when a parameter changed
             self._scorer.set_gnn(self.state_dict(), self.T, self.p, key=key)

@@ -18,8 +18,8 @@ class GraphChoice:
     """
     verbose = False     # the reference prints 'graph requires: <s>' on every call (graph_score.py:36)
 
-    def __init__(self, init_mask, model_name, linear=False, math=None):
-        model = GraphNet(2, 64, math=math)                          # graph_score.py:9
+    def __init__(self, init_mask, model_name, linear=False, math=None, rescore=False):
+        model = GraphNet(2, 64, math=math, rescore=rescore)         # graph_score.py:9
         model.load_state_dict(torch.load(model_name, map_location='cpu'))
         model.eval()
         self.model = model.cuda()

@@ -27,7 +27,9 @@ enum gnnb_status {
     GNNB_ERR_CUDA = 2,         /* a CUDA runtime call failed (message in gnnb_last_error) */
     GNNB_ERR_STATE = 3,        /* weights or network not set */
     GNNB_ERR_NAN = 4,          /* NaN appeared in an embedding: the reference stops in pdb here
-                                  (graphnet/graph_conv.py:184-186, 339-341); outputs are still written */
+                                  (graphnet/graph_conv.py:184-186, 339-341); outputs are still written.  In tensor-core mode
+                                  this includes activations beyond the fp16 operand range (|x| >= 524 288), unless option
+                                  "rescore" scores those subdomains again in exact fp32 */
     GNNB_ERR_UNSUPPORTED = 5
 };
 
@@ -108,8 +110,16 @@ int gnnb_set_network(gnnb_ctx* ctx, const gnnb_layer_desc* layers, int n_layers,
 /* Options: "math" (gnnb_math_mode), "chunk" (subdomains per wave; 0 = auto), "fuse" (0/1, default 1: propagation and
  * node update of a layer in one launch, tensor-core mode; 0 = two launches), "snapshot" (0/1: keep per-stage copies
  * for gnnb_debug_snapshot; debugging only), "profile" (0/1: time every stage launch with CUDA events for
- * gnnb_profile_read).  Any other key of gnnb_set_option fails with GNNB_ERR_INVALID.
- * gnnb_get_option also reads these, and "n_hidden" (hidden ReLUs of the network), "workspace_domains" (subdomains the
+ * gnnb_profile_read), "rescore" (0/1, default 0; see below).  Any other key of gnnb_set_option fails with GNNB_ERR_INVALID.
+ * "rescore" = 1, tensor-core mode: gnnb_score and gnnb_score_winners record every subdomain in which the tensor-core pass met
+ * a NaN (activations beyond the fp16 operand range, |x| >= 524 288), score those subdomains again with the exact-fp32 SIMT
+ * schedule on the same GPU and write their results (best score and index or winner record, dense scores) over the tensor-core
+ * ones; every other subdomain keeps its tensor-core result bit for bit.  Cost on a frontier without such subdomains: one 4-byte
+ * device -> host copy and one synchronise of `stream` per call, also with DEVICE buffers (no extra launch or allocation).
+ * The NaN count is reset before the fp32 pass, so GNNB_ERR_NAN (returned for HOST calls, through gnnb_check for DEVICE calls)
+ * then reports only NaN that exact fp32 gives too.  The option does nothing in SIMT mode; snapshots keep the tensor-core pass.
+ * gnnb_get_option also reads these, "rescored" (subdomains the last scoring call scored again), and "n_hidden" (hidden ReLUs of
+ * the network), "workspace_domains" (subdomains the
  * workspace holds) and "plan_density_pct_f<k>" / "plan_density_pct_b<k>" (percentage of the MACs issued by forward /
  * backward propagation plan k that are useful); it returns -1 for an unknown key. */
 int gnnb_set_option(gnnb_ctx* ctx, const char* key, int64_t value);
