@@ -11,11 +11,12 @@ GNNB_OK, GNNB_ERR_INVALID, GNNB_ERR_CUDA, GNNB_ERR_STATE, GNNB_ERR_NAN, GNNB_ERR
 LAYER_CONV, LAYER_LINEAR = 0, 1
 MEM_DEVICE, MEM_HOST = 0, 1
 MATH_TC_FP16X3, MATH_SIMT_FP32 = 0, 1
+TOPK_MAX = 64                                      # GNNB_TOPK_MAX
 KERNEL_CLASSES = ['relax', 'update_fwd', 'update_bwd', 'update_bwd_score', 'input_embed', 'input_update', 'prop_fwd',
                   'prop_bwd', 'output', 'argmax', 'layer_fwd', 'layer_bwd', 'layer_bwd_score']
 
 EXPORTS = ['gnnb_create', 'gnnb_destroy', 'gnnb_set_gnn_weights', 'gnnb_set_network', 'gnnb_set_option',
-           'gnnb_get_option', 'gnnb_score', 'gnnb_score_winners', 'gnnb_check', 'gnnb_launch_count', 'gnnb_last_error',
+           'gnnb_get_option', 'gnnb_score', 'gnnb_score_winners', 'gnnb_score_topk', 'gnnb_topk', 'gnnb_check', 'gnnb_launch_count', 'gnnb_last_error',
            'gnnb_debug_snapshot', 'gnnb_abi_version', 'gnnb_profile_read', 'gnnb_profile_reset', 'gnnb_babsr',
            'gnnb_score_grad', 'gnnb_get_gradients', 'gnnb_get_gnn_weights', 'gnnb_adam_step', 'gnnb_adam_reset',
            'gnnb_kw_bounds', 'gnnb_child_bounds', 'gnnb_root_bounds', 'gnnb_queue_create', 'gnnb_queue_destroy', 'gnnb_queue_add', 'gnnb_queue_pick', 'gnnb_queue_prune', 'gnnb_queue_stats']
@@ -73,6 +74,8 @@ def load() -> C.CDLL:
     lib.gnnb_score.argtypes = [vp, C.POINTER(FrontierDesc), _fp, C.POINTER(C.c_int32), _fp, vp]
     lib.gnnb_score_winners.argtypes = [vp, C.POINTER(FrontierDesc), vp, _fp, vp]
     _ip = C.POINTER(C.c_int32)
+    lib.gnnb_score_topk.argtypes = [vp, C.POINTER(FrontierDesc), C.c_int32, _fp, _ip, _fp, vp]
+    lib.gnnb_topk.argtypes = [vp, C.c_int32, C.c_int32, _fp, _fp, C.c_int32, _fp, _ip, vp]
     lib.gnnb_babsr.argtypes = [vp, C.POINTER(FrontierDesc), C.c_int32, C.c_float, _ip, _ip, _ip, _ip, _ip, _fp, vp]
     lib.gnnb_score_grad.argtypes = [vp, C.POINTER(FrontierDesc), C.c_int32, _ip, _ip, _fp, _fp, vp]
     lib.gnnb_get_gradients.argtypes = [vp, _fpp, C.POINTER(C.c_int64), C.c_int]

@@ -92,7 +92,7 @@ struct gnnb_ctx {
     } stg[2];
     float* res_best = nullptr;      // winners of a whole host-buffer call (one device->host copy at the end, so that a
     int32_t* res_idx = nullptr;     // pageable result buffer cannot stall the wave pipeline)
-    int res_cap = 0;
+    int64_t res_cap = 0;            // entries (subdomains x k)
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr};
     unsigned long long* d_nan = nullptr;
@@ -180,7 +180,8 @@ int ensure_workspace(gnnb_ctx* ctx, int Bc, bool host_staging) {
             }
             o.pout = take(Bc); o.pin = take((size_t)Bc * ctx->n[0]); o.wp = take((size_t)Bc * ctx->n[L]);
             o.bp = take(Bc); o.mask = take((size_t)Bc * ctx->n_hidden);
-            o.best = take(Bc); o.idx = take(Bc); o.sc = take((size_t)Bc * ctx->n_hidden);
+            o.best = take((size_t)Bc * GNNB_TOPK_MAX); o.idx = take((size_t)Bc * GNNB_TOPK_MAX);   // k results per row (re-score pass)
+            o.sc = take((size_t)Bc * ctx->n_hidden);
         }
     }
     CU(cudaMalloc(&ctx->d_ws, total * sizeof(float)));
@@ -289,9 +290,9 @@ struct ChunkPtrs {
 #define TRY(expr) do { int s__ = (expr); if (s__ != GNNB_OK) return s__; } while (0)
 
 // the stage schedule for one chunk in arithmetic `math`; every pointer is a device pointer; nd: where the tensor-core NaN watch
-// records the subdomains it flags (nd.flag = null: nowhere)
-int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, int math, const NanDoms& nd, float* scores, float* best_score, int32_t* best_idx,
-              gnnb_winner* winners, cudaStream_t st) {
+// records the subdomains it flags (nd.flag = null: nowhere); best_score / best_idx: [Bc, k], the k best candidates per subdomain
+int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, int math, const NanDoms& nd, float* scores, int k, float* best_score,
+              int32_t* best_idx, gnnb_winner* winners, cudaStream_t st) {
     const int L = (int)ctx->layers.size();
     const GnnParams& g = ctx->gp;
     const bool tc = math == GNNB_MATH_TC_FP16X3;
@@ -428,7 +429,8 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, int math, const NanDom
     }
     {
         ProfScope ps(ctx, GNNB_K_ARGMAX, Bc, st);
-        masked_argmax(scores, in.mask, ctx->n_hidden, Bc, best_score, best_idx, winners, st, lc);
+        if (k == 1) masked_argmax(scores, in.mask, ctx->n_hidden, Bc, best_score, best_idx, winners, st, lc);
+        else masked_topk(scores, in.mask, ctx->n_hidden, Bc, k, best_score, best_idx, st, lc);
     }
     CU(cudaGetLastError());
     return GNNB_OK;
@@ -454,11 +456,11 @@ void reset_nan_doms(gnnb_ctx* ctx, cudaStream_t st) {
 
 // Option "rescore", after the tensor-core pass of a call: read how many subdomains its NaN watch flagged (one device -> host copy
 // and one synchronise of `st`; nothing else when there are none), then score those again with the exact-fp32 schedule, in waves
-// of up to `chunk` gathered into staging set 0, and write their results over the tensor-core ones.  best / idx or winners:
+// of up to `chunk` gathered into staging set 0, and write their results over the tensor-core ones.  best / idx [B, k] or winners:
 // device arrays of the whole call; scores: the caller's dense scores (in->mem) or null.  The NaN count is reset first, so that
 // afterwards it counts the fp32 pass only.
-int rescore_flagged(gnnb_ctx* ctx, const gnnb_frontier* in, int chunk, float* best, int32_t* idx, gnnb_winner* winners, float* scores,
-                    cudaStream_t st) {
+int rescore_flagged(gnnb_ctx* ctx, const gnnb_frontier* in, int chunk, int k, float* best, int32_t* idx, gnnb_winner* winners,
+                    float* scores, cudaStream_t st) {
     const bool host = in->mem == GNNB_MEM_HOST;
     const int L = (int)ctx->layers.size(), nh = ctx->n_hidden;
     const std::vector<int>& n = ctx->n;
@@ -511,8 +513,8 @@ int rescore_flagged(gnnb_ctx* ctx, const gnnb_frontier* in, int chunk, float* be
         } else {
             gather_rows(ctx->d_gather, (int)tab.size(), nd.list + s0, Bs, st, &ctx->launches);
         }
-        TRY(run_chunk(ctx, cp, Bs, GNNB_MATH_SIMT_FP32, NanDoms{nullptr, nullptr, nullptr, 0}, sg.scores, sg.best, sg.idx, nullptr, st));
-        scatter_rescored(nd.list + s0, Bs, sg.best, sg.idx, sg.scores, nh, best, idx, winners, host ? nullptr : scores, nd.flag, st,
+        TRY(run_chunk(ctx, cp, Bs, GNNB_MATH_SIMT_FP32, NanDoms{nullptr, nullptr, nullptr, 0}, sg.scores, k, sg.best, sg.idx, nullptr, st));
+        scatter_rescored(nd.list + s0, Bs, k, sg.best, sg.idx, sg.scores, nh, best, idx, winners, host ? nullptr : scores, nd.flag, st,
                          &ctx->launches);
         if (host && scores)
             for (int i = 0; i < Bs; ++i)
@@ -929,8 +931,9 @@ int64_t gnnb_get_option(gnnb_ctx* ctx, const char* key) {
     return -1;
 }
 
-static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score, int32_t* best_idx, gnnb_winner* winners, float* scores,
-                      void* stream) {
+// best_score / best_idx: [B, k] (k = 1: gnnb_score), or winner records (k = 1)
+static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, int k, float* best_score, int32_t* best_idx, gnnb_winner* winners,
+                      float* scores, void* stream) {
     if (!ctx || !in || ((!best_score || !best_idx) && !winners)) return fail(ctx, GNNB_ERR_INVALID, "null argument");
     if (!ctx->have_gnn || !ctx->have_net) return fail(ctx, GNNB_ERR_STATE, "gnnb_set_gnn_weights and gnnb_set_network must be called first");
     if (in->B < 0) return fail(ctx, GNNB_ERR_INVALID, "negative batch");
@@ -960,13 +963,14 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
         nd = nan_doms(ctx);
     }
     const std::vector<int>& n = ctx->n;
-    if (host && !winners && ctx->res_cap < in->B) {
+    const int64_t n_res = (int64_t)in->B * k;
+    if (host && !winners && ctx->res_cap < n_res) {
         if (ctx->res_best) cudaFree(ctx->res_best);
         if (ctx->res_idx) cudaFree(ctx->res_idx);
         ctx->res_best = nullptr; ctx->res_idx = nullptr; ctx->res_cap = 0;
-        CU(cudaMalloc(&ctx->res_best, (size_t)in->B * sizeof(float)));
-        CU(cudaMalloc(&ctx->res_idx, (size_t)in->B * sizeof(int32_t)));
-        ctx->res_cap = in->B;
+        CU(cudaMalloc(&ctx->res_best, (size_t)n_res * sizeof(float)));
+        CU(cudaMalloc(&ctx->res_idx, (size_t)n_res * sizeof(int32_t)));
+        ctx->res_cap = n_res;
     }
 
     // host buffers: the first wave is small so that the kernels start after a short copy; a later wave's copy (copy stream, the
@@ -1013,11 +1017,11 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
         }
 
         float* d_scores = host ? sg.scores : (scores ? scores + (size_t)c0 * ctx->n_hidden : ctx->ws_scores);
-        float* d_best = winners ? nullptr : (host ? ctx->res_best + c0 : best_score + c0);
-        int32_t* d_idx = winners ? nullptr : (host ? ctx->res_idx + c0 : best_idx + c0);
+        float* d_best = winners ? nullptr : (host ? ctx->res_best : best_score) + (size_t)c0 * k;
+        int32_t* d_idx = winners ? nullptr : (host ? ctx->res_idx : best_idx) + (size_t)c0 * k;
         {
             nd.dom0 = c0;
-            const int rc = run_chunk(ctx, cp, Bc, ctx->math, nd, d_scores, d_best, d_idx, winners ? winners + c0 : nullptr, st);
+            const int rc = run_chunk(ctx, cp, Bc, ctx->math, nd, d_scores, k, d_best, d_idx, winners ? winners + c0 : nullptr, st);
             if (rc != GNNB_OK) {      // nothing of this call may still be touching the caller's buffers or the staging sets
                 if (host) cudaStreamSynchronize(ctx->copy_stream);
                 cudaStreamSynchronize(st);
@@ -1033,7 +1037,7 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
         }
     }
     if (resc) {
-        const int rc = rescore_flagged(ctx, in, chunk, winners ? nullptr : (host ? ctx->res_best : best_score),
+        const int rc = rescore_flagged(ctx, in, chunk, k, winners ? nullptr : (host ? ctx->res_best : best_score),
                                        winners ? nullptr : (host ? ctx->res_idx : best_idx), winners, scores, st);
         if (rc != GNNB_OK) {
             reset_nan_doms(ctx, st);
@@ -1042,8 +1046,8 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
     }
     if (host) {
         if (!winners) {
-            CU(cudaMemcpyAsync(best_score, ctx->res_best, (size_t)in->B * sizeof(float), cudaMemcpyDeviceToHost, st));
-            CU(cudaMemcpyAsync(best_idx, ctx->res_idx, (size_t)in->B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(best_score, ctx->res_best, (size_t)n_res * sizeof(float), cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(best_idx, ctx->res_idx, (size_t)n_res * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         }
         return gnnb_check(ctx, stream, nullptr);
     }
@@ -1052,13 +1056,36 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score,
 
 int gnnb_score(gnnb_ctx* ctx, const gnnb_frontier* in, float* best_score, int32_t* best_idx, float* scores, void* stream) {
     if (!best_score || !best_idx) return fail(ctx, GNNB_ERR_INVALID, "null argument");
-    return score_impl(ctx, in, best_score, best_idx, nullptr, scores, stream);
+    return score_impl(ctx, in, 1, best_score, best_idx, nullptr, scores, stream);
 }
 
 int gnnb_score_winners(gnnb_ctx* ctx, const gnnb_frontier* in, gnnb_winner* winners, float* scores, void* stream) {
     if (!winners) return fail(ctx, GNNB_ERR_INVALID, "null argument");
     if (in && in->mem == GNNB_MEM_HOST && scores) return fail(ctx, GNNB_ERR_INVALID, "dense scores of a HOST frontier: use gnnb_score");
-    return score_impl(ctx, in, nullptr, nullptr, winners, scores, stream);
+    return score_impl(ctx, in, 1, nullptr, nullptr, winners, scores, stream);
+}
+
+int gnnb_score_topk(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t k, float* top_score, int32_t* top_idx, float* scores, void* stream) {
+    if (k < 1 || k > GNNB_TOPK_MAX) return fail(ctx, GNNB_ERR_INVALID, "k must be in [1, GNNB_TOPK_MAX]");
+    if (!top_score || !top_idx) return fail(ctx, GNNB_ERR_INVALID, "null argument");
+    return score_impl(ctx, in, k, top_score, top_idx, nullptr, scores, stream);
+}
+
+int gnnb_topk(gnnb_ctx* ctx, int32_t B, int32_t n, const float* scores, const float* mask, int32_t k, float* top_score,
+              int32_t* top_idx, void* stream) {
+    if (!ctx) return GNNB_ERR_INVALID;
+    if (k < 1 || k > GNNB_TOPK_MAX) return fail(ctx, GNNB_ERR_INVALID, "k must be in [1, GNNB_TOPK_MAX]");
+    if (!scores || !top_score || !top_idx) return fail(ctx, GNNB_ERR_INVALID, "null argument");
+    if (B < 0 || n < 0) return fail(ctx, GNNB_ERR_INVALID, "negative size");
+    if (B == 0) return GNNB_OK;
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    {
+        ProfScope ps(ctx, GNNB_K_ARGMAX, B, st);
+        masked_topk(scores, mask, n, B, k, top_score, top_idx, st, &ctx->launches);
+    }
+    CU(cudaGetLastError());
+    return GNNB_OK;
 }
 
 int gnnb_babsr(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t sparsest_layer, float decision_threshold,

@@ -179,14 +179,18 @@ void output_node(const GnnParams& g, const float* wp, const float* bp, const flo
 // best_score / best_idx (both or neither) and / or packed winner records
 void masked_argmax(const float* scores, const float* mask, int n_hidden, int Bc, float* best_score, int32_t* best_idx,
                    gnnb_winner* winners, cudaStream_t st, int64_t* launches);
+// the k best candidates of every row of scores [Bc, n] (mask [Bc, n] or null = all), 1 <= k <= GNNB_TOPK_MAX, in the order of
+// masked_argmax extended to k (NaN first, then descending, ties by ascending index); top_score / top_idx [Bc, k]
+void masked_topk(const float* scores, const float* mask, int n, int Bc, int k, float* top_score, int32_t* top_idx, cudaStream_t st,
+                 int64_t* launches);
 // re-score pass of option "rescore": one launch copies row rows[i] of every array of `tab` (floats per row = per) to row i of
-// its destination, i < n; the second writes the results of those n rows back to rows rows[i] of the call's outputs (best / idx
-// or winner records, and the dense score rows when `scores` is not null) and clears their flags
+// its destination, i < n; the second writes the results of those n rows back to rows rows[i] of the call's outputs (k best
+// scores / indices per row or winner records, and the dense score rows when `scores` is not null) and clears their flags
 struct RowGather { const float* src; float* dst; int64_t per; };
 void gather_rows(const RowGather* tab, int n_arrays, const int32_t* rows, int n, cudaStream_t st, int64_t* launches);
-void scatter_rescored(const int32_t* rows, int n, const float* sub_best, const int32_t* sub_idx, const float* sub_scores, int n_hidden,
-                      float* best_score, int32_t* best_idx, gnnb_winner* winners, float* scores, int32_t* flag, cudaStream_t st,
-                      int64_t* launches);
+void scatter_rescored(const int32_t* rows, int n, int k, const float* sub_best, const int32_t* sub_idx, const float* sub_scores,
+                      int n_hidden, float* best_score, int32_t* best_idx, gnnb_winner* winners, float* scores, int32_t* flag,
+                      cudaStream_t st, int64_t* launches);
 
 // tensor-core propagation (gnnb_prop_tc.cu): block plans built once per network, gather-GEMM kernel
 struct PropPlan;

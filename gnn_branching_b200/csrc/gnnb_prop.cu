@@ -10,6 +10,7 @@
 //   prop_property_backward   nb[b,n,:] = Wp[b,n] * mu[L+1][b,:]   (graph_conv.py:324-326, rank-1)
 //   output_node    graph_conv.py:196-210
 //   masked_argmax  torch.max over the candidate rows + index mapping (graph_score.py:41-47)
+//   masked_topk    the k best candidates per row in the argmax's order (radix select + bitonic sort of at most 64 entries)
 //   gather_rows / scatter_rescored   the sub-frontier of option "rescore" in, its results out
 #include <cuda_fp16.h>
 #include <math.h>
@@ -281,6 +282,138 @@ __global__ void __launch_bounds__(256) k_masked_argmax(const float* __restrict__
     }
 }
 
+// Order-preserving key of a candidate's score: a larger key comes first in the order of better().  Every NaN maps above +inf
+// (NaN first, and NaN ties go by index), -0.0 maps to the key of +0.0 (better() compares with a > b).  0 is no float's key
+// (the smallest, -inf, is 0x007fffff) and marks an entry that is not a candidate.
+__device__ __forceinline__ uint32_t topk_key(float s, float m) {
+    if (m == 0.f) return 0u;
+    if (s != s) return 0xffffffffu;
+    const uint32_t u = s == 0.f ? 0u : __float_as_uint(s);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+constexpr int TOPK_BT = 256;             // threads per block; the 256 histogram bins are one per thread
+constexpr int TOPK_SMEM_KEYS = 11264;    // rows up to this length keep their keys in shared memory (44 KB): the row is read once
+
+// one block per row: the k best candidates, ordered by (key descending, index ascending); (-inf, -1) past the last candidate.
+// 1. radix select with 8-bit digits (four histogram passes) finds T, the key of the kk-th candidate, kk = min(k, candidates),
+//    and how many candidates with key T belong to the top kk;
+// 2. one pass in index order takes every candidate above T and the first of those equal to T (ballot + block prefix count);
+// 3. a bitonic sort orders the at most 64 taken entries.
+// Histogram counts are integers and the sort sees a set of distinct (key, index) pairs: no result depends on the order of the
+// atomics or on the block size.
+__global__ void __launch_bounds__(TOPK_BT) k_masked_topk(const float* __restrict__ scores, const float* __restrict__ mask, int n,
+                                                         int k, float* __restrict__ top_score, int32_t* __restrict__ top_idx) {
+    extern __shared__ uint32_t skey[];                    // [n] when n <= TOPK_SMEM_KEYS
+    __shared__ uint32_t hist[256];
+    __shared__ uint32_t sel_key[GNNB_TOPK_MAX];
+    __shared__ int sel_idx[GNNB_TOPK_MAX];
+    __shared__ int wcnt[TOPK_BT / 32];
+    __shared__ uint32_t s_prefix, s_rem, s_kk;
+    __shared__ int s_above;
+    const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const float* s = scores + (int64_t)b * n;
+    const float* m = mask ? mask + (int64_t)b * n : nullptr;
+    const bool cached = n <= TOPK_SMEM_KEYS;
+    auto key_at = [&](int i) { return cached ? skey[i] : topk_key(s[i], m ? m[i] : 1.f); };
+    if (cached)
+        for (int i = t; i < n; i += TOPK_BT) skey[i] = topk_key(s[i], m ? m[i] : 1.f);
+
+    uint32_t prefix = 0u, pmask = 0u, rem = 0u;
+    for (int shift = 24; shift >= 0; shift -= 8) {
+        hist[t] = 0u;
+        __syncthreads();
+        for (int i = t; i < n; i += TOPK_BT) {
+            const uint32_t key = key_at(i);
+            if (key != 0u && (key & pmask) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1u);
+        }
+        __syncthreads();
+        if (warp == 0) {                                  // lane l holds digits 255 - 8 l - j, j = 0..7: descending digit order
+            uint32_t c[8], sum = 0u;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) { c[j] = hist[255 - 8 * lane - j]; sum += c[j]; }
+            uint32_t incl = sum;
+#pragma unroll
+            for (int off = 1; off < 32; off <<= 1) {
+                const uint32_t v = __shfl_up_sync(0xffffffffu, incl, off);
+                if (lane >= off) incl += v;
+            }
+            uint32_t r = rem;
+            if (shift == 24) {                            // the first pass counts every candidate
+                const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+                r = total < (uint32_t)k ? total : (uint32_t)k;
+                if (lane == 0) s_kk = r;
+            }
+            const uint32_t excl = incl - sum;
+            if (r > 0u && excl < r && r <= incl) {        // the digit of the r-th largest key lies in this lane's bins
+                uint32_t acc = excl;
+                int j = -1;
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj)           // unrolled: c stays in registers
+                    if (j < 0) { if (acc + c[jj] >= r) j = jj; else acc += c[jj]; }
+                s_prefix = prefix | ((uint32_t)(255 - 8 * lane - j) << shift);
+                s_rem = r - acc;
+            }
+        }
+        __syncthreads();
+        if (s_kk == 0u) break;
+        prefix = s_prefix;
+        rem = s_rem;
+        pmask |= 255u << shift;
+    }
+    const int kk = (int)s_kk;
+    if (kk > 0) {
+        const uint32_t T = prefix;
+        const int need_eq = (int)rem, above = kk - (int)rem;
+        if (t == 0) s_above = 0;
+        __syncthreads();
+        int eq_run = 0;
+        for (int base = 0; base < n; base += TOPK_BT) {
+            const int i = base + t;
+            const uint32_t key = i < n ? key_at(i) : 0u;
+            if (key > T) {
+                const int slot = atomicAdd(&s_above, 1);
+                sel_key[slot] = key; sel_idx[slot] = i;
+            }
+            const unsigned bal = __ballot_sync(0xffffffffu, key == T);
+            if (lane == 0) wcnt[warp] = __popc(bal);
+            __syncthreads();
+            int pos = eq_run + __popc(bal & ((1u << lane) - 1u)), tile = 0;
+#pragma unroll
+            for (int w = 0; w < TOPK_BT / 32; ++w) { const int c = wcnt[w]; if (w < warp) pos += c; tile += c; }
+            if (key == T && pos < need_eq) { sel_key[above + pos] = key; sel_idx[above + pos] = i; }
+            eq_run += tile;
+            const bool done = eq_run >= need_eq && s_above == above;
+            __syncthreads();
+            if (done) break;
+        }
+        if (t < GNNB_TOPK_MAX && t >= kk) { sel_key[t] = 0u; sel_idx[t] = 0x7fffffff; }     // padding sorts last
+        __syncthreads();
+        for (int size = 2; size <= GNNB_TOPK_MAX; size <<= 1)
+            for (int stride = size >> 1; stride > 0; stride >>= 1) {
+                if (t < GNNB_TOPK_MAX) {
+                    const int p = t ^ stride;
+                    if (p > t) {
+                        const uint32_t ka = sel_key[t], kb = sel_key[p];
+                        const int ia = sel_idx[t], ib = sel_idx[p];
+                        const bool p_first = kb > ka || (kb == ka && ib < ia);
+                        if (p_first == ((t & size) == 0)) {
+                            sel_key[t] = kb; sel_key[p] = ka; sel_idx[t] = ib; sel_idx[p] = ia;
+                        }
+                    }
+                }
+                __syncthreads();
+            }
+    }
+    for (int j = t; j < k; j += TOPK_BT) {
+        float v = -INFINITY;
+        int ix = -1;
+        if (j < kk) { ix = sel_idx[j]; v = s[ix]; }       // the score's own bits (-0.0 stays -0.0)
+        top_score[(int64_t)b * k + j] = v;
+        top_idx[(int64_t)b * k + j] = ix;
+    }
+}
+
 // block (i, a): row rows[i] of array a -> row i of its destination
 __global__ void __launch_bounds__(256) k_gather_rows(const RowGather* __restrict__ tab, const int32_t* __restrict__ rows) {
     const RowGather t = tab[blockIdx.y];
@@ -289,16 +422,19 @@ __global__ void __launch_bounds__(256) k_gather_rows(const RowGather* __restrict
     for (int64_t j = threadIdx.x; j < t.per; j += blockDim.x) dst[j] = src[j];
 }
 
-// block i: the re-scored results of sub-frontier row i -> row rows[i] of the call's outputs
-__global__ void __launch_bounds__(256) k_scatter_rescored(const int32_t* __restrict__ rows, const float* __restrict__ sub_best,
+// block i: the re-scored results of sub-frontier row i (k entries) -> row rows[i] of the call's outputs
+__global__ void __launch_bounds__(256) k_scatter_rescored(const int32_t* __restrict__ rows, int k, const float* __restrict__ sub_best,
                                                           const int32_t* __restrict__ sub_idx, const float* __restrict__ sub_scores,
                                                           int n_hidden, float* __restrict__ best_score, int32_t* __restrict__ best_idx,
                                                           gnnb_winner* __restrict__ winners, float* __restrict__ scores,
                                                           int32_t* __restrict__ flag) {
     const int i = blockIdx.x;
     const int64_t b = rows[i];
+    if (best_score != nullptr && threadIdx.x < k) {
+        best_score[b * k + threadIdx.x] = sub_best[(int64_t)i * k + threadIdx.x];
+        best_idx[b * k + threadIdx.x] = sub_idx[(int64_t)i * k + threadIdx.x];
+    }
     if (threadIdx.x == 0) {
-        if (best_score != nullptr) { best_score[b] = sub_best[i]; best_idx[b] = sub_idx[i]; }
         if (winners != nullptr) {
             gnnb_winner w; w.score = sub_best[i]; w.index = sub_idx[i];
             winners[b] = w;
@@ -365,15 +501,22 @@ void masked_argmax(const float* scores, const float* mask, int n_hidden, int Bc,
     ++*launches;
 }
 
+void masked_topk(const float* scores, const float* mask, int n, int Bc, int k, float* top_score, int32_t* top_idx, cudaStream_t st,
+                 int64_t* launches) {
+    const size_t smem = n <= TOPK_SMEM_KEYS ? (size_t)n * sizeof(uint32_t) : 0;
+    k_masked_topk<<<Bc, TOPK_BT, smem, st>>>(scores, mask, n, k, top_score, top_idx);
+    ++*launches;
+}
+
 void gather_rows(const RowGather* tab, int n_arrays, const int32_t* rows, int n, cudaStream_t st, int64_t* launches) {
     k_gather_rows<<<dim3((unsigned)n, (unsigned)n_arrays), 256, 0, st>>>(tab, rows);
     ++*launches;
 }
 
-void scatter_rescored(const int32_t* rows, int n, const float* sub_best, const int32_t* sub_idx, const float* sub_scores, int n_hidden,
-                      float* best_score, int32_t* best_idx, gnnb_winner* winners, float* scores, int32_t* flag, cudaStream_t st,
-                      int64_t* launches) {
-    k_scatter_rescored<<<n, 256, 0, st>>>(rows, sub_best, sub_idx, sub_scores, n_hidden, best_score, best_idx, winners, scores, flag);
+void scatter_rescored(const int32_t* rows, int n, int k, const float* sub_best, const int32_t* sub_idx, const float* sub_scores,
+                      int n_hidden, float* best_score, int32_t* best_idx, gnnb_winner* winners, float* scores, int32_t* flag,
+                      cudaStream_t st, int64_t* launches) {
+    k_scatter_rescored<<<n, 256, 0, st>>>(rows, k, sub_best, sub_idx, sub_scores, n_hidden, best_score, best_idx, winners, scores, flag);
     ++*launches;
 }
 

@@ -146,6 +146,43 @@ class Scorer:
         host->device and results device->host inside the call (pin the frontier for full copy speed).
         Returns (best_score [B] f32, best_idx [B] i32, scores [B, sum n_k] f32 or None).
         """
+        return self._score(fr, None, return_scores, check)
+
+    def score_topk(self, fr: Frontier, k: int, return_scores: bool = False, check: bool = True
+                   ) -> Tuple[torch.Tensor, torch.Tensor, Optional[torch.Tensor]]:
+        """Score every subdomain of ``fr`` and return its ``k`` best branching candidates (1 <= k <= 64), device and host
+        frontiers as in ``score``.  Returns (top_score [B, k] f32, top_idx [B, k] i32, scores [B, sum n_k] f32 or None).
+        Order: NaN scores first, then descending score, ties by ascending flat index; (-inf, -1) past the last candidate.
+        Column 0 is ``score``'s (best_score, best_idx) bit for bit."""
+        if not 1 <= int(k) <= _lib.TOPK_MAX:
+            raise ValueError(f'k must be in [1, {_lib.TOPK_MAX}], got {k}')
+        return self._score(fr, int(k), return_scores, check)
+
+    def topk(self, scores: torch.Tensor, k: int, mask: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """The ``k`` best entries of every row of ``scores`` [B, n] (CUDA) among those with ``mask`` != 0 (``mask`` [B, n] or
+        None = every entry), in ``score_topk``'s order: (top_score [B, k] f32, top_idx [B, k] i32), CUDA tensors."""
+        if not 1 <= int(k) <= _lib.TOPK_MAX:
+            raise ValueError(f'k must be in [1, {_lib.TOPK_MAX}], got {k}')
+        if not scores.is_cuda or scores.dim() != 2:
+            raise ValueError('scores must be a [B, n] CUDA tensor')
+        B, n = int(scores.shape[0]), int(scores.shape[1])
+        scores = self._as_f32(scores, (B, n))
+        if mask is not None:
+            if not mask.is_cuda:
+                raise ValueError('mask must be a CUDA tensor')
+            mask = self._as_f32(mask, (B, n))
+        top_score = torch.empty(B, int(k), dtype=torch.float32, device=scores.device)
+        top_idx = torch.empty(B, int(k), dtype=torch.int32, device=scores.device)
+        if B == 0:
+            return top_score, top_idx
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            self._ok(self.lib.gnnb_topk(self.h, B, n, _lib.fptr(scores), _lib.fptr(mask) if mask is not None else None, int(k),
+                                        _lib.fptr(top_score), C.cast(top_idx.data_ptr(), C.POINTER(C.c_int32)), C.c_void_p(stream)))
+        return top_score, top_idx
+
+    def _score(self, fr: Frontier, n_top: Optional[int], return_scores: bool, check: bool):
+        """gnnb_score (n_top = None) or gnnb_score_topk with k = n_top."""
         if self.net is None:
             raise RuntimeError('set_network first')
         net, B = self.net, fr.B
@@ -169,8 +206,9 @@ class Scorer:
         wp, bp, mask = f(fr.Wp, (B, sizes[L])), f(fr.bp, (B,)), f(fr.mask, (B, net.n_hidden))
         dev = fr.device
         pinned = host and torch.cuda.is_available()      # pinned results: device->host copies stay asynchronous
-        best = torch.empty(B, dtype=torch.float32, device=dev, pin_memory=pinned)
-        idx = torch.empty(B, dtype=torch.int32, device=dev, pin_memory=pinned)
+        shape = (B,) if n_top is None else (B, n_top)
+        best = torch.empty(shape, dtype=torch.float32, device=dev, pin_memory=pinned)
+        idx = torch.empty(shape, dtype=torch.int32, device=dev, pin_memory=pinned)
         scores = torch.empty(B, net.n_hidden, dtype=torch.float32, device=dev, pin_memory=pinned) if return_scores else None
         if B == 0:
             return best, idx, scores
@@ -184,8 +222,12 @@ class Scorer:
         d.prim_out, d.primal_input, d.wp, d.bp, d.mask = map(_lib.fptr, (pout, pin, wp, bp, mask))
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream().cuda_stream
-            st = self.lib.gnnb_score(self.h, C.byref(d), _lib.fptr(best), C.cast(idx.data_ptr(), C.POINTER(C.c_int32)),
-                                     _lib.fptr(scores) if scores is not None else None, C.c_void_p(stream))
+            out = (_lib.fptr(best), C.cast(idx.data_ptr(), C.POINTER(C.c_int32)), _lib.fptr(scores) if scores is not None else None,
+                   C.c_void_p(stream))
+            if n_top is None:
+                st = self.lib.gnnb_score(self.h, C.byref(d), *out)
+            else:
+                st = self.lib.gnnb_score_topk(self.h, C.byref(d), n_top, *out)
             if st != _lib.GNNB_OK:
                 self._raise(st)
             if check and not host:

@@ -103,6 +103,13 @@ class GraphNet(nn.Module):
         sc.set_network(fr.net, key=fr.net.key)
         return sc.score(fr, return_scores=return_scores)
 
+    def score_frontier_topk(self, fr: Frontier, k: int, return_scores: bool = False):
+        """The ``k`` best branching candidates of every subdomain (addition to the reference API): (top_score [B, k],
+        top_idx [B, k], scores [B, sum n_k] or None); column 0 is ``score_frontier``'s decision."""
+        sc = self.scorer(fr.device.index if fr.device.type == 'cuda' else None)
+        sc.set_network(fr.net, key=fr.net.key)
+        return sc.score_topk(fr, k, return_scores=return_scores)
+
     def forward(self, lower_bounds_all, upper_bounds_all, dual_vars, primals, primal_inputs, layers, masks) -> List[torch.Tensor]:
         """Same arguments and return value as the reference (graph_conv.py:479-483): a list with, per subdomain,
         the scores of the ReLUs whose mask entry is non-zero, in flat order.  Runs without autograd, as the

@@ -33,6 +33,14 @@ class GraphChoice:
     def decision(self, lower_bounds_all, upper_bounds_all, dual_vars, primal_input, primals, layers, mask):
         """-> [dec_lay, dec_idx].  Note the (primal_input, primals) order, swapped w.r.t. GraphNet.forward
         (graph_score.py:21 vs graph_conv.py:479)."""
+        return self._decide(lower_bounds_all, upper_bounds_all, dual_vars, primal_input, primals, layers, mask, None)[0]
+
+    def decision_topk(self, lower_bounds_all, upper_bounds_all, dual_vars, primal_input, primals, layers, mask, k):
+        """-> up to ``k`` [dec_lay, dec_idx] pairs, best first (addition to the reference API); the first is ``decision``'s,
+        there are min(k, undecided ReLUs) of them."""
+        return self._decide(lower_bounds_all, upper_bounds_all, dual_vars, primal_input, primals, layers, mask, int(k))
+
+    def _decide(self, lower_bounds_all, upper_bounds_all, dual_vars, primal_input, primals, layers, mask, k):
         mask = [(i == -1).float() for i in mask]                     # graph_score.py:22-24
         mask_1d = torch.cat([i for i in mask], 0).unsqueeze(0)
         start = time.time()
@@ -45,10 +53,13 @@ class GraphChoice:
         with torch.no_grad():
             fr = Frontier.from_reference_args(lower_bounds_all, upper_bounds_all, dual_vars, primals, primal_input,
                                               layers, mask_1d.to(dev))
-            best, idx, _ = self.model.score_frontier(fr, return_scores=False)
-        flat = int(idx[0].item())
+            if k is None:
+                _, idx, _ = self.model.score_frontier(fr, return_scores=False)
+            else:
+                _, idx, _ = self.model.score_frontier_topk(fr, k, return_scores=False)
+        flat = [int(i) for i in idx.reshape(-1).tolist()]
         if self.verbose:
             print(f'graph requires: {time.time() - start}')
-        if flat < 0:      # the reference's torch.max raises on an empty candidate set (graph_score.py:41)
+        if flat[0] < 0:   # the reference's torch.max raises on an empty candidate set (graph_score.py:41)
             raise RuntimeError('max(): no undecided ReLU (mask has no -1 entry)')
-        return flat_to_layer_index(flat, self.hidden_sizes)
+        return [flat_to_layer_index(f, self.hidden_sizes) for f in flat if f >= 0]

@@ -111,9 +111,10 @@ int gnnb_set_network(gnnb_ctx* ctx, const gnnb_layer_desc* layers, int n_layers,
  * node update of a layer in one launch, tensor-core mode; 0 = two launches), "snapshot" (0/1: keep per-stage copies
  * for gnnb_debug_snapshot; debugging only), "profile" (0/1: time every stage launch with CUDA events for
  * gnnb_profile_read), "rescore" (0/1, default 0; see below).  Any other key of gnnb_set_option fails with GNNB_ERR_INVALID.
- * "rescore" = 1, tensor-core mode: gnnb_score and gnnb_score_winners record every subdomain in which the tensor-core pass met
- * a NaN (activations beyond the fp16 operand range, |x| >= 524 288), score those subdomains again with the exact-fp32 SIMT
- * schedule on the same GPU and write their results (best score and index or winner record, dense scores) over the tensor-core
+ * "rescore" = 1, tensor-core mode: gnnb_score, gnnb_score_winners and gnnb_score_topk record every subdomain in which the
+ * tensor-core pass met a NaN (activations beyond the fp16 operand range, |x| >= 524 288), score those subdomains again with the
+ * exact-fp32 SIMT schedule on the same GPU and write their results (best score and index, the k best, or winner record, dense
+ * scores) over the tensor-core
  * ones; every other subdomain keeps its tensor-core result bit for bit.  Cost on a frontier without such subdomains: one 4-byte
  * device -> host copy and one synchronise of `stream` per call, also with DEVICE buffers (no extra launch or allocation).
  * The NaN count is reset before the fp32 pass, so GNNB_ERR_NAN (returned for HOST calls, through gnnb_check for DEVICE calls)
@@ -149,6 +150,24 @@ typedef struct gnnb_winner {
     int32_t index;                       /* flat index into the concatenated hidden layers, -1 when none */
 } gnnb_winner;
 int gnnb_score_winners(gnnb_ctx* ctx, const gnnb_frontier* in, gnnb_winner* winners, float* scores, void* stream);
+
+/* The k best branching candidates per subdomain instead of the best one: what strong branching over the GNN's top candidates
+ * (and a caller-side top-k) needs, without the dense [B, sum n_k] scores.  Order, per subdomain: the candidates are the
+ * entries with mask != 0 (a -inf score is still a candidate); NaN scores come first in ascending index, then the others by
+ * score, descending, equal scores (-0.0 == +0.0) by ascending index; top_score[b, j] is the bit pattern of the score of
+ * top_idx[b, j]; slots past the last candidate hold (-inf, -1).  Entry 0 is gnnb_score's (best_score, best_idx) bit for bit.
+ * A k outside [1, GNNB_TOPK_MAX], a null output or a negative B fails with GNNB_ERR_INVALID before anything is enqueued. */
+#define GNNB_TOPK_MAX 64
+/* gnnb_score with the k best candidates per subdomain instead of the best one; order contract above.
+ * top_score [B, k] f32, top_idx [B, k] i32 in in->mem (HOST: returns after they have landed);
+ * scores [B, sum n_k] or NULL as in gnnb_score.  Same launches as gnnb_score (the last one per wave is the top-k kernel,
+ * profiled as GNNB_K_ARGMAX; k = 1 runs the argmax kernel itself); option "rescore" applies as in gnnb_score. */
+int gnnb_score_topk(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t k, float* top_score, int32_t* top_idx,
+                    float* scores, void* stream);
+/* The same selection over caller-provided DEVICE arrays: scores [B, n], mask [B, n] or NULL (= every entry is a
+ * candidate).  Enqueues one launch on `stream`; needs no weights or network. */
+int gnnb_topk(gnnb_ctx* ctx, int32_t B, int32_t n, const float* scores, const float* mask, int32_t k,
+              float* top_score, int32_t* top_idx, void* stream);
 
 /* BaBSR / KW branching heuristic for B subdomains at once.  Replaces choose_node_conv (plnn/kw_score_conv.py:41-156),
  * the hand-written score the reference falls back to when the GNN decision did not improve the bound
