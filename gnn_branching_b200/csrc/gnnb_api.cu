@@ -679,7 +679,7 @@ int gnnb_create(gnnb_ctx** out, int device) {
     }
     if (cudaMalloc(&ctx->d_nan, sizeof(unsigned long long)) != cudaSuccess ||
         cudaMemset(ctx->d_nan, 0, sizeof(unsigned long long)) != cudaSuccess ||
-        simt_init() != 0 || prop_init(64 * 1024) != 0 || tc_init() != 0 || prop_tc_init() != 0 || train_init() != 0) {
+        simt_init() != 0 || prop_init(64 * 1024) != 0 || tc_init() != 0 || prop_tc_init() != 0 || kw_init() != 0 || train_init() != 0) {
         fprintf(stderr, "libgnnb: initialisation failed: %s\n", cudaGetErrorString(cudaGetLastError()));
         if (ctx->d_nan) cudaFree(ctx->d_nan);
         delete ctx;

@@ -228,6 +228,7 @@ float* queue_stage(DomainQueue* q, size_t bytes);
 // blocks go through the tensor-core propagation kernel — plans[j] = un-normalised transposed plan of layer j + 1 -> j, maps[k] =
 // slot order of layer k
 struct KwTc { const std::vector<PropPlan*>* plans; const std::vector<RowMap>* maps; };
+int kw_init();   // opt-in shared memory size of the cone kernel on the current device; returns cudaError_t
 int kw_bounds(const std::vector<LayerDev>& layers, const std::vector<int>& n, int B, const float* x, float eps, const float* wp, const float* bp,
               const float* const* prov_lb, const float* const* prov_ub, float* const* out_lb, float* const* out_ub, const KwTc* tc, float** ws,
               size_t* ws_cap, cudaStream_t st, int64_t* launches, std::string* err);

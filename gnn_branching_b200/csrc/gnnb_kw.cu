@@ -413,6 +413,7 @@ __global__ void __launch_bounds__(256) k_kw_img_reduce(const uint16_t* __restric
 // position (y, x)), columns = the C_k output channels at that position (they share the cone), the window tensors
 // [element][column] in shared memory, ping-pong.  Same sums as the dense form, different summation order.
 constexpr int CONE_MAX_DEPTH = 8;
+constexpr int CONE_MAX_SMEM = 200 * 1024;     // dynamic shared memory of k_kw_cone, opted in per device by kw_init
 struct ConeArgs {
     LayerDev layer[CONE_MAX_DEPTH];      // A_1 .. A_k
     const float* zl[CONE_MAX_DEPTH];     // bounds of layers 1 .. k - 1 (index j - 1), [B, n_j]
@@ -592,12 +593,7 @@ bool kw_cone_layer(const std::vector<LayerDev>& layers, const std::vector<int>& 
     size_t buf = max_elems * cols;
     if (buf < (size_t)5 * cols * R) buf = (size_t)5 * cols * R;
     const size_t smem = 2 * buf * sizeof(float);
-    if (smem > 200 * 1024) return false;
-    static bool attr_set = false;
-    if (!attr_set) {
-        if (cudaFuncSetAttribute(k_kw_cone, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) return false;
-        attr_set = true;
-    }
+    if (smem > CONE_MAX_SMEM) return false;
     ConeArgs a{};
     for (int j = 1; j <= k; ++j) a.layer[j - 1] = layers[j - 1];
     for (int j = 1; j < k; ++j) { a.zl[j - 1] = out_lb[j]; a.zu[j - 1] = out_ub[j]; }
@@ -624,6 +620,11 @@ bool kw_cone_layer(const std::vector<LayerDev>& layers, const std::vector<int>& 
 }
 
 }  // namespace
+
+// The shared-memory opt-in is a property of the device's context, so every context sets it (gnnb_create), not once per process
+int kw_init() {
+    return cudaFuncSetAttribute(k_kw_cone, cudaFuncAttributeMaxDynamicSharedMemorySize, CONE_MAX_SMEM);
+}
 
 // One KW pass.  Every pointer is a device pointer.  x [B, n0]; wp [B, n_L]; bp [B]; prov_lb / prov_ub: L + 1 arrays [B, n_k]
 // (k = 1..L+1, the last one — the property output — may be null) or null; out_lb / out_ub: L + 2 arrays [B, n_k] (k = 0..L+1),

@@ -621,19 +621,20 @@ def test_domain_queue_reference_function_api():
 _ISO_TIMED_OUT = set()
 
 
-def _run_isolated(what, arg, timeout=120, env=None):
-    """Run a check in its own process (its own CUDA context) with a timeout: a hang or a sticky CUDA error there cannot take
-    the rest of the suite with it.  After one time-out of a kind of check the others of that kind fail at once."""
+def _run_isolated(what, arg, timeout=120, env=None, script='gpu_isolated.py'):
+    """Run a check of ``script`` (in tests/) in its own process (its own CUDA context) with a timeout: a hang or a sticky CUDA
+    error there cannot take the rest of the suite with it.  After one time-out of a kind of check the others of that kind fail
+    at once."""
     import subprocess
     import sys
-    if what in _ISO_TIMED_OUT:
+    if (script, what) in _ISO_TIMED_OUT:
         pytest.fail(f'{what}: an earlier isolated check timed out')
     here = os.path.dirname(os.path.abspath(__file__))
     try:
-        r = subprocess.run([sys.executable, os.path.join(here, 'gpu_isolated.py'), what, arg], capture_output=True, text=True, timeout=timeout,
+        r = subprocess.run([sys.executable, os.path.join(here, script), what, arg], capture_output=True, text=True, timeout=timeout,
                            env=dict(os.environ, **(env or {})))
     except subprocess.TimeoutExpired:
-        _ISO_TIMED_OUT.add(what)
+        _ISO_TIMED_OUT.add((script, what))
         raise
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-2000:])
 
