@@ -59,6 +59,7 @@ struct gnnb_ctx {
     std::vector<PropPlan*> plan_kw_own;          // un-normalised transposed plans of the conv layers k > 0 (bound producer), else null
     std::vector<PropPlan*> plan_kw;              // per layer: plan_kw_own[k] or plan_bwd[k] (already un-normalised: layer 0, linear layers)
     std::vector<int> n;             // n[0] = input nodes, n[1..L] hidden, n[L+1] = 1
+    int zero_tap_layer = 0;         // first conv layer j >= 2 (1-based) with an input position no tap reaches, else 0
     // slot order of the tensor-core path (gnnb_common.cuh): tiling and device map of layers 0..L
     std::vector<LayerTiling> tiling;
     std::vector<RowMap> rowmap;
@@ -124,6 +125,38 @@ namespace {
 int fail(gnnb_ctx* c, int status, const std::string& msg) {
     if (c) { c->last_status = status; c->err = msg; }
     return status;
+}
+
+// taps of conv_transpose2d along one axis that reach input position i (the per-axis count of k_div_freq)
+int axis_taps(int i, int ksize, int stride, int pad, int n_out) {
+    int t = 0;
+    for (int k = 0; k < ksize; ++k) {
+        const int a = i + pad - k;
+        if (a >= 0 && a % stride == 0 && a / stride < n_out) ++t;
+    }
+    return t;
+}
+
+// First conv layer j >= 2 (1-based) with an input position that no tap of conv_transpose2d reaches (stride > kernel), else 0.
+// The GNN's backward propagation divides such a position by freq = 0 (graph_conv.py:306-312): 0/0 in the reference.  Layer 1's
+// transpose feeds the input nodes and is not normalised, so it may have such positions.
+int first_zero_tap_layer(const std::vector<LayerDev>& layers) {
+    for (size_t k = 1; k < layers.size(); ++k) {
+        const LayerDev& L = layers[k];
+        if (L.kind != GNNB_LAYER_CONV) continue;
+        for (int y = 0; y < L.h_in; ++y)
+            if (axis_taps(y, L.ksize, L.stride, L.pad, L.h_out) == 0) return (int)k + 1;
+        for (int x = 0; x < L.w_in; ++x)
+            if (axis_taps(x, L.ksize, L.stride, L.pad, L.w_out) == 0) return (int)k + 1;
+    }
+    return 0;
+}
+
+// the GNN scoring entries (score, winners, top-k, score_grad) refuse a network whose normalisation divides by zero
+int check_zero_taps(gnnb_ctx* c) {
+    if (!c->zero_tap_layer) return GNNB_OK;
+    return fail(c, GNNB_ERR_UNSUPPORTED, "layer " + std::to_string(c->zero_tap_layer) +
+                " (conv, stride > kernel) has input positions no tap reaches: the GNN's tap-count normalisation divides by zero");
 }
 
 #define CU(call)                                                                                          \
@@ -880,6 +913,7 @@ int gnnb_set_network(gnnb_ctx* ctx, const gnnb_layer_desc* layers, int n_layers,
     ctx->tiling = tiling; ctx->rowmap = rowmap;
     ctx->layers = devs;
     ctx->n = n;
+    ctx->zero_tap_layer = first_zero_tap_layer(devs);
     ctx->hidden_off = hidden_off;
     ctx->n_hidden = n_hidden;
     ctx->have_net = true;
@@ -938,6 +972,7 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, int k, float* best
     if (!ctx->have_gnn || !ctx->have_net) return fail(ctx, GNNB_ERR_STATE, "gnnb_set_gnn_weights and gnnb_set_network must be called first");
     if (in->B < 0) return fail(ctx, GNNB_ERR_INVALID, "negative batch");
     ctx->rescored = 0;
+    TRY(check_zero_taps(ctx));
     if (in->B == 0) return GNNB_OK;
     if (!in->lb || !in->ub || !in->dual || !in->prim_pre || !in->prim_post || !in->prim_out || !in->primal_input || !in->wp ||
         !in->bp || !in->mask)
@@ -1169,6 +1204,7 @@ int gnnb_score_grad(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t n_terms, con
     if (!ctx || !in || !term_domain || !term_index || !term_coeff) return fail(ctx, GNNB_ERR_INVALID, "null argument");
     if (!ctx->have_gnn || !ctx->have_net) return fail(ctx, GNNB_ERR_STATE, "gnnb_set_gnn_weights and gnnb_set_network must be called first");
     if (in->B < 1 || n_terms < 1) return fail(ctx, GNNB_ERR_INVALID, "need at least one subdomain and one term");
+    TRY(check_zero_taps(ctx));
     if (!in->lb || !in->ub || !in->dual || !in->prim_pre || !in->prim_post || !in->prim_out || !in->primal_input || !in->wp || !in->bp)
         return fail(ctx, GNNB_ERR_INVALID, "null frontier field");
     for (int i = 0; i < n_terms; ++i)

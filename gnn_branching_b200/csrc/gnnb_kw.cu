@@ -750,6 +750,7 @@ int kw_bounds(const std::vector<LayerDev>& layers, const std::vector<int>& n, in
               const float* const* prov_lb, const float* const* prov_ub, float* const* out_lb, float* const* out_ub, const KwTc* tc, float** ws,
               size_t* ws_cap, cudaStream_t st, int64_t* launches, std::string* err) {
     const int L = (int)layers.size();
+    if (L > KW_MAX_LAYERS) { *err = "KW bounds: too many layers"; return GNNB_ERR_UNSUPPORTED; }
     const float* pl[KW_MAX_LAYERS + 1];
     const float* pu[KW_MAX_LAYERS + 1];
     for (int k = 0; k <= L; ++k) { pl[k] = (prov_lb && k < L) ? prov_lb[k] : nullptr; pu[k] = (prov_ub && k < L) ? prov_ub[k] : nullptr; }

@@ -104,7 +104,12 @@ int gnnb_set_gnn_weights(gnnb_ctx* ctx, const float* const* tensors, const int64
                          int T, int p);
 
 /* Describe the verified network (the graph).  Replaces the per-call walk over layers['fixed_layers']
- * (graph_conv.py:107-137, 222-249). */
+ * (graph_conv.py:107-137, 222-249).  Conv layers: conv_transpose2d must land on the input grid (no output_padding) and the
+ * weights must fit 64 KB, else GNNB_ERR_UNSUPPORTED.  A conv layer j >= 2 with stride > kernel may leave input positions
+ * that no tap reaches; the GNN's backward propagation divides those by a tap count of 0 (0/0 in the reference).  Such a
+ * network is accepted, and the KW bounds, BaBSR and the domain queue work on it, but gnnb_score, gnnb_score_winners,
+ * gnnb_score_topk and gnnb_score_grad return GNNB_ERR_UNSUPPORTED before enqueuing anything (the message names the layer).
+ * Layer 1 may have such positions: its transpose feeds the input nodes and is not normalised. */
 int gnnb_set_network(gnnb_ctx* ctx, const gnnb_layer_desc* layers, int n_layers, int c0, int h0, int w0);
 
 /* Options: "math" (gnnb_math_mode), "chunk" (subdomains per wave; 0 = auto), "fuse" (0/1, default 1: propagation and
