@@ -85,8 +85,8 @@ struct gnnb_ctx {
     // staged copies of host inputs: two sets, so that the copies of the next chunk (copy stream) overlap the kernels of
     // the current one (caller's stream)
     struct Staging {
-        std::vector<float*> lb, ub, dual, pre, post;
-        float *pout = nullptr, *pin = nullptr, *wp = nullptr, *bp = nullptr, *mask = nullptr;
+        std::vector<float*> inputs;  // the GNN's input arrays of a wave, in the order of walk_inputs
+        float* mask = nullptr;
         float* best = nullptr;
         int32_t* idx = nullptr;
         float* scores = nullptr;
@@ -159,6 +159,37 @@ int check_zero_taps(gnnb_ctx* c) {
                 " (conv, stride > kernel) has input positions no tap reaches: the GNN's tap-count normalisation divides by zero");
 }
 
+// The arrays of a frontier the GNN reads, in one fixed order: lb[k] and ub[k] for k = 0 .. L + 1, then dual, prim_pre and
+// prim_post of each hidden layer, then prim_out, primal_input, wp and bp.  Calls f(src, slot, per) for each: src = the
+// frontier's array (null also when its per-layer table is null), slot = the matching pointer of `in`, per = floats per subdomain.
+// Staging, gathering, copying and checking a frontier all go through this walk, and the staging sets are laid out in its order.
+template <class F>
+void walk_inputs(const gnnb_frontier& fr, GnnInputs& in, const std::vector<int>& n, F f) {
+    const int L = (int)n.size() - 2;
+    auto at = [](const float* const* table, int k) { return table ? table[k] : nullptr; };
+    for (int k = 0; k <= L + 1; ++k) {
+        f(at(fr.lb, k), in.lb[k], (int64_t)n[k]);
+        f(at(fr.ub, k), in.ub[k], (int64_t)n[k]);
+    }
+    for (int k = 0; k < L; ++k) {
+        f(at(fr.dual, k), in.dual[k], (int64_t)n[k + 1] * 3);
+        f(at(fr.prim_pre, k), in.pre[k], (int64_t)n[k + 1]);
+        f(at(fr.prim_post, k), in.post[k], (int64_t)n[k + 1]);
+    }
+    f(fr.prim_out, in.pout, (int64_t)1);
+    f(fr.primal_input, in.pin, (int64_t)n[0]);
+    f(fr.wp, in.wp, (int64_t)n[L]);
+    f(fr.bp, in.bp, (int64_t)1);
+}
+
+// *out = the frontier's arrays the GNN reads; GNNB_ERR_INVALID when one of them, or the mask when `mask`, is null.  Called before
+// anything is enqueued, so that an error return never leaves copies in flight.
+int frontier_inputs(gnnb_ctx* ctx, const gnnb_frontier* fr, bool mask, GnnInputs* out) {
+    bool ok = !mask || fr->mask;
+    walk_inputs(*fr, *out, ctx->n, [&](const float* src, const float*& slot, int64_t) { slot = src; ok = ok && src; });
+    return ok ? GNNB_OK : fail(ctx, GNNB_ERR_INVALID, "null frontier array");
+}
+
 #define CU(call)                                                                                          \
     do {                                                                                                  \
         cudaError_t e__ = (call);                                                                         \
@@ -200,19 +231,14 @@ int ensure_workspace(gnnb_ctx* ctx, int Bc, bool host_staging) {
     const size_t o_nb = take(nb_rows * P);
     const size_t o_sc = take((size_t)Bc * ctx->n_hidden);
     const size_t o_best = take(Bc), o_idx = take(Bc);
-    struct StgOff { std::vector<size_t> lb, ub, du, pr, po; size_t pout, pin, wp, bp, mask, best, idx, sc; } so[2];
+    struct StgOff { std::vector<size_t> inputs; size_t mask, best, idx, sc; } so[2];
     if (host_staging) {
-        for (int i = 0; i < 2; ++i) {
-            StgOff& o = so[i];
-            o.lb.resize(L + 2); o.ub.resize(L + 2); o.du.resize(L); o.pr.resize(L); o.po.resize(L);
-            for (int k = 0; k <= L + 1; ++k) { o.lb[k] = take((size_t)Bc * ctx->n[k]); o.ub[k] = take((size_t)Bc * ctx->n[k]); }
-            for (int k = 0; k < L; ++k) {
-                o.du[k] = take((size_t)Bc * ctx->n[k + 1] * 3);
-                o.pr[k] = take((size_t)Bc * ctx->n[k + 1]);
-                o.po[k] = take((size_t)Bc * ctx->n[k + 1]);
-            }
-            o.pout = take(Bc); o.pin = take((size_t)Bc * ctx->n[0]); o.wp = take((size_t)Bc * ctx->n[L]);
-            o.bp = take(Bc); o.mask = take((size_t)Bc * ctx->n_hidden);
+        GnnInputs unused(L);
+        for (StgOff& o : so) {
+            walk_inputs(gnnb_frontier{}, unused, ctx->n, [&](const float*, const float*&, int64_t per) {
+                o.inputs.push_back(take((size_t)Bc * per));
+            });
+            o.mask = take((size_t)Bc * ctx->n_hidden);
             o.best = take((size_t)Bc * GNNB_TOPK_MAX); o.idx = take((size_t)Bc * GNNB_TOPK_MAX);   // k results per row (re-score pass)
             o.sc = take((size_t)Bc * ctx->n_hidden);
         }
@@ -234,10 +260,9 @@ int ensure_workspace(gnnb_ctx* ctx, int Bc, bool host_staging) {
         for (int i = 0; i < 2; ++i) {
             gnnb_ctx::Staging& g = ctx->stg[i];
             const StgOff& o = so[i];
-            g.lb.assign(L + 2, nullptr); g.ub.assign(L + 2, nullptr); g.dual.assign(L, nullptr); g.pre.assign(L, nullptr); g.post.assign(L, nullptr);
-            for (int k = 0; k <= L + 1; ++k) { g.lb[k] = base + o.lb[k]; g.ub[k] = base + o.ub[k]; }
-            for (int k = 0; k < L; ++k) { g.dual[k] = base + o.du[k]; g.pre[k] = base + o.pr[k]; g.post[k] = base + o.po[k]; }
-            g.pout = base + o.pout; g.pin = base + o.pin; g.wp = base + o.wp; g.bp = base + o.bp; g.mask = base + o.mask;
+            g.inputs.clear();
+            for (size_t off : o.inputs) g.inputs.push_back(base + off);
+            g.mask = base + o.mask;
             g.best = base + o.best; g.idx = reinterpret_cast<int32_t*>(base + o.idx); g.scores = base + o.sc;
         }
         if (!ctx->copy_stream) {
@@ -315,17 +340,12 @@ int snap_img(gnnb_ctx* ctx, bool on, const std::string& name, const float* img, 
     return GNNB_OK;
 }
 
-struct ChunkPtrs {
-    std::vector<const float*> lb, ub, dual, pre, post;
-    const float *pout, *pin, *wp, *bp, *mask;
-};
-
 #define TRY(expr) do { int s__ = (expr); if (s__ != GNNB_OK) return s__; } while (0)
 
 // the stage schedule for one chunk in arithmetic `math`; every pointer is a device pointer; nd: where the tensor-core NaN watch
 // records the subdomains it flags (nd.flag = null: nowhere); best_score / best_idx: [Bc, k], the k best candidates per subdomain
-int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, int math, const NanDoms& nd, float* scores, int k, float* best_score,
-              int32_t* best_idx, gnnb_winner* winners, cudaStream_t st) {
+int run_chunk(gnnb_ctx* ctx, const GnnInputs& in, const float* mask, int Bc, int math, const NanDoms& nd, float* scores, int k,
+              float* best_score, int32_t* best_idx, gnnb_winner* winners, cudaStream_t st) {
     const int L = (int)ctx->layers.size();
     const GnnParams& g = ctx->gp;
     const bool tc = math == GNNB_MATH_TC_FP16X3;
@@ -462,8 +482,8 @@ int run_chunk(gnnb_ctx* ctx, const ChunkPtrs& in, int Bc, int math, const NanDom
     }
     {
         ProfScope ps(ctx, GNNB_K_ARGMAX, Bc, st);
-        if (k == 1) masked_argmax(scores, in.mask, ctx->n_hidden, Bc, best_score, best_idx, winners, st, lc);
-        else masked_topk(scores, in.mask, ctx->n_hidden, Bc, k, best_score, best_idx, st, lc);
+        if (k == 1) masked_argmax(scores, mask, ctx->n_hidden, Bc, best_score, best_idx, winners, st, lc);
+        else masked_topk(scores, mask, ctx->n_hidden, Bc, k, best_score, best_idx, st, lc);
     }
     CU(cudaGetLastError());
     return GNNB_OK;
@@ -476,6 +496,15 @@ int ensure_nan_doms(gnnb_ctx* ctx, int B) {
     CU(cudaMalloc(&ctx->d_resc, (1 + 2 * (size_t)B) * sizeof(int32_t)));
     CU(cudaMemset(ctx->d_resc, 0, (1 + 2 * (size_t)B) * sizeof(int32_t)));
     ctx->resc_cap = B;
+    return GNNB_OK;
+}
+
+// grow-only per-domain scratch of gnnb_child_bounds / gnnb_root_bounds for B domains (3 B + 1 int32)
+int ensure_kw_iscratch(gnnb_ctx* ctx, int B, cudaStream_t st) {
+    if (ctx->kw_iscratch_cap >= B) return GNNB_OK;
+    if (ctx->kw_iscratch) { CU(cudaStreamSynchronize(st)); cudaFree(ctx->kw_iscratch); ctx->kw_iscratch = nullptr; ctx->kw_iscratch_cap = 0; }
+    CU(cudaMalloc(&ctx->kw_iscratch, (3 * (size_t)B + 1) * sizeof(int32_t)));
+    ctx->kw_iscratch_cap = B;
     return GNNB_OK;
 }
 
@@ -495,8 +524,7 @@ void reset_nan_doms(gnnb_ctx* ctx, cudaStream_t st) {
 int rescore_flagged(gnnb_ctx* ctx, const gnnb_frontier* in, int chunk, int k, float* best, int32_t* idx, gnnb_winner* winners,
                     float* scores, cudaStream_t st) {
     const bool host = in->mem == GNNB_MEM_HOST;
-    const int L = (int)ctx->layers.size(), nh = ctx->n_hidden;
-    const std::vector<int>& n = ctx->n;
+    const int nh = ctx->n_hidden;
     const NanDoms nd = nan_doms(ctx);
     int32_t count = 0;
     CU(cudaMemcpyAsync(&count, nd.count, sizeof count, cudaMemcpyDeviceToHost, st));
@@ -513,20 +541,13 @@ int rescore_flagged(gnnb_ctx* ctx, const gnnb_frontier* in, int chunk, int k, fl
     CU(cudaMemsetAsync(ctx->d_nan, 0, sizeof(unsigned long long), st));
     gnnb_ctx::Staging& sg = ctx->stg[0];
     std::vector<RowGather> tab;
-    ChunkPtrs cp;
-    auto add = [&](const float* src, float* dst, int64_t per) { tab.push_back(RowGather{src, dst, per}); return dst; };
-    cp.lb.resize(L + 2); cp.ub.resize(L + 2); cp.dual.resize(L); cp.pre.resize(L); cp.post.resize(L);
-    for (int k = 0; k <= L + 1; ++k) { cp.lb[k] = add(in->lb[k], sg.lb[k], n[k]); cp.ub[k] = add(in->ub[k], sg.ub[k], n[k]); }
-    for (int k = 0; k < L; ++k) {
-        cp.dual[k] = add(in->dual[k], sg.dual[k], (int64_t)n[k + 1] * 3);
-        cp.pre[k] = add(in->prim_pre[k], sg.pre[k], n[k + 1]);
-        cp.post[k] = add(in->prim_post[k], sg.post[k], n[k + 1]);
-    }
-    cp.pout = add(in->prim_out, sg.pout, 1);
-    cp.pin = add(in->primal_input, sg.pin, n[0]);
-    cp.wp = add(in->wp, sg.wp, n[L]);
-    cp.bp = add(in->bp, sg.bp, 1);
-    cp.mask = add(in->mask, sg.mask, nh);
+    GnnInputs cp((int)ctx->layers.size());
+    walk_inputs(*in, cp, ctx->n, [&](const float* src, const float*& slot, int64_t per) {
+        float* dst = sg.inputs[tab.size()];
+        tab.push_back(RowGather{src, dst, per});
+        slot = dst;
+    });
+    tab.push_back(RowGather{in->mask, sg.mask, nh});
     if (!host) {
         if (ctx->gather_cap < tab.size()) {
             if (ctx->d_gather) cudaFree(ctx->d_gather);
@@ -546,7 +567,7 @@ int rescore_flagged(gnnb_ctx* ctx, const gnnb_frontier* in, int chunk, int k, fl
         } else {
             gather_rows(ctx->d_gather, (int)tab.size(), nd.list + s0, Bs, st, &ctx->launches);
         }
-        TRY(run_chunk(ctx, cp, Bs, GNNB_MATH_SIMT_FP32, NanDoms{nullptr, nullptr, nullptr, 0}, sg.scores, k, sg.best, sg.idx, nullptr, st));
+        TRY(run_chunk(ctx, cp, sg.mask, Bs, GNNB_MATH_SIMT_FP32, NanDoms{nullptr, nullptr, nullptr, 0}, sg.scores, k, sg.best, sg.idx, nullptr, st));
         scatter_rescored(nd.list + s0, Bs, k, sg.best, sg.idx, sg.scores, nh, best, idx, winners, host ? nullptr : scores, nd.flag, st,
                          &ctx->launches);
         if (host && scores)
@@ -974,18 +995,11 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, int k, float* best
     ctx->rescored = 0;
     TRY(check_zero_taps(ctx));
     if (in->B == 0) return GNNB_OK;
-    if (!in->lb || !in->ub || !in->dual || !in->prim_pre || !in->prim_post || !in->prim_out || !in->primal_input || !in->wp ||
-        !in->bp || !in->mask)
-        return fail(ctx, GNNB_ERR_INVALID, "null frontier field");
+    GnnInputs cp((int)ctx->layers.size());         // the arrays of each wave, staged or in place
+    TRY(frontier_inputs(ctx, in, true, &cp));
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    const int L = (int)ctx->layers.size();
     const bool host = in->mem == GNNB_MEM_HOST;
-    // every array pointer is checked before anything is enqueued: an error return never leaves copies in flight
-    for (int k = 0; k <= L + 1; ++k)
-        if (!in->lb[k] || !in->ub[k]) return fail(ctx, GNNB_ERR_INVALID, "null bound array");
-    for (int k = 0; k < L; ++k)
-        if (!in->dual[k] || !in->prim_pre[k] || !in->prim_post[k]) return fail(ctx, GNNB_ERR_INVALID, "null dual/primal array");
     // subdomains per wave: large waves amortise launches and tails; with host buffers smaller waves let the copies of
     // wave i + 1 (copy stream, second staging set) run under the kernels of wave i
     int chunk = ctx->chunk > 0 ? ctx->chunk : 1024;
@@ -997,7 +1011,6 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, int k, float* best
         TRY(ensure_nan_doms(ctx, in->B));
         nd = nan_doms(ctx);
     }
-    const std::vector<int>& n = ctx->n;
     const int64_t n_res = (int64_t)in->B * k;
     if (host && !winners && ctx->res_cap < n_res) {
         if (ctx->res_best) cudaFree(ctx->res_best);
@@ -1023,28 +1036,17 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, int k, float* best
         // this staging set's previous user (an earlier wave of this call, or the last waves of an earlier call — possibly on
         // another stream, or one that ended in an error) is done; an event that was never recorded is a no-op
         if (host) CU(cudaStreamWaitEvent(cs, ctx->ev_free[wave & 1], 0));
-        ChunkPtrs cp;
-        cp.lb.resize(L + 2); cp.ub.resize(L + 2); cp.dual.resize(L); cp.pre.resize(L); cp.post.resize(L);
         auto stage = [&](const float* src, float* dst, size_t per_domain) -> const float* {
             const float* p = src + (size_t)c0 * per_domain;
             if (!host) return p;
             cudaMemcpyAsync(dst, p, (size_t)Bc * per_domain * sizeof(float), cudaMemcpyHostToDevice, cs);
             return dst;
         };
-        for (int k = 0; k <= L + 1; ++k) {
-            cp.lb[k] = stage(in->lb[k], host ? sg.lb[k] : nullptr, n[k]);
-            cp.ub[k] = stage(in->ub[k], host ? sg.ub[k] : nullptr, n[k]);
-        }
-        for (int k = 0; k < L; ++k) {
-            cp.dual[k] = stage(in->dual[k], host ? sg.dual[k] : nullptr, (size_t)n[k + 1] * 3);
-            cp.pre[k] = stage(in->prim_pre[k], host ? sg.pre[k] : nullptr, n[k + 1]);
-            cp.post[k] = stage(in->prim_post[k], host ? sg.post[k] : nullptr, n[k + 1]);
-        }
-        cp.pout = stage(in->prim_out, sg.pout, 1);
-        cp.pin = stage(in->primal_input, sg.pin, n[0]);
-        cp.wp = stage(in->wp, sg.wp, n[L]);
-        cp.bp = stage(in->bp, sg.bp, 1);
-        cp.mask = stage(in->mask, sg.mask, ctx->n_hidden);
+        size_t a = 0;
+        walk_inputs(*in, cp, ctx->n, [&](const float* src, const float*& slot, int64_t per) {
+            slot = stage(src, host ? sg.inputs[a++] : nullptr, per);
+        });
+        const float* mask = stage(in->mask, sg.mask, ctx->n_hidden);
         CU(cudaGetLastError());
         if (host) {
             CU(cudaEventRecord(ctx->ev_copied[wave & 1], cs));
@@ -1056,7 +1058,7 @@ static int score_impl(gnnb_ctx* ctx, const gnnb_frontier* in, int k, float* best
         int32_t* d_idx = winners ? nullptr : (host ? ctx->res_idx : best_idx) + (size_t)c0 * k;
         {
             nd.dom0 = c0;
-            const int rc = run_chunk(ctx, cp, Bc, ctx->math, nd, d_scores, k, d_best, d_idx, winners ? winners + c0 : nullptr, st);
+            const int rc = run_chunk(ctx, cp, mask, Bc, ctx->math, nd, d_scores, k, d_best, d_idx, winners ? winners + c0 : nullptr, st);
             if (rc != GNNB_OK) {      // nothing of this call may still be touching the caller's buffers or the staging sets
                 if (host) cudaStreamSynchronize(ctx->copy_stream);
                 cudaStreamSynchronize(st);
@@ -1205,49 +1207,27 @@ int gnnb_score_grad(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t n_terms, con
     if (!ctx->have_gnn || !ctx->have_net) return fail(ctx, GNNB_ERR_STATE, "gnnb_set_gnn_weights and gnnb_set_network must be called first");
     if (in->B < 1 || n_terms < 1) return fail(ctx, GNNB_ERR_INVALID, "need at least one subdomain and one term");
     TRY(check_zero_taps(ctx));
-    if (!in->lb || !in->ub || !in->dual || !in->prim_pre || !in->prim_post || !in->prim_out || !in->primal_input || !in->wp || !in->bp)
-        return fail(ctx, GNNB_ERR_INVALID, "null frontier field");
+    GnnInputs ti((int)ctx->layers.size());
+    TRY(frontier_inputs(ctx, in, false, &ti));
     for (int i = 0; i < n_terms; ++i)
         if (term_domain[i] < 0 || term_domain[i] >= in->B || term_index[i] < 0 || term_index[i] >= ctx->n_hidden)
             return fail(ctx, GNNB_ERR_INVALID, "term " + std::to_string(i) + " is out of range");
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    const int L = (int)ctx->layers.size(), B = in->B;
-    const std::vector<int>& n = ctx->n;
-    const bool host = in->mem == GNNB_MEM_HOST;
+    const int B = in->B;
+    // host buffers: one temporary device block for the inputs of this call (this entry is not the hot path)
     float* tmp = nullptr;
-    TrainInputs ti;
-    ti.lb.resize(L + 2); ti.ub.resize(L + 2); ti.dual.resize(L); ti.pre.resize(L); ti.post.resize(L);
-    size_t total = 0;
-    auto take = [&](size_t elems) { size_t o = total; total += align4(elems); return o; };
-    if (host) {
-        for (int k = 0; k <= L + 1; ++k) total += 2 * align4((size_t)B * n[k]);
-        for (int k = 0; k < L; ++k) total += align4((size_t)B * n[k + 1] * 3) + 2 * align4((size_t)B * n[k + 1]);
-        total += 2 * align4(B) + align4((size_t)B * n[0]) + align4((size_t)B * n[L]);
+    if (in->mem == GNNB_MEM_HOST) {
+        size_t total = 0;
+        walk_inputs(*in, ti, ctx->n, [&](const float*, const float*&, int64_t per) { total += align4((size_t)B * per); });
         CU(cudaMalloc(&tmp, total * sizeof(float)));
-        total = 0;
+        float* dst = tmp;
+        walk_inputs(*in, ti, ctx->n, [&](const float* src, const float*& slot, int64_t per) {
+            cudaMemcpyAsync(dst, src, (size_t)B * per * sizeof(float), cudaMemcpyHostToDevice, st);
+            slot = dst;
+            dst += align4((size_t)B * per);
+        });
     }
-    auto stage = [&](const float* src, size_t elems) -> const float* {
-        if (!host) return src;
-        float* dst = tmp + take(elems);
-        cudaMemcpyAsync(dst, src, elems * sizeof(float), cudaMemcpyHostToDevice, st);
-        return dst;
-    };
-    bool bad = false;
-    for (int k = 0; k <= L + 1; ++k) {
-        if (!in->lb[k] || !in->ub[k]) { bad = true; break; }
-        ti.lb[k] = stage(in->lb[k], (size_t)B * n[k]);
-        ti.ub[k] = stage(in->ub[k], (size_t)B * n[k]);
-    }
-    for (int k = 0; k < L && !bad; ++k) {
-        if (!in->dual[k] || !in->prim_pre[k] || !in->prim_post[k]) { bad = true; break; }
-        ti.dual[k] = stage(in->dual[k], (size_t)B * n[k + 1] * 3);
-        ti.pre[k] = stage(in->prim_pre[k], (size_t)B * n[k + 1]);
-        ti.post[k] = stage(in->prim_post[k], (size_t)B * n[k + 1]);
-    }
-    if (bad) { if (tmp) { cudaStreamSynchronize(st); cudaFree(tmp); } return fail(ctx, GNNB_ERR_INVALID, "null bound / dual / primal array"); }
-    ti.pout = stage(in->prim_out, B); ti.pin = stage(in->primal_input, (size_t)B * n[0]);
-    ti.wp = stage(in->wp, (size_t)B * n[L]); ti.bp = stage(in->bp, B);
     // optimizer.zero_grad() (graph_score_online.py:73), then loss.backward()
     cudaMemsetAsync(ctx->d_train + ctx->n_params, 0, (size_t)ctx->n_params * sizeof(float), st);
     std::string err;
@@ -1470,11 +1450,7 @@ int gnnb_child_bounds(gnnb_ctx* ctx, int32_t B, const float* x, float eps, const
         for (int k = 0; k < L; ++k) if (!out_mask[k]) return fail(ctx, GNNB_ERR_INVALID, "null mask array");
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    if (ctx->kw_iscratch_cap < B) {
-        if (ctx->kw_iscratch) { CU(cudaStreamSynchronize(st)); cudaFree(ctx->kw_iscratch); ctx->kw_iscratch = nullptr; ctx->kw_iscratch_cap = 0; }
-        CU(cudaMalloc(&ctx->kw_iscratch, (3 * (size_t)B + 1) * sizeof(int32_t)));
-        ctx->kw_iscratch_cap = B;
-    }
+    TRY(ensure_kw_iscratch(ctx, B, st));
     std::string err;
     const KwTc tc{&ctx->plan_kw, &ctx->rowmap};
     const int rc = child_bounds(ctx->layers, ctx->n, B, x, eps, wp, bp, parent_lb, parent_ub, dec_layer, dec_index, choice, out_lb, out_ub, out_mask,
@@ -1495,11 +1471,7 @@ int gnnb_root_bounds(gnnb_ctx* ctx, int32_t B, const float* x, float eps, const 
         for (int k = 0; k < L; ++k) if (!out_mask[k]) return fail(ctx, GNNB_ERR_INVALID, "null mask array");
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    if (ctx->kw_iscratch_cap < B) {
-        if (ctx->kw_iscratch) { CU(cudaStreamSynchronize(st)); cudaFree(ctx->kw_iscratch); ctx->kw_iscratch = nullptr; ctx->kw_iscratch_cap = 0; }
-        CU(cudaMalloc(&ctx->kw_iscratch, (3 * (size_t)B + 1) * sizeof(int32_t)));
-        ctx->kw_iscratch_cap = B;
-    }
+    TRY(ensure_kw_iscratch(ctx, B, st));
     std::string err;
     const KwTc tc{&ctx->plan_kw, &ctx->rowmap};
     const int rc = root_bounds(ctx->layers, ctx->n, B, x, eps, wp, bp, out_lb, out_ub, out_mask, second_pass, ctx->kw_iscratch,

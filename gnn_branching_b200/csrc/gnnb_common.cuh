@@ -187,6 +187,14 @@ void masked_topk(const float* scores, const float* mask, int n, int Bc, int k, f
 // its destination, i < n; the second writes the results of those n rows back to rows rows[i] of the call's outputs (k best
 // scores / indices per row or winner records, and the dense score rows when `scores` is not null) and clears their flags
 struct RowGather { const float* src; float* dst; int64_t per; };
+// The arrays of a batch of subdomains the GNN reads, device pointers, node order: every field of gnnb_frontier but `mask`
+// (run_chunk of gnnb_api.cu, train_backward of gnnb_train.cu).  walk_inputs (gnnb_api.cu) lists them in one fixed order.
+struct GnnInputs {
+    std::vector<const float*> lb, ub;            // L + 2 arrays [B, n_k]
+    std::vector<const float*> dual, pre, post;   // L arrays [B, n_k, 3] / [B, n_k] / [B, n_k], hidden layer k = 1..L
+    const float *pout = nullptr, *pin = nullptr, *wp = nullptr, *bp = nullptr;
+    explicit GnnInputs(int L) : lb(L + 2), ub(L + 2), dual(L), pre(L), post(L) {}
+};
 void gather_rows(const RowGather* tab, int n_arrays, const int32_t* rows, int n, cudaStream_t st, int64_t* launches);
 void scatter_rescored(const int32_t* rows, int n, int k, const float* sub_best, const int32_t* sub_idx, const float* sub_scores,
                       int n_hidden, float* best_score, int32_t* best_idx, gnnb_winner* winners, float* scores, int32_t* flag,

@@ -425,7 +425,7 @@ int train_init() {
 }
 
 int train_backward(const GnnParams& g, const TrainParams& tp, const std::vector<LayerDev>& layers, const std::vector<int>& n,
-                   const std::vector<int>& hidden_off, const TrainInputs& in, int B, int n_terms, const int32_t* term_domain,
+                   const std::vector<int>& hidden_off, const GnnInputs& in, int B, int n_terms, const int32_t* term_domain,
                    const int32_t* term_index, const float* term_coeff, float* term_scores_host, float** arena, size_t* arena_cap,
                    cudaStream_t st, int64_t* launches, std::string* err) {
     const int L = (int)layers.size(), T = g.T;

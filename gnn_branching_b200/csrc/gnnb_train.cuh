@@ -16,19 +16,13 @@ struct TrainParams {
     float* db[N_LIN];
 };
 
-// one batch of subdomains, device pointers, node order (the fields of gnnb_frontier the GNN reads)
-struct TrainInputs {
-    std::vector<const float*> lb, ub, dual, pre, post;
-    const float *pout, *pin, *wp, *bp;
-};
-
 int train_init();   // opt-in shared memory sizes; returns cudaError_t
 
 // d(sum_i coeff_i * score[domain_i][index_i]) / d(parameters) is ADDED to tp.dw / tp.db; the terms' scores are written to
 // term_scores_host (may be null).  term_* are host arrays.  *arena / *arena_cap (floats): the caller-kept tape arena, grown when
 // too small.  Synchronises `st` before returning.
 int train_backward(const GnnParams& g, const TrainParams& tp, const std::vector<LayerDev>& layers, const std::vector<int>& n,
-                   const std::vector<int>& hidden_off, const TrainInputs& in, int B, int n_terms, const int32_t* term_domain,
+                   const std::vector<int>& hidden_off, const GnnInputs& in, int B, int n_terms, const int32_t* term_domain,
                    const int32_t* term_index, const float* term_coeff, float* term_scores_host, float** arena, size_t* arena_cap,
                    cudaStream_t st, int64_t* launches, std::string* err);
 

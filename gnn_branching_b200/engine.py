@@ -181,12 +181,12 @@ class Scorer:
                                         _lib.fptr(top_score), C.cast(top_idx.data_ptr(), C.POINTER(C.c_int32)), C.c_void_p(stream)))
         return top_score, top_idx
 
-    def _score(self, fr: Frontier, n_top: Optional[int], return_scores: bool, check: bool):
-        """gnnb_score (n_top = None) or gnnb_score_topk with k = n_top."""
+    def _frontier_desc(self, fr: Frontier):
+        """gnnb_frontier of every array of ``fr`` (on this scorer's GPU, or on the CPU) + the objects that keep its arrays
+        alive."""
         if self.net is None:
             raise RuntimeError('set_network first')
-        net, B = self.net, fr.B
-        L = net.L
+        net, B, L = self.net, fr.B, self.net.L
         host = fr.device.type == 'cpu'
         if not host and fr.device.index not in (None, self.device):
             raise ValueError(f'frontier is on {fr.device}, scorer on cuda:{self.device}')
@@ -202,24 +202,30 @@ class Scorer:
         dual = [f(fr.dual[k], (B, sizes[k + 1], 3)) for k in range(L)]
         pre = [f(fr.prim_pre[k], (B, sizes[k + 1])) for k in range(L)]
         post = [f(fr.prim_post[k], (B, sizes[k + 1])) for k in range(L)]
-        pout, pin = f(fr.prim_out, (B,)), f(fr.primal_input, (B, net.n0))
-        wp, bp, mask = f(fr.Wp, (B, sizes[L])), f(fr.bp, (B,)), f(fr.mask, (B, net.n_hidden))
-        dev = fr.device
-        pinned = host and torch.cuda.is_available()      # pinned results: device->host copies stay asynchronous
-        shape = (B,) if n_top is None else (B, n_top)
-        best = torch.empty(shape, dtype=torch.float32, device=dev, pin_memory=pinned)
-        idx = torch.empty(shape, dtype=torch.int32, device=dev, pin_memory=pinned)
-        scores = torch.empty(B, net.n_hidden, dtype=torch.float32, device=dev, pin_memory=pinned) if return_scores else None
-        if B == 0:
-            return best, idx, scores
+        flat = [f(fr.prim_out, (B,)), f(fr.primal_input, (B, net.n0)), f(fr.Wp, (B, sizes[L])), f(fr.bp, (B,)),
+                f(fr.mask, (B, net.n_hidden))]
         d = _lib.FrontierDesc()
         d.B, d.mem = B, (_lib.MEM_HOST if host else _lib.MEM_DEVICE)
-        keep = []
+        keep = [lb, ub, dual, pre, post, flat]
         for name, arrs in (('lb', lb), ('ub', ub), ('dual', dual), ('prim_pre', pre), ('prim_post', post)):
             p, k = _lib.fptr_array(arrs)
             setattr(d, name, p)
             keep.append(k)
-        d.prim_out, d.primal_input, d.wp, d.bp, d.mask = map(_lib.fptr, (pout, pin, wp, bp, mask))
+        d.prim_out, d.primal_input, d.wp, d.bp, d.mask = map(_lib.fptr, flat)
+        return d, keep
+
+    def _score(self, fr: Frontier, n_top: Optional[int], return_scores: bool, check: bool):
+        """gnnb_score (n_top = None) or gnnb_score_topk with k = n_top."""
+        d, keep = self._frontier_desc(fr)
+        B, dev = fr.B, fr.device
+        host = dev.type == 'cpu'
+        pinned = host and torch.cuda.is_available()      # pinned results: device->host copies stay asynchronous
+        shape = (B,) if n_top is None else (B, n_top)
+        best = torch.empty(shape, dtype=torch.float32, device=dev, pin_memory=pinned)
+        idx = torch.empty(shape, dtype=torch.int32, device=dev, pin_memory=pinned)
+        scores = torch.empty(B, self.net.n_hidden, dtype=torch.float32, device=dev, pin_memory=pinned) if return_scores else None
+        if B == 0:
+            return best, idx, scores
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream().cuda_stream
             out = (_lib.fptr(best), C.cast(idx.data_ptr(), C.POINTER(C.c_int32)), _lib.fptr(scores) if scores is not None else None,
@@ -232,14 +238,13 @@ class Scorer:
                 self._raise(st)
             if check and not host:
                 self.check()
+        del keep
         return best, idx, scores
 
     def score_winners(self, fr: Frontier, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Score every subdomain of ``fr`` (CUDA or pinned CPU) and return the winners as packed records on the GPU:
         int32 ``[B, 2]`` = (bit pattern of the fp32 score, flat index) — the buffer the multi-GPU winner all-gather sends
         (``dist.gather_winner_records``); ``out``: a preallocated ``[>= B, 2]`` int32 CUDA tensor to write into."""
-        if self.net is None:
-            raise RuntimeError('set_network first')
         d, keep = self._frontier_desc(fr)
         dev = torch.device('cuda', self.device)
         if out is None:
@@ -299,33 +304,10 @@ class Scorer:
         return dec, cout, kind, scores
 
     # ---- online fine-tuning (graph_score_online.py:62-77) ----
-    def _frontier_desc(self, fr: Frontier):
-        """gnnb_frontier of ``fr`` (the fields the GNN reads) + the objects that keep its arrays alive."""
-        net, B, L = self.net, fr.B, self.net.L
-        sizes = [net.n0] + net.hidden_sizes + [1]
-        lb = [self._as_f32(fr.lb[k], (B, sizes[k])) for k in range(L + 2)]
-        ub = [self._as_f32(fr.ub[k], (B, sizes[k])) for k in range(L + 2)]
-        dual = [self._as_f32(fr.dual[k], (B, sizes[k + 1], 3)) for k in range(L)]
-        pre = [self._as_f32(fr.prim_pre[k], (B, sizes[k + 1])) for k in range(L)]
-        post = [self._as_f32(fr.prim_post[k], (B, sizes[k + 1])) for k in range(L)]
-        flat = [self._as_f32(fr.prim_out, (B,)), self._as_f32(fr.primal_input, (B, net.n0)),
-                self._as_f32(fr.Wp, (B, sizes[L])), self._as_f32(fr.bp, (B,)), self._as_f32(fr.mask, (B, net.n_hidden))]
-        d = _lib.FrontierDesc()
-        d.B, d.mem = B, (_lib.MEM_HOST if fr.device.type == 'cpu' else _lib.MEM_DEVICE)
-        keep = [lb, ub, dual, pre, post, flat]
-        for name, arrs in (('lb', lb), ('ub', ub), ('dual', dual), ('prim_pre', pre), ('prim_post', post)):
-            p, k = _lib.fptr_array(arrs)
-            setattr(d, name, p)
-            keep.append(k)
-        d.prim_out, d.primal_input, d.wp, d.bp, d.mask = map(_lib.fptr, flat)
-        return d, keep
-
     def score_grad(self, fr: Frontier, terms) -> torch.Tensor:
         """Back-propagate ``sum_i coeff_i * score[domain_i][flat_index_i]`` into the gradient buffers of the context
         (zeroed first, like ``optimizer.zero_grad(); loss.backward()``).  ``terms``: iterable of (domain, flat index,
         coeff).  Returns the terms' scores (fp32, CPU)."""
-        if self.net is None:
-            raise RuntimeError('set_network first')
         terms = list(terms)
         nt = len(terms)
         dom = (C.c_int32 * nt)(*[int(t[0]) for t in terms])
@@ -370,10 +352,10 @@ class Scorer:
         self._ok(self.lib.gnnb_adam_reset(self.h))
 
     # ---- batched KW bounds (gnnb_kw.cu) ----
-    def kw_bounds(self, x: torch.Tensor, eps: float, Wp: torch.Tensor, bp: torch.Tensor, provided_lb=None, provided_ub=None):
-        """KW intermediate bounds of B domains (init_kw_bounds of the reference, batched).  ``x`` [B, n0] (or [n0], shared),
-        ``Wp`` [B, n_L], ``bp`` [B]; ``provided_lb`` / ``provided_ub``: L tensors [B, n_k] (the parent's pre-ReLU bounds with
-        the split applied) or None.  Returns (lbs, ubs): L + 2 CUDA tensors [B, n_k] each."""
+    def _kw_io(self, x: torch.Tensor, Wp: torch.Tensor, bp: torch.Tensor, with_mask: bool):
+        """Inputs and outputs of the KW bound entries: B, the layer sizes, ``x`` [B, n0] (or [n0], shared), ``Wp`` [B, n_L] and
+        ``bp`` [B] as contiguous fp32 on this scorer's GPU, L + 2 output tensors [B, n_k] each for the lower and the upper
+        bounds, and L int8 output masks with their pointer array (both None without ``with_mask``)."""
         if self.net is None:
             raise RuntimeError('set_network first')
         net, L = self.net, self.net.L
@@ -386,6 +368,19 @@ class Scorer:
         bp = bp.to(dev, torch.float32).reshape(B).contiguous()
         lbs = [torch.empty(B, n, dtype=torch.float32, device=dev) for n in sizes]
         ubs = [torch.empty(B, n, dtype=torch.float32, device=dev) for n in sizes]
+        masks = mptr = None
+        if with_mask:
+            masks = [torch.empty(B, n, dtype=torch.int8, device=dev) for n in sizes[1:L + 1]]
+            marr = (C.POINTER(C.c_int8) * L)(*[C.cast(m.data_ptr(), C.POINTER(C.c_int8)) for m in masks])
+            mptr = C.cast(marr, C.POINTER(C.POINTER(C.c_int8)))      # keeps marr alive
+        return B, sizes, x, Wp, bp, lbs, ubs, masks, mptr
+
+    def kw_bounds(self, x: torch.Tensor, eps: float, Wp: torch.Tensor, bp: torch.Tensor, provided_lb=None, provided_ub=None):
+        """KW intermediate bounds of B domains (init_kw_bounds of the reference, batched).  ``x`` [B, n0] (or [n0], shared),
+        ``Wp`` [B, n_L], ``bp`` [B]; ``provided_lb`` / ``provided_ub``: L tensors [B, n_k] (the parent's pre-ReLU bounds with
+        the split applied) or None.  Returns (lbs, ubs): L + 2 CUDA tensors [B, n_k] each."""
+        B, sizes, x, Wp, bp, lbs, ubs, _, _ = self._kw_io(x, Wp, bp, with_mask=False)
+        dev = x.device
         plb = pub = None
         keep = []
         if provided_lb is not None:
@@ -408,26 +403,10 @@ class Scorer:
         """Bounds of B root domains — the bounds part of ``KWConvGen.build_the_model`` (plnn/conv_kwinter_gen.py:199-270):
         KW bounds intersected with interval bounds, and a KW pass where that moved a hidden layer.  ``x`` [B, n0] (or [n0]),
         ``Wp`` [B, n_L], ``bp`` [B].  Returns (lbs, ubs, masks, second_pass) like ``child_bounds``."""
-        if self.net is None:
-            raise RuntimeError('set_network first')
-        net, L = self.net, self.net.L
-        dev = torch.device('cuda', self.device)
-        sizes = [net.n0] + net.hidden_sizes + [1]
-        Wp = Wp.to(dev, torch.float32).reshape(-1, sizes[L]).contiguous()
-        B = int(Wp.shape[0])
-        x = x.to(dev, torch.float32).reshape(-1, net.n0)
-        x = (x.expand(B, net.n0) if x.shape[0] == 1 else x).contiguous()
-        bp = bp.to(dev, torch.float32).reshape(B).contiguous()
-        lbs = [torch.empty(B, n, dtype=torch.float32, device=dev) for n in sizes]
-        ubs = [torch.empty(B, n, dtype=torch.float32, device=dev) for n in sizes]
-        masks = [torch.empty(B, n, dtype=torch.int8, device=dev) for n in sizes[1:L + 1]] if with_mask else None
-        second = torch.empty(B, dtype=torch.int32, device=dev)
+        B, _, x, Wp, bp, lbs, ubs, masks, mptr = self._kw_io(x, Wp, bp, with_mask)
+        second = torch.empty(B, dtype=torch.int32, device=x.device)
         olb, k3 = _lib.fptr_array(lbs)
         oub, k4 = _lib.fptr_array(ubs)
-        mptr = None
-        if with_mask:
-            marr = (C.POINTER(C.c_int8) * L)(*[C.cast(m.data_ptr(), C.POINTER(C.c_int8)) for m in masks])
-            mptr = C.cast(marr, C.POINTER(C.POINTER(C.c_int8)))
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream().cuda_stream
             self._ok(self.lib.gnnb_root_bounds(self.h, B, _lib.fptr(x), float(eps), _lib.fptr(Wp), _lib.fptr(bp), olb, oub, mptr,
@@ -442,32 +421,17 @@ class Scorer:
         property output); ``dec_layer`` (0-based hidden layer), ``dec_index``, ``choice`` (0 blocked / 1 passing): [B] ints.
         Returns (lbs, ubs, masks, second_pass): L + 2 CUDA tensors [B, n_k] each, L int8 masks in the BaB convention
         (or None), [B] int32 flags of the domains that took the second KW pass."""
-        if self.net is None:
-            raise RuntimeError('set_network first')
-        net, L = self.net, self.net.L
-        dev = torch.device('cuda', self.device)
-        sizes = [net.n0] + net.hidden_sizes + [1]
-        Wp = Wp.to(dev, torch.float32).reshape(-1, sizes[L]).contiguous()
-        B = int(Wp.shape[0])
-        x = x.to(dev, torch.float32).reshape(-1, net.n0)
-        x = (x.expand(B, net.n0) if x.shape[0] == 1 else x).contiguous()
-        bp = bp.to(dev, torch.float32).reshape(B).contiguous()
+        B, sizes, x, Wp, bp, lbs, ubs, masks, mptr = self._kw_io(x, Wp, bp, with_mask)
+        dev = x.device
         pl = [self._as_f32(t.to(dev).reshape(B, -1), (B, sizes[k])) for k, t in enumerate(parent_lb)]
         pu = [self._as_f32(t.to(dev).reshape(B, -1), (B, sizes[k])) for k, t in enumerate(parent_ub)]
         ints = [t.to(dev, torch.int32).reshape(B).contiguous() for t in (dec_layer, dec_index, choice)]
-        lbs = [torch.empty(B, n, dtype=torch.float32, device=dev) for n in sizes]
-        ubs = [torch.empty(B, n, dtype=torch.float32, device=dev) for n in sizes]
-        masks = [torch.empty(B, n, dtype=torch.int8, device=dev) for n in sizes[1:L + 1]] if with_mask else None
         second = torch.empty(B, dtype=torch.int32, device=dev)
         plb, k1 = _lib.fptr_array(pl)
         pub, k2 = _lib.fptr_array(pu)
         olb, k3 = _lib.fptr_array(lbs)
         oub, k4 = _lib.fptr_array(ubs)
         ip = lambda t: C.cast(t.data_ptr(), C.POINTER(C.c_int32))
-        mptr = None
-        if with_mask:
-            marr = (C.POINTER(C.c_int8) * L)(*[C.cast(m.data_ptr(), C.POINTER(C.c_int8)) for m in masks])
-            mptr = C.cast(marr, C.POINTER(C.POINTER(C.c_int8)))
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream().cuda_stream
             self._ok(self.lib.gnnb_child_bounds(self.h, B, _lib.fptr(x), float(eps), _lib.fptr(Wp), _lib.fptr(bp), plb, pub,

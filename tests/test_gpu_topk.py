@@ -278,6 +278,49 @@ def test_invalid_arguments():
     del keep
 
 
+def test_null_frontier_arrays_are_rejected():
+    """A frontier with one null array (a bound, a dual, the input point, the mask) fails gnnb_score, gnnb_score_winners and
+    gnnb_score_topk with GNNB_ERR_INVALID before anything is enqueued, with DEVICE and HOST descriptors, and the context
+    scores a valid frontier afterwards.  gnnb_score_grad rejects a null bound but does not read the mask."""
+    fr = _frontier('base', 4, seed=2, device='cpu')
+    sc = _scorer(fr.net)
+    fp, ip = _lib.fptr, (lambda t: C.cast(t.data_ptr(), C.POINTER(C.c_int32)))
+    st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    winners = torch.empty(4, 2, dtype=torch.int32, device='cuda')
+
+    def desc_without(f, field, k=None):
+        d, keep = sc._frontier_desc(f)
+        if k is None:
+            setattr(d, field, None)
+        else:
+            getattr(d, field)[k] = None                          # the per-layer table lives in `keep`
+        return d, keep
+
+    for mem, f in (('device', fr.to('cuda')), ('host', fr.pin())):
+        want_best, want_idx, _ = sc.score(f, return_scores=False)
+        best = torch.empty(4, 64, device=f.device, pin_memory=mem == 'host')
+        idx = torch.empty(4, 64, dtype=torch.int32, device=f.device, pin_memory=mem == 'host')
+        for name in (('lb', 1), ('dual', 2), ('primal_input',), ('mask',)):
+            d, keep = desc_without(f, *name)
+            n0 = sc.launches
+            assert sc.lib.gnnb_score(sc.h, C.byref(d), fp(best), ip(idx), None, st) == _lib.GNNB_ERR_INVALID, (mem, name)
+            assert sc.lib.gnnb_score_winners(sc.h, C.byref(d), C.c_void_p(winners.data_ptr()), None, st) == _lib.GNNB_ERR_INVALID
+            assert sc.lib.gnnb_score_topk(sc.h, C.byref(d), 5, fp(best), ip(idx), None, st) == _lib.GNNB_ERR_INVALID
+            assert sc.launches == n0, (mem, name)
+            d.B = 0                                              # an empty frontier is never read
+            assert sc.lib.gnnb_score(sc.h, C.byref(d), fp(best), ip(idx), None, st) == _lib.GNNB_OK
+            del keep
+            got_best, got_idx, _ = sc.score(f, return_scores=False)
+            assert torch.equal(got_idx, want_idx) and torch.equal(_bits(got_best), _bits(want_best)), (mem, name)
+        term = ((C.c_int32 * 1)(1), (C.c_int32 * 1)(5), (C.c_float * 1)(1.0), (C.c_float * 1)())
+        for name, status in ((('lb', 1), _lib.GNNB_ERR_INVALID), (('mask',), _lib.GNNB_OK)):
+            d, keep = desc_without(f, *name)
+            n0 = sc.launches
+            assert sc.lib.gnnb_score_grad(sc.h, C.byref(d), 1, *term, st) == status, (mem, name)
+            assert (sc.launches == n0) == (status != _lib.GNNB_OK), (mem, name)
+            del keep
+
+
 def test_decision_topk(tmp_path):
     fr = _frontier('base', 3, seed=21, device='cpu')
     fr.mask[2].zero_()
