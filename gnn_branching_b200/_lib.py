@@ -18,7 +18,7 @@ KERNEL_CLASSES = ['relax', 'update_fwd', 'update_bwd', 'update_bwd_score', 'inpu
 EXPORTS = ['gnnb_create', 'gnnb_destroy', 'gnnb_set_gnn_weights', 'gnnb_set_network', 'gnnb_set_option',
            'gnnb_get_option', 'gnnb_score', 'gnnb_score_winners', 'gnnb_score_topk', 'gnnb_topk', 'gnnb_check', 'gnnb_launch_count', 'gnnb_last_error',
            'gnnb_debug_snapshot', 'gnnb_abi_version', 'gnnb_profile_read', 'gnnb_profile_reset', 'gnnb_babsr',
-           'gnnb_score_grad', 'gnnb_get_gradients', 'gnnb_get_gnn_weights', 'gnnb_adam_step', 'gnnb_adam_reset',
+           'gnnb_score_grad', 'gnnb_score_grad_device', 'gnnb_get_gradients', 'gnnb_get_gnn_weights', 'gnnb_adam_step', 'gnnb_adam_reset',
            'gnnb_kw_bounds', 'gnnb_child_bounds', 'gnnb_root_bounds', 'gnnb_queue_create', 'gnnb_queue_destroy', 'gnnb_queue_add', 'gnnb_queue_pick', 'gnnb_queue_prune', 'gnnb_queue_stats']
 
 _fp = C.POINTER(C.c_float)
@@ -78,6 +78,7 @@ def load() -> C.CDLL:
     lib.gnnb_topk.argtypes = [vp, C.c_int32, C.c_int32, _fp, _fp, C.c_int32, _fp, _ip, vp]
     lib.gnnb_babsr.argtypes = [vp, C.POINTER(FrontierDesc), C.c_int32, C.c_float, _ip, _ip, _ip, _ip, _ip, _fp, vp]
     lib.gnnb_score_grad.argtypes = [vp, C.POINTER(FrontierDesc), C.c_int32, _ip, _ip, _fp, _fp, vp]
+    lib.gnnb_score_grad_device.argtypes = [vp, C.POINTER(FrontierDesc), C.c_int32, _ip, _ip, _fp, _fp, vp]
     lib.gnnb_get_gradients.argtypes = [vp, _fpp, C.POINTER(C.c_int64), C.c_int]
     lib.gnnb_get_gnn_weights.argtypes = [vp, _fpp, C.POINTER(C.c_int64), C.c_int]
     lib.gnnb_adam_step.argtypes = [vp, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, vp]

@@ -30,6 +30,21 @@ is the stored decision, whose children the step bounds anyway; every further ran
 parents that have such a candidate.  The improvement is measured on the KW / interval surrogate bounds of the children, not
 on the LP bounds the reference would compute (see below).  Strong branching and the threshold rule are exclusive.
 
+With ``online=True`` (which needs ``kw_fallback=True``: the threshold rule is the trigger) the step also fine-tunes the GNN
+online, as the reference's ``--bab_online`` loop does (plnn/relu_conv_online.py:198-211 with GraphChoice.online_learning,
+graphnet/graph_score_online.py:62-77): when the KW decision of m > 0 parents replaced their GNN decision, one Adam step
+(``online_lr``, ``online_wd``: the reference's ``GraphChoice(lr=1e-4, wd=1e-4)``) is taken on the loss
+``(1/m) sum_parents (gnn_score - kw_score)`` over the parents' GNN frontier, with the gradient pass of
+``gnnb_score_grad_device`` on terms built on the device; the children are then decided by the updated GNN, as in the
+reference, where ``online_learning`` precedes the children's ``decision`` calls.  The updated parameters are copied device to
+device into ``model``, so ``state_dict()`` follows the fine-tuning.  Where this differs from the reference:
+  - one Adam step on the mean loss of a batch, not one step per parent; the mean keeps the single-parent gradient scale, so
+    the weight decay weighs as in the reference;
+  - the + term is the parent's stored GNN decision.  The reference differentiates the scores of its last ``decision()`` call,
+    a one-at-a-time detail with no batched counterpart;
+  - the reference driver's constant ``pref_online_thd = 2`` (SURVEY §5) is not modelled: its use in relu_conv_online.py
+    could not be checked against the reference source.
+
 What is NOT here is the LP: Gurobi is out of scope (SURVEY §8), so the values the reference takes from the LP solution are
 SURROGATES and the step is labelled as such wherever it is reported — the child's lower bound is the lower bound of the
 property output from the KW / interval pass (valid, but looser than the LP's), its upper bound is the parent's, the GNN's
@@ -64,13 +79,14 @@ class StepStats:
     kw_used: int = 0         # ... and won
     sb_bounded: int = 0      # strong branching: child pairs bounded beyond the stored decision's
     sb_changed: int = 0      # strong branching: parents whose split is not the stored GNN decision
+    online_trained: int = 0  # online: parents whose loss terms went into this step's Adam step (= kw_used)
 
 
 class FrontierStep:
     def __init__(self, model: GraphNet, net: NetSpec, x: torch.Tensor, eps: float, Wp: torch.Tensor, bp: float,
                  capacity: int = 1 << 16, decision_bound: float = 0.0, device: int = 0, kw_fallback: bool = False,
                  branching_threshold: float = 0.2, kwbd_threshold: int = 20, sparsest_layer: int = 0, strong_branching_k: int = 1,
-                 strong_branching_kw_k: int = 0):
+                 strong_branching_kw_k: int = 0, online: bool = False, online_lr: float = 1e-4, online_wd: float = 1e-4):
         self.model, self.net, self.eps, self.decision_bound = model, net, float(eps), float(decision_bound)
         self.kw_fallback, self.branching_threshold, self.kwbd_threshold = bool(kw_fallback), float(branching_threshold), int(kwbd_threshold)
         self.sparsest_layer = int(sparsest_layer)
@@ -81,6 +97,11 @@ class FrontierStep:
         if self.strong and self.kw_fallback:
             raise ValueError('strong branching and kw_fallback (the threshold rule) cannot be combined')
         self.last_strong = None          # (candidates [B, K, 2], improvement [B, K], chosen rank [B]) of the last strong step
+        self.online, self.online_lr, self.online_wd = bool(online), float(online_lr), float(online_wd)
+        if self.online and not self.kw_fallback:
+            raise ValueError('online=True needs kw_fallback=True: the threshold rule triggers the online update')
+        # (parent rows in the step's pick order, GNN flat index, KW flat index, term scores [2 m]) of the last online update
+        self.last_online = None
         self.dev = torch.device('cuda', device)
         self.scorer = model.scorer(device)
         self.scorer.set_network(net, key=net.key)
@@ -102,6 +123,8 @@ class FrontierStep:
         self.prim_out = (post[-1] @ self.Wp.t()).reshape(1) + self.bp
         self._zeros = {}
         self.ineff_kw = torch.zeros(net.n_hidden, dtype=torch.int32, device=self.dev)      # relu_conv_gnnkwthreshold.py:134 ineff_kw_dc
+        if self.online:
+            self.scorer.adam_reset()     # a fresh optimiser per run, as the reference builds GraphChoice per verification
 
     # ---- seeding ----
     def seed_root(self, lbs: List[torch.Tensor] = None, ubs: List[torch.Tensor] = None) -> None:
@@ -129,6 +152,7 @@ class FrontierStep:
                                                            [rep(t) for t in parents.lb], [rep(t) for t in parents.ub],
                                                            dec[:, 0], dec[:, 1], choice)
         kw_tried = kw_used = sb_bounded = sb_changed = 0
+        self.last_online = None
         if self.kw_fallback:
             kw_tried, kw_used = self._kw_fallback(parents, lbs, ubs, masks, second)
         elif self.strong:
@@ -153,7 +177,8 @@ class FrontierStep:
         children = DomainBatch(lower.contiguous(), rep(parents.upper_bound).contiguous(), lbs, ubs, mask, new_dec)
         added = self.queue.add(children, keep=keep)
         glb = self.queue.global_lb if len(self.queue) else float('nan')
-        return StepStats(B, 2 * B, int(second.sum()), int(bad.sum()), added, glb, kw_tried, kw_used, sb_bounded, sb_changed)
+        return StepStats(B, 2 * B, int(second.sum()), int(bad.sum()), added, glb, kw_tried, kw_used, sb_bounded, sb_changed,
+                         kw_used if self.online else 0)
 
     # ---- the threshold rule (relu_conv_gnnkwthreshold.py:145-203) ----
     def _improvement(self, plb: torch.Tensor, lbs, ubs) -> torch.Tensor:
@@ -191,7 +216,24 @@ class FrontierStep:
                                       gnn_imp[idx], ok, lbs, ubs, masks, second)                  # :177-190
         bad_kw = ok & (kw_imp < gnn_imp[idx]) & (kw_imp < 0.05)                                   # :171-176
         self.ineff_kw.index_add_(0, flat, bad_kw.to(torch.int32))
-        return m, int(use.sum())
+        used = int(use.sum())
+        if self.online and used:
+            self._online_update(parents, idx, use, self.offsets[gnn_dec[:, 0].long()] + gnn_dec[:, 1].long(), flat, used)
+        return m, used
+
+    def _online_update(self, parents: DomainBatch, idx, use, gnn_flat, kw_flat, used: int):
+        """One Adam step on (1/m) sum (score at the stored GNN decision - score at the KW decision) over the ``used`` parents
+        (rows ``idx[use]``) on the parents' GNN frontier (graph_score_online.py:62-77), then the new parameters into
+        ``model``.  The 2 len(idx) terms are built on the device; parents where KW did not win get inactive terms (domain -1)."""
+        dom = torch.where(use, idx, torch.full_like(idx, -1)).to(torch.int32)
+        coeff = torch.full((idx.numel(),), 1.0 / used, dtype=torch.float32, device=self.dev)
+        terms = (torch.cat([dom, dom]), torch.cat([gnn_flat, kw_flat]).to(torch.int32), torch.cat([coeff, -coeff]))
+        fr = self._frontier(parents.lb, parents.ub, parents.mask)
+        vals = self.scorer.score_grad(fr, terms)
+        self.scorer.adam_step(self.online_lr, weight_decay=self.online_wd)
+        self.model.adopt_weights(self.scorer)
+        n = idx.numel()
+        self.last_online = (idx[use], gnn_flat[use], kw_flat[use], torch.cat([vals[:n][use], vals[n:][use]]))
 
     def _try_split(self, plower, plb, pub, idx, dec, beat, ok, lbs, ubs, masks, second):
         """Bound the two children of the parents ``idx`` (lower bounds ``plower``, bounds ``plb`` / ``pub``: [m, .]) split on

@@ -13,6 +13,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <map>
 #include <string>
 #include <vector>
@@ -45,11 +46,14 @@ struct gnnb_ctx {
     int64_t n_params = 0;
     size_t po_w[N_LIN] = {0}, po_b[N_LIN] = {0};
     int adam_steps = 0;
-    float* train_ws = nullptr;      // activation tape + gradient temporaries of gnnb_score_grad (grow-only)
+    float* train_ws = nullptr;      // gnnb_score_grad(_device): tape of a wave, staged input rows, gather table (grow-only)
     size_t train_ws_cap = 0;
+    int grad_chunk = 0;             // subdomains per wave of the gradient pass; 0 = the most whose tape fits GRAD_TAPE_BYTES
+    int grad_ws_domains = 0;        // subdomains per wave of the last gradient call
+    int64_t grad_bad_terms = 0;     // out-of-range terms of the last gradient call
     float* kw_ws = nullptr;         // column buffers of gnnb_kw_bounds (grow-only)
     size_t kw_ws_cap = 0;
-    int32_t* kw_iscratch = nullptr; // per-domain flags of gnnb_child_bounds (grow-only)
+    int32_t* kw_iscratch = nullptr; // per-domain flags of gnnb_child_bounds, named subdomains of gnnb_score_grad_device (grow-only)
     int kw_iscratch_cap = 0;
     // verified network
     bool have_net = false;
@@ -499,11 +503,11 @@ int ensure_nan_doms(gnnb_ctx* ctx, int B) {
     return GNNB_OK;
 }
 
-// grow-only per-domain scratch of gnnb_child_bounds / gnnb_root_bounds for B domains (3 B + 1 int32)
+// grow-only per-domain scratch of gnnb_child_bounds / gnnb_root_bounds / gnnb_score_grad_device for B domains (3 B + 2 int32)
 int ensure_kw_iscratch(gnnb_ctx* ctx, int B, cudaStream_t st) {
     if (ctx->kw_iscratch_cap >= B) return GNNB_OK;
     if (ctx->kw_iscratch) { CU(cudaStreamSynchronize(st)); cudaFree(ctx->kw_iscratch); ctx->kw_iscratch = nullptr; ctx->kw_iscratch_cap = 0; }
-    CU(cudaMalloc(&ctx->kw_iscratch, (3 * (size_t)B + 1) * sizeof(int32_t)));
+    CU(cudaMalloc(&ctx->kw_iscratch, (3 * (size_t)B + 2) * sizeof(int32_t)));
     ctx->kw_iscratch_cap = B;
     return GNNB_OK;
 }
@@ -701,11 +705,11 @@ int download_quarter(gnnb_ctx* ctx, int quarter, float* const* tensors, const in
             return fail(ctx, GNNB_ERR_INVALID, "tensor " + std::to_string(2 * l) + " has the wrong number of elements");
     CU(cudaSetDevice(ctx->device));
     CU(cudaDeviceSynchronize());
-    std::vector<float> host((size_t)ctx->n_params);
-    CU(cudaMemcpy(host.data(), ctx->d_train + (size_t)quarter * ctx->n_params, host.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    // host or device destinations: the direction follows from the pointer (unified addressing)
+    const float* src = ctx->d_train + (size_t)quarter * ctx->n_params;
     for (int l = 0; l < N_LIN; ++l) {
-        memcpy(tensors[2 * l], &host[ctx->po_w[l]], sizeof(float) * lin_in(l) * lin_out(l));
-        memcpy(tensors[2 * l + 1], &host[ctx->po_b[l]], sizeof(float) * lin_out(l));
+        CU(cudaMemcpy(tensors[2 * l], src + ctx->po_w[l], sizeof(float) * lin_in(l) * lin_out(l), cudaMemcpyDefault));
+        CU(cudaMemcpy(tensors[2 * l + 1], src + ctx->po_b[l], sizeof(float) * lin_out(l), cudaMemcpyDefault));
     }
     return GNNB_OK;
 }
@@ -959,6 +963,9 @@ int gnnb_set_option(gnnb_ctx* ctx, const char* key, int64_t value) {
         ctx->profile = value ? 1 : 0;
     } else if (k == "rescore") {
         ctx->rescore = value ? 1 : 0;
+    } else if (k == "grad_chunk") {
+        if (value < 0 || value > 0x7fffffff) return fail(ctx, GNNB_ERR_INVALID, "grad_chunk must be in [0, 2^31)");
+        ctx->grad_chunk = (int)value;
     } else {
         return fail(ctx, GNNB_ERR_INVALID, "unknown option " + k);
     }
@@ -975,6 +982,9 @@ int64_t gnnb_get_option(gnnb_ctx* ctx, const char* key) {
     if (k == "profile") return ctx->profile;
     if (k == "rescore") return ctx->rescore;
     if (k == "rescored") return ctx->rescored;
+    if (k == "grad_chunk") return ctx->grad_chunk;
+    if (k == "grad_workspace_domains") return ctx->grad_ws_domains;
+    if (k == "grad_bad_terms") return ctx->grad_bad_terms;
     if (k == "n_hidden") return ctx->n_hidden;
     if (k == "workspace_domains") return ctx->ws_cap;
     if (k.rfind("plan_density_pct_", 0) == 0) {      // e.g. plan_density_pct_f0 / plan_density_pct_b1
@@ -1201,41 +1211,143 @@ int gnnb_babsr(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t sparsest_layer, f
     return GNNB_OK;
 }
 
-int gnnb_score_grad(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t n_terms, const int32_t* term_domain, const int32_t* term_index,
-                    const float* term_coeff, float* term_scores, void* stream) {
-    if (!ctx || !in || !term_domain || !term_index || !term_coeff) return fail(ctx, GNNB_ERR_INVALID, "null argument");
+// tape of one wave of the gradient pass with option grad_chunk = 0 (about 25 MB per base subdomain: ~170 per wave)
+static const size_t GRAD_TAPE_BYTES = size_t(4) << 30;
+
+// argument checks of gnnb_score_grad(_device) that need no term values; *ti = the frontier's arrays
+static int grad_args(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t n_terms, GnnInputs* ti) {
     if (!ctx->have_gnn || !ctx->have_net) return fail(ctx, GNNB_ERR_STATE, "gnnb_set_gnn_weights and gnnb_set_network must be called first");
     if (in->B < 1 || n_terms < 1) return fail(ctx, GNNB_ERR_INVALID, "need at least one subdomain and one term");
     TRY(check_zero_taps(ctx));
+    return frontier_inputs(ctx, in, false, ti);
+}
+
+// host frontier: copy its arrays into one temporary device block *tmp (the caller frees it after synchronising `st`) and point
+// *ti at them
+static int stage_grad_frontier(gnnb_ctx* ctx, const gnnb_frontier* in, GnnInputs* ti, float** tmp, cudaStream_t st) {
+    const int B = in->B;
+    size_t total = 0;
+    walk_inputs(*in, *ti, ctx->n, [&](const float*, const float*&, int64_t per) { total += align4((size_t)B * per); });
+    CU(cudaMalloc(tmp, total * sizeof(float)));
+    float* dst = *tmp;
+    walk_inputs(*in, *ti, ctx->n, [&](const float* src, const float*& slot, int64_t per) {
+        cudaMemcpyAsync(dst, src, (size_t)B * per * sizeof(float), cudaMemcpyHostToDevice, st);
+        slot = dst;
+        dst += align4((size_t)B * per);
+    });
+    CU(cudaGetLastError());
+    return GNNB_OK;
+}
+
+// The gradient pass over device terms.  in: device arrays of the frontier's B subdomains.  The subdomains some active term
+// names are listed on the device; the count is read back (one synchronise of `st`), and those subdomains run through the
+// taped forward and the backward in waves of at most W, each gathered into staging rows of the arena first.
+static int score_grad_impl(gnnb_ctx* ctx, GnnInputs& in, int B, int n_terms, const int32_t* term_domain, const int32_t* term_index,
+                           const float* term_coeff, float* term_scores, cudaStream_t st) {
+    const int L = (int)ctx->layers.size();
+    TRY(ensure_kw_iscratch(ctx, B, st));
+    int32_t* cnt = ctx->kw_iscratch;                     // [named, bad | flag [B] | list [B] | row_of [B]]
+    int32_t *flag = cnt + 2, *list = flag + B, *row_of = list + B;
+    CU(cudaMemsetAsync(cnt, 0, (2 + (size_t)B) * sizeof(int32_t), st));
+    // optimizer.zero_grad() (graph_score_online.py:73), then loss.backward()
+    CU(cudaMemsetAsync(ctx->d_train + ctx->n_params, 0, (size_t)ctx->n_params * sizeof(float), st));
+    name_terms(term_domain, term_index, n_terms, B, ctx->n_hidden, term_scores, cnt, flag, list, row_of, st, &ctx->launches);
+    int32_t hc[2] = {0, 0};
+    CU(cudaMemcpyAsync(hc, cnt, sizeof hc, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    const int named = hc[0];
+    ctx->grad_bad_terms = hc[1];
+    ctx->grad_ws_domains = 0;
+    if (named == 0) return GNNB_OK;
+    size_t W = (size_t)ctx->grad_chunk;
+    if (W == 0) W = std::max<size_t>(1, GRAD_TAPE_BYTES / (sizeof(float) * train_tape_floats(ctx->n, ctx->gp.T, 1)));
+    W = std::min<size_t>(W, (size_t)named);
+    // arena: tape of a wave | the wave's input rows, in walk_inputs order | their gather table
+    auto align64 = [](size_t x) { return (x + 63) & ~size_t(63); };
+    size_t total = align64(train_tape_floats(ctx->n, ctx->gp.T, (int)W));
+    std::vector<RowGather> tab;
+    std::vector<size_t> off;
+    walk_inputs(gnnb_frontier{}, in, ctx->n, [&](const float*, const float*& src, int64_t per) {
+        tab.push_back(RowGather{src, nullptr, per});
+        off.push_back(total);
+        total += align64(W * per);
+    });
+    const size_t o_tab = total;
+    total += align64((tab.size() * sizeof(RowGather) + sizeof(float) - 1) / sizeof(float));
+    if (ctx->train_ws_cap < total) {
+        if (ctx->train_ws) { CU(cudaStreamSynchronize(st)); cudaFree(ctx->train_ws); }
+        ctx->train_ws = nullptr; ctx->train_ws_cap = 0;
+        CU(cudaMalloc(&ctx->train_ws, total * sizeof(float)));
+        ctx->train_ws_cap = total;
+    }
+    GnnInputs cp(L);
+    size_t i = 0;
+    walk_inputs(gnnb_frontier{}, cp, ctx->n, [&](const float*, const float*& slot, int64_t) {
+        tab[i].dst = ctx->train_ws + off[i];
+        slot = tab[i++].dst;
+    });
+    RowGather* d_tab = reinterpret_cast<RowGather*>(ctx->train_ws + o_tab);
+    // a stream-ordered copy from pageable memory returns after the source has been read: `tab` may go out of scope
+    CU(cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(RowGather), cudaMemcpyHostToDevice, st));
+    const TrainParams tp = train_params(ctx);
+    for (int row0 = 0, Bw = 0; row0 < named; row0 += Bw) {
+        Bw = std::min((int)W, named - row0);
+        gather_rows(d_tab, (int)tab.size(), list + row0, Bw, st, &ctx->launches);
+        const WaveTerms wt{term_domain, term_index, term_coeff, row_of, n_terms, B, ctx->n_hidden, row0, term_scores};
+        const int e = train_wave(ctx->gp, tp, ctx->layers, ctx->n, ctx->hidden_off, cp, (int)W, Bw, wt, ctx->train_ws, st,
+                                 &ctx->launches);
+        if (e != cudaSuccess) return fail(ctx, GNNB_ERR_CUDA, std::string("gradient pass: ") + cudaGetErrorString((cudaError_t)e));
+    }
+    ctx->grad_ws_domains = (int)W;
+    return GNNB_OK;
+}
+
+int gnnb_score_grad_device(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t n_terms, const int32_t* term_domain,
+                           const int32_t* term_index, const float* term_coeff, float* term_scores, void* stream) {
+    if (!ctx || !in || !term_domain || !term_index || !term_coeff || !term_scores) return fail(ctx, GNNB_ERR_INVALID, "null argument");
     GnnInputs ti((int)ctx->layers.size());
-    TRY(frontier_inputs(ctx, in, false, &ti));
+    TRY(grad_args(ctx, in, n_terms, &ti));
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    float* tmp = nullptr;
+    int rc = in->mem == GNNB_MEM_HOST ? stage_grad_frontier(ctx, in, &ti, &tmp, st) : GNNB_OK;
+    if (rc == GNNB_OK) rc = score_grad_impl(ctx, ti, in->B, n_terms, term_domain, term_index, term_coeff, term_scores, st);
+    if (tmp) { cudaStreamSynchronize(st); cudaFree(tmp); }
+    return rc;
+}
+
+int gnnb_score_grad(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t n_terms, const int32_t* term_domain, const int32_t* term_index,
+                    const float* term_coeff, float* term_scores, void* stream) {
+    if (!ctx || !in || !term_domain || !term_index || !term_coeff) return fail(ctx, GNNB_ERR_INVALID, "null argument");
+    GnnInputs ti((int)ctx->layers.size());
+    TRY(grad_args(ctx, in, n_terms, &ti));
     for (int i = 0; i < n_terms; ++i)
         if (term_domain[i] < 0 || term_domain[i] >= in->B || term_index[i] < 0 || term_index[i] >= ctx->n_hidden)
             return fail(ctx, GNNB_ERR_INVALID, "term " + std::to_string(i) + " is out of range");
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    const int B = in->B;
-    // host buffers: one temporary device block for the inputs of this call (this entry is not the hot path)
+    // the terms in, their scores out: one temporary device block [domain | index | coeff | scores] (this entry is not the hot path)
+    const size_t nt = (size_t)n_terms;
+    int32_t* d_terms = nullptr;
+    CU(cudaMalloc(&d_terms, 4 * nt * sizeof(int32_t)));
+    float* d_coeff = reinterpret_cast<float*>(d_terms + 2 * nt);
+    float* d_scores = d_coeff + nt;
     float* tmp = nullptr;
-    if (in->mem == GNNB_MEM_HOST) {
-        size_t total = 0;
-        walk_inputs(*in, ti, ctx->n, [&](const float*, const float*&, int64_t per) { total += align4((size_t)B * per); });
-        CU(cudaMalloc(&tmp, total * sizeof(float)));
-        float* dst = tmp;
-        walk_inputs(*in, ti, ctx->n, [&](const float* src, const float*& slot, int64_t per) {
-            cudaMemcpyAsync(dst, src, (size_t)B * per * sizeof(float), cudaMemcpyHostToDevice, st);
-            slot = dst;
-            dst += align4((size_t)B * per);
-        });
+    cudaError_t e = cudaMemcpyAsync(d_terms, term_domain, nt * sizeof(int32_t), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_terms + nt, term_index, nt * sizeof(int32_t), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_coeff, term_coeff, nt * sizeof(float), cudaMemcpyHostToDevice, st);
+    int rc = e == cudaSuccess ? GNNB_OK : fail(ctx, GNNB_ERR_CUDA, std::string("copying the terms: ") + cudaGetErrorString(e));
+    if (rc == GNNB_OK && in->mem == GNNB_MEM_HOST) rc = stage_grad_frontier(ctx, in, &ti, &tmp, st);
+    if (rc == GNNB_OK) rc = score_grad_impl(ctx, ti, in->B, n_terms, d_terms, d_terms + nt, d_coeff, d_scores, st);
+    if (rc == GNNB_OK && term_scores) {
+        e = cudaMemcpyAsync(term_scores, d_scores, nt * sizeof(float), cudaMemcpyDeviceToHost, st);
+        if (e != cudaSuccess) rc = fail(ctx, GNNB_ERR_CUDA, std::string("copying the term scores: ") + cudaGetErrorString(e));
     }
-    // optimizer.zero_grad() (graph_score_online.py:73), then loss.backward()
-    cudaMemsetAsync(ctx->d_train + ctx->n_params, 0, (size_t)ctx->n_params * sizeof(float), st);
-    std::string err;
-    const int rc = train_backward(ctx->gp, train_params(ctx), ctx->layers, ctx->n, ctx->hidden_off, ti, B, n_terms, term_domain, term_index,
-                                  term_coeff, term_scores, &ctx->train_ws, &ctx->train_ws_cap, st, &ctx->launches, &err);
-    if (tmp) { cudaStreamSynchronize(st); cudaFree(tmp); }
-    if (rc != GNNB_OK) return fail(ctx, rc, err);
-    return GNNB_OK;
+    e = cudaStreamSynchronize(st);          // returns after the gradients are complete
+    if (rc == GNNB_OK && e != cudaSuccess) rc = fail(ctx, GNNB_ERR_CUDA, std::string("gradient pass: ") + cudaGetErrorString(e));
+    if (tmp) cudaFree(tmp);
+    cudaFree(d_terms);
+    return rc;
 }
 
 int gnnb_get_gradients(gnnb_ctx* ctx, float* const* tensors, const int64_t* numels, int n_tensors) {

@@ -327,23 +327,36 @@ __global__ void k_add(float* __restrict__ dst, const float* __restrict__ src, in
 }
 
 // One block of 64 threads per loss term: score = fscore(relu(fnode(mu_row))) (graph_conv.py:448-449) and its backward with
-// upstream gradient coeff.  mu_rows[t] points at the 64 channels of the term's node after the last backward sweep.
+// upstream gradient coeff.  A term is this wave's when its domain is valid and sits at list position row0 .. row0 + rows - 1
+// (row_of); other terms (inactive, out of range, another wave's) return at once, and their score stays as it is.  The row of
+// the term's node after the last backward sweep is found from the per-layer table (flat index -> layer, node).
 struct ScoreTermArgs {
-    const float* const* mu_rows;   // [n_terms] device pointers
-    float* const* dmu_rows;        // [n_terms] where d loss / d mu_row is accumulated
-    const float* coeff;            // [n_terms]
+    const int32_t *domain, *index;  // [n_terms] the caller's terms
+    const float* coeff;             // [n_terms]
+    const int32_t* row_of;          // [B] position of a named subdomain in the list of named subdomains
+    int B, n_hidden, row0, rows;
+    const TermLayer* layers;        // [L] hidden layers k = 1..L
+    int L;
     const float *w_fnode, *b_fnode, *w_fscore, *b_fscore;      // nn.Linear layouts
     float *dW_fnode, *db_fnode, *dW_fscore, *db_fscore;
-    float* scores;                 // [n_terms]
+    float* scores;                  // [n_terms]
 };
 __global__ void __launch_bounds__(64) k_score_terms(ScoreTermArgs a) {
     __shared__ float x[P], dh[P];
     __shared__ float red[2];
     const int t = blockIdx.x, c = threadIdx.x;
-    x[c] = a.mu_rows[t][c];
+    const int d = a.domain[t], flat = a.index[t];
+    if (d < 0 || d >= a.B || flat < 0 || flat >= a.n_hidden) return;
+    const int r = a.row_of[d] - a.row0;
+    if (r < 0 || r >= a.rows) return;
+    int k = 0;
+    while (k + 1 < a.L && flat >= a.layers[k + 1].off) ++k;
+    const TermLayer lay = a.layers[k];
+    const int64_t row = ((int64_t)r * lay.n + (flat - lay.off)) * P;
+    x[c] = lay.mu[row + c];
     __syncthreads();
     float z = a.b_fnode[c];
-    for (int k = 0; k < P; ++k) z = fmaf(x[k], a.w_fnode[c * P + k], z);
+    for (int k2 = 0; k2 < P; ++k2) z = fmaf(x[k2], a.w_fnode[c * P + k2], z);
     const float h = relu_keep_nan(z);
     float part = h * a.w_fscore[c];
 #pragma unroll
@@ -356,14 +369,56 @@ __global__ void __launch_bounds__(64) k_score_terms(ScoreTermArgs a) {
         atomicAdd(a.db_fscore, g);
     }
     atomicAdd(a.dW_fscore + c, g * h);
-    const float d = (z > 0.f) ? g * a.w_fscore[c] : 0.f;
-    dh[c] = d;
-    atomicAdd(a.db_fnode + c, d);
-    for (int k = 0; k < P; ++k) atomicAdd(a.dW_fnode + c * P + k, d * x[k]);
+    const float dd = (z > 0.f) ? g * a.w_fscore[c] : 0.f;
+    dh[c] = dd;
+    atomicAdd(a.db_fnode + c, dd);
+    for (int k2 = 0; k2 < P; ++k2) atomicAdd(a.dW_fnode + c * P + k2, dd * x[k2]);
     __syncthreads();
     float dm = 0.f;
     for (int n = 0; n < P; ++n) dm = fmaf(dh[n], a.w_fnode[n * P + c], dm);
-    atomicAdd(a.dmu_rows[t] + c, dm);
+    atomicAdd(lay.dmu + row + c, dm);
+}
+
+// Terms -> named subdomains.  k_name_terms: every term's score is NaN until its wave writes it; an active term (domain >= 0)
+// flags its domain, or counts as bad when its domain or index is out of range.  k_list_named (one block): the flagged domains
+// in ascending order -> list, their positions -> row_of, the count -> cnt[0].  cnt = [named, bad].
+__global__ void k_name_terms(const int32_t* __restrict__ domain, const int32_t* __restrict__ index, int n_terms, int B, int n_hidden,
+                             float* __restrict__ scores, int32_t* __restrict__ cnt, int32_t* __restrict__ flag) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_terms) return;
+    scores[t] = __int_as_float(0x7fc00000);
+    const int d = domain[t], i = index[t];
+    if (d < 0) return;
+    if (d >= B || i < 0 || i >= n_hidden) { atomicAdd(cnt + 1, 1); return; }
+    flag[d] = 1;
+}
+
+constexpr int LIST_TH = 1024;
+__global__ void __launch_bounds__(LIST_TH) k_list_named(const int32_t* __restrict__ flag, int B, int32_t* __restrict__ list,
+                                                        int32_t* __restrict__ row_of, int32_t* __restrict__ cnt) {
+    __shared__ int warp_sum[LIST_TH / 32];
+    __shared__ int base;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    if (threadIdx.x == 0) base = 0;
+    __syncthreads();
+    for (int j0 = 0; j0 < B; j0 += LIST_TH) {
+        const int j = j0 + threadIdx.x;
+        const int v = (j < B && flag[j]) ? 1 : 0;
+        const unsigned bal = __ballot_sync(0xffffffffu, v);
+        if (lane == 0) warp_sum[wid] = __popc(bal);
+        __syncthreads();
+        int before = base + __popc(bal & ((1u << lane) - 1u));
+        for (int w = 0; w < wid; ++w) before += warp_sum[w];
+        if (v) { list[before] = j; row_of[j] = before; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            int s = 0;
+            for (int w = 0; w < LIST_TH / 32; ++w) s += warp_sum[w];
+            base += s;
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) cnt[0] = base;
 }
 
 // torch.optim.Adam (amsgrad = False, maximize = False): weight decay is added to the gradient, moments are bias-corrected
@@ -417,6 +472,50 @@ struct Ctx {      // launch helpers bound to one call
     void zero(float* p, int64_t numel) const { cudaMemsetAsync(p, 0, (size_t)numel * sizeof(float), st); }
 };
 
+// Offsets (floats) of a wave's activation tape and gradient temporaries in the arena, laid out for waves of up to Bcap
+// subdomains; a smaller wave uses the first rows of each array.
+struct Tape {
+    struct Layer { size_t rs, featf, featb, h1, rlxf, g1, g2, s1, g3, rlxb, drlxf, drlxb; std::vector<size_t> nbF, h3F, eF, h4F, nbB, h3B, eB, h4B; };
+    std::vector<Layer> lt;
+    size_t o_f3, o_f2, o_f4, o_e1, o_i1, o_i2, o_dout, o_dsm, o_bufA, o_bufB, o_bufC, o_bufD, o_tab;
+    std::vector<size_t> o_nb0, o_i3, o_o1, o_nbo, o_o2, o_mu, o_dF, o_dB;
+    size_t total = 0;
+
+    Tape(const std::vector<int>& n, int T, int Bcap) {
+        const int L = (int)n.size() - 2;
+        auto R = [&](int k) { return (int64_t)Bcap * n[k]; };
+        auto take = [&](int64_t elems) { size_t o = total; total += ((size_t)elems + 63) & ~size_t(63); return o; };
+        int64_t rmax = 0;
+        for (int k = 0; k <= L; ++k) rmax = R(k) > rmax ? R(k) : rmax;
+        lt.resize(L + 1);
+        for (int k = 1; k <= L; ++k) {
+            Layer& q = lt[k];
+            const int64_t r = R(k);
+            q.rs = take(6 * r); q.featf = take(7 * r); q.featb = take(7 * r);
+            q.h1 = take(r * P); q.rlxf = take(r * P); q.g1 = take(r * P); q.g2 = take(r * P); q.s1 = take(r * P); q.g3 = take(r * P);
+            q.rlxb = take(r * P); q.drlxf = take(r * P); q.drlxb = take(r * P);
+            for (int t = 0; t < T; ++t) {
+                q.nbF.push_back(take(r * P)); q.h3F.push_back(take(r * P)); q.eF.push_back(take(r * P)); q.h4F.push_back(take(r * P));
+                q.nbB.push_back(take(r * P)); q.h3B.push_back(take(r * P)); q.eB.push_back(take(r * P)); q.h4B.push_back(take(r * P));
+            }
+        }
+        const int64_t r0n = R(0);
+        o_f3 = take(r0n * 3); o_f2 = take(r0n * 2); o_f4 = take((int64_t)Bcap * 4);
+        o_e1 = take(r0n * P); o_i1 = take(r0n * P); o_i2 = take(r0n * P);
+        o_nb0.assign(T, 0); o_i3.assign(T, 0); o_o1.assign(T, 0); o_nbo.assign(T, 0); o_o2.assign(T, 0);
+        for (int t = 0; t < T; ++t) {
+            if (t < T - 1) { o_nb0[t] = take(r0n * P); o_i3[t] = take(r0n * P); }
+            o_o1[t] = take((int64_t)Bcap * P); o_nbo[t] = take((int64_t)Bcap * P); o_o2[t] = take((int64_t)Bcap * P);
+        }
+        o_mu.assign(L + 2, 0); o_dF.assign(L + 1, 0); o_dB.assign(L + 1, 0);
+        for (int k = 0; k <= L; ++k) { o_mu[k] = take(R(k) * P); o_dF[k] = take(R(k) * P); o_dB[k] = take(R(k) * P); }
+        o_mu[L + 1] = take((int64_t)Bcap * P);
+        o_dout = take((int64_t)Bcap * P); o_dsm = take(4 * (int64_t)Bcap * P);
+        o_bufA = take(rmax * P); o_bufB = take(rmax * P); o_bufC = take(rmax * P); o_bufD = take(rmax * P);
+        o_tab = take((int64_t)((L * sizeof(TermLayer) + sizeof(float) - 1) / sizeof(float)));
+    }
+};
+
 }  // namespace
 
 int train_init() {
@@ -424,54 +523,29 @@ int train_init() {
     return (int)e;
 }
 
-int train_backward(const GnnParams& g, const TrainParams& tp, const std::vector<LayerDev>& layers, const std::vector<int>& n,
-                   const std::vector<int>& hidden_off, const GnnInputs& in, int B, int n_terms, const int32_t* term_domain,
-                   const int32_t* term_index, const float* term_coeff, float* term_scores_host, float** arena, size_t* arena_cap,
-                   cudaStream_t st, int64_t* launches, std::string* err) {
+size_t train_tape_floats(const std::vector<int>& n, int T, int Bcap) { return Tape(n, T, Bcap).total; }
+
+void name_terms(const int32_t* domain, const int32_t* index, int n_terms, int B, int n_hidden, float* scores, int32_t* cnt,
+                int32_t* flag, int32_t* list, int32_t* row_of, cudaStream_t st, int64_t* launches) {
+    k_name_terms<<<blocks_for(n_terms, 256), 256, 0, st>>>(domain, index, n_terms, B, n_hidden, scores, cnt, flag);
+    k_list_named<<<1, LIST_TH, 0, st>>>(flag, B, list, row_of, cnt);
+    *launches += 2;
+}
+
+int train_wave(const GnnParams& g, const TrainParams& tp, const std::vector<LayerDev>& layers, const std::vector<int>& n,
+               const std::vector<int>& hidden_off, const GnnInputs& in, int Bcap, int B, const WaveTerms& wt, float* arena,
+               cudaStream_t st, int64_t* launches) {
     const int L = (int)layers.size(), T = g.T;
     auto R = [&](int k) { return (int64_t)B * n[k]; };
-    int64_t rmax = 0;
-    for (int k = 0; k <= L; ++k) rmax = R(k) > rmax ? R(k) : rmax;
-
-    // ---- arena ----
-    size_t total = 0;
-    auto take = [&](int64_t elems) { size_t o = total; total += ((size_t)elems + 63) & ~size_t(63); return o; };
-    struct LayerTape { size_t rs, featf, featb, h1, rlxf, g1, g2, s1, g3, rlxb, drlxf, drlxb; std::vector<size_t> nbF, h3F, eF, h4F, nbB, h3B, eB, h4B; };
-    std::vector<LayerTape> lt(L + 1);
-    for (int k = 1; k <= L; ++k) {
-        LayerTape& q = lt[k];
-        const int64_t r = R(k);
-        q.rs = take(6 * r); q.featf = take(7 * r); q.featb = take(7 * r);
-        q.h1 = take(r * P); q.rlxf = take(r * P); q.g1 = take(r * P); q.g2 = take(r * P); q.s1 = take(r * P); q.g3 = take(r * P);
-        q.rlxb = take(r * P); q.drlxf = take(r * P); q.drlxb = take(r * P);
-        for (int t = 0; t < T; ++t) {
-            q.nbF.push_back(take(r * P)); q.h3F.push_back(take(r * P)); q.eF.push_back(take(r * P)); q.h4F.push_back(take(r * P));
-            q.nbB.push_back(take(r * P)); q.h3B.push_back(take(r * P)); q.eB.push_back(take(r * P)); q.h4B.push_back(take(r * P));
-        }
-    }
+    const Tape tz(n, T, Bcap);
+    using LayerTape = Tape::Layer;
+    const std::vector<LayerTape>& lt = tz.lt;
+    const size_t o_f3 = tz.o_f3, o_f2 = tz.o_f2, o_f4 = tz.o_f4, o_e1 = tz.o_e1, o_i1 = tz.o_i1, o_i2 = tz.o_i2;
+    const size_t o_dout = tz.o_dout, o_dsm = tz.o_dsm;
+    const std::vector<size_t>&o_nb0 = tz.o_nb0, &o_i3 = tz.o_i3, &o_o1 = tz.o_o1, &o_nbo = tz.o_nbo, &o_o2 = tz.o_o2;
+    const std::vector<size_t>&o_mu = tz.o_mu, &o_dF = tz.o_dF, &o_dB = tz.o_dB;
     const int64_t r0n = R(0);
-    const size_t o_f3 = take(r0n * 3), o_f2 = take(r0n * 2), o_f4 = take((int64_t)B * 4);
-    const size_t o_e1 = take(r0n * P), o_i1 = take(r0n * P), o_i2 = take(r0n * P);
-    std::vector<size_t> o_nb0(T), o_i3(T), o_o1(T), o_nbo(T), o_o2(T);
-    for (int t = 0; t < T; ++t) {
-        if (t < T - 1) { o_nb0[t] = take(r0n * P); o_i3[t] = take(r0n * P); }
-        o_o1[t] = take((int64_t)B * P); o_nbo[t] = take((int64_t)B * P); o_o2[t] = take((int64_t)B * P);
-    }
-    std::vector<size_t> o_mu(L + 2), o_dF(L + 1), o_dB(L + 1);
-    for (int k = 0; k <= L; ++k) { o_mu[k] = take(R(k) * P); o_dF[k] = take(R(k) * P); o_dB[k] = take(R(k) * P); }
-    o_mu[L + 1] = take((int64_t)B * P);
-    const size_t o_dout = take((int64_t)B * P), o_dsm = take(4 * (int64_t)B * P);
-    const size_t o_bufA = take(rmax * P), o_bufB = take(rmax * P), o_bufC = take(rmax * P), o_bufD = take(rmax * P);
-    const size_t o_tsc = take(n_terms), o_tco = take(n_terms), o_tptr = take(4 * (int64_t)n_terms + 8);
-    cudaError_t ce = cudaSuccess;
-    if (*arena_cap < total) {           // the tape arena lives in the context and only grows
-        if (*arena) { cudaStreamSynchronize(st); cudaFree(*arena); }
-        *arena = nullptr; *arena_cap = 0;
-        ce = cudaMalloc(arena, total * sizeof(float));
-        if (ce != cudaSuccess) { *err = std::string("training workspace: ") + cudaGetErrorString(ce); return GNNB_ERR_CUDA; }
-        *arena_cap = total;
-    }
-    float* base = *arena;
+    float* base = arena;
     auto Pp = [&](size_t off) { return base + off; };
     Ctx c{g, tp, st, launches};
 
@@ -539,34 +613,23 @@ int train_backward(const GnnParams& g, const TrainParams& tp, const std::vector<
 
     // ---- backward ----
     for (int k = 1; k <= L; ++k) c.zero(Pp(o_dB[k]), R(k) * P);
-    {   // score head on the rows the loss names
-        std::vector<const float*> mu_rows(n_terms);
-        std::vector<float*> dmu_rows(n_terms);
-        for (int i = 0; i < n_terms; ++i) {
-            const int b = term_domain[i], flat = term_index[i];
-            int k = 1;
-            while (k < L && flat >= hidden_off[k + 1]) ++k;
-            const int64_t row = (int64_t)b * n[k] + (flat - hidden_off[k]);
-            mu_rows[i] = Pp(o_mu[k]) + row * P;
-            dmu_rows[i] = Pp(o_dB[k]) + row * P;
-        }
-        float* d_ptrs = Pp(o_tptr);
-        cudaMemcpyAsync(d_ptrs, mu_rows.data(), n_terms * sizeof(float*), cudaMemcpyHostToDevice, st);
-        cudaMemcpyAsync(reinterpret_cast<float**>(d_ptrs) + n_terms, dmu_rows.data(), n_terms * sizeof(float*), cudaMemcpyHostToDevice, st);
-        cudaMemcpyAsync(Pp(o_tco), term_coeff, n_terms * sizeof(float), cudaMemcpyHostToDevice, st);
-        cudaStreamSynchronize(st);          // the pageable sources above are locals
+    {   // score head on the rows the loss names; the layer table points into this arena (a stream-ordered copy from pageable
+        // memory returns after the source has been read)
+        std::vector<TermLayer> tab(L);
+        for (int k = 1; k <= L; ++k) tab[k - 1] = TermLayer{Pp(o_mu[k]), Pp(o_dB[k]), hidden_off[k], n[k]};
+        TermLayer* d_tab = reinterpret_cast<TermLayer*>(Pp(tz.o_tab));
+        cudaMemcpyAsync(d_tab, tab.data(), L * sizeof(TermLayer), cudaMemcpyHostToDevice, st);
         ScoreTermArgs a{};
-        a.mu_rows = reinterpret_cast<const float* const*>(d_ptrs);
-        a.dmu_rows = reinterpret_cast<float* const*>(reinterpret_cast<float**>(d_ptrs) + n_terms);
-        a.coeff = Pp(o_tco);
+        a.domain = wt.domain; a.index = wt.index; a.coeff = wt.coeff; a.row_of = wt.row_of;
+        a.B = wt.B; a.n_hidden = wt.n_hidden; a.row0 = wt.row0; a.rows = B;
+        a.layers = d_tab; a.L = L;
         a.w_fnode = tp.w[FNODE]; a.b_fnode = tp.b[FNODE]; a.w_fscore = tp.w[FSCORE]; a.b_fscore = tp.b[FSCORE];
         a.dW_fnode = tp.dw[FNODE]; a.db_fnode = tp.db[FNODE]; a.dW_fscore = tp.dw[FSCORE]; a.db_fscore = tp.db[FSCORE];
-        a.scores = Pp(o_tsc);
-        k_score_terms<<<n_terms, 64, 0, st>>>(a);
+        a.scores = wt.scores;
+        k_score_terms<<<wt.n_terms, 64, 0, st>>>(a);
         ++*launches;
-        if (term_scores_host) cudaMemcpyAsync(term_scores_host, Pp(o_tsc), n_terms * sizeof(float), cudaMemcpyDeviceToHost, st);
     }
-    float *bufA = Pp(o_bufA), *bufB = Pp(o_bufB), *bufC = Pp(o_bufC), *bufD = Pp(o_bufD);
+    float *bufA = Pp(tz.o_bufA), *bufB = Pp(tz.o_bufB), *bufC = Pp(tz.o_bufC), *bufD = Pp(tz.o_bufD);
     for (int t = T - 1; t >= 0; --t) {
         if (t < T - 1) {
             // input-layer update of round t produced the mu[0] that round t + 1 read: its gradient is dF[0] (graph_conv.py:360-385)
@@ -638,10 +701,7 @@ int train_backward(const GnnParams& g, const TrainParams& tp, const std::vector<
         c.bwd(BC1_1, {{{Pp(q.g1), nullptr, P}, bufB, false}}, bufA, Pp(q.g2), nullptr, r);
         c.bwd(BC1, {{{Pp(q.featb), nullptr, 7}, nullptr, false}}, bufB, Pp(q.g1), nullptr, r);
     }
-    ce = cudaStreamSynchronize(st);
-    if (ce == cudaSuccess) ce = cudaGetLastError();
-    if (ce != cudaSuccess) { *err = std::string("training pass: ") + cudaGetErrorString(ce); return GNNB_ERR_CUDA; }
-    return GNNB_OK;
+    return (int)cudaGetLastError();
 }
 
 void adam_step(float* p, const float* grad, float* m, float* v, int64_t numel, float lr, float b1, float b2, float eps, float wd,

@@ -307,7 +307,12 @@ class Scorer:
     def score_grad(self, fr: Frontier, terms) -> torch.Tensor:
         """Back-propagate ``sum_i coeff_i * score[domain_i][flat_index_i]`` into the gradient buffers of the context
         (zeroed first, like ``optimizer.zero_grad(); loss.backward()``).  ``terms``: iterable of (domain, flat index,
-        coeff).  Returns the terms' scores (fp32, CPU)."""
+        coeff); returns the terms' scores (fp32, CPU).  Or ``terms`` = (domain int32, index int32, coeff float32), three
+        CUDA tensors [n] on this scorer's GPU (``gnnb_score_grad_device``): a term with domain < 0 is inactive, one out of
+        range is skipped and counted (option ``grad_bad_terms``), both score NaN; returns the scores as a CUDA tensor [n],
+        and nothing but the count of named subdomains is read back."""
+        if isinstance(terms, tuple) and len(terms) == 3 and all(isinstance(t, torch.Tensor) for t in terms):
+            return self._score_grad_device(fr, *terms)
         terms = list(terms)
         nt = len(terms)
         dom = (C.c_int32 * nt)(*[int(t[0]) for t in terms])
@@ -320,6 +325,35 @@ class Scorer:
             self._ok(self.lib.gnnb_score_grad(self.h, C.byref(d), nt, dom, idx, coeff, out, C.c_void_p(stream)))
         del keep
         return torch.tensor(list(out), dtype=torch.float32)
+
+    def _score_grad_device(self, fr: Frontier, dom: torch.Tensor, idx: torch.Tensor, coeff: torch.Tensor) -> torch.Tensor:
+        dev = torch.device('cuda', self.device)
+        n = int(dom.numel())
+        for t, dt in ((dom, torch.int32), (idx, torch.int32), (coeff, torch.float32)):
+            if t.device != dev or t.dtype != dt or t.dim() != 1 or t.numel() != n:
+                raise ValueError(f'device terms must be [n] tensors on {dev}: domain / index int32, coeff float32')
+        dom, idx, coeff = dom.contiguous(), idx.contiguous(), coeff.contiguous()
+        out = torch.empty(n, dtype=torch.float32, device=dev)
+        d, keep = self._frontier_desc(fr)
+        ip = lambda t: C.cast(t.data_ptr(), C.POINTER(C.c_int32))
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            self._ok(self.lib.gnnb_score_grad_device(self.h, C.byref(d), n, ip(dom), ip(idx), _lib.fptr(coeff), _lib.fptr(out),
+                                                     C.c_void_p(stream)))
+        del keep
+        return out
+
+    def copy_weights_to(self, tensors) -> None:
+        """Copy the parameters the context scores with into 52 contiguous fp32 tensors in state_dict order, on the CPU or on
+        this scorer's GPU (device to device, no host round trip)."""
+        tensors = list(tensors)
+        for t in tensors:
+            if t.dtype != torch.float32 or not t.is_contiguous() or (t.is_cuda and t.device.index != self.device):
+                raise ValueError('copy_weights_to needs contiguous fp32 tensors on the CPU or on the scorer\'s GPU')
+        ptrs, keep = _lib.fptr_array(tensors)
+        numels = (C.c_int64 * len(tensors))(*[t.numel() for t in tensors])
+        self._ok(self.lib.gnnb_get_gnn_weights(self.h, ptrs, numels, len(tensors)))
+        del keep
 
     def _download(self, fn) -> Dict[str, torch.Tensor]:
         shapes = []

@@ -12,7 +12,7 @@ from typing import List, Optional
 import torch
 from torch import nn
 
-from .engine import Scorer
+from .engine import STATE_DICT_KEYS, Scorer
 from .frontier import Frontier
 
 
@@ -90,11 +90,17 @@ class GraphNet(nn.Module):
 
     def adopt_weights(self, sc: Scorer) -> None:
         """After a device-side optimiser step: copy the context's parameters into this module (so ``state_dict()`` and
-        checkpoints follow the fine-tuning) without triggering a re-upload."""
-        new = sc.weights()
+        checkpoints follow the fine-tuning) without triggering a re-upload.  Parameters on the scorer's GPU are written
+        device to device; others through the host."""
+        sd = self.state_dict()
+        ts = [sd[k] for k in STATE_DICT_KEYS]
         with torch.no_grad():
-            for k, q in self.state_dict().items():
-                q.copy_(new[k])
+            if all(t.is_cuda and t.device.index == sc.device and t.dtype == torch.float32 and t.is_contiguous() for t in ts):
+                sc.copy_weights_to(ts)
+            else:
+                new = sc.weights()
+                for k, q in sd.items():
+                    q.copy_(new[k])
         sc._gnn_key = tuple((q.data_ptr(), q._version) for q in self.parameters())
 
     def score_frontier(self, fr: Frontier, return_scores: bool = True):

@@ -124,9 +124,12 @@ int gnnb_set_network(gnnb_ctx* ctx, const gnnb_layer_desc* layers, int n_layers,
  * device -> host copy and one synchronise of `stream` per call, also with DEVICE buffers (no extra launch or allocation).
  * The NaN count is reset before the fp32 pass, so GNNB_ERR_NAN (returned for HOST calls, through gnnb_check for DEVICE calls)
  * then reports only NaN that exact fp32 gives too.  The option does nothing in SIMT mode; snapshots keep the tensor-core pass.
+ * "grad_chunk" (>= 0, default 0): subdomains per wave of gnnb_score_grad(_device); 0 = the most whose activation tape fits
+ * 4 GiB.
  * gnnb_get_option also reads these, "rescored" (subdomains the last scoring call scored again), and "n_hidden" (hidden ReLUs of
  * the network), "workspace_domains" (subdomains the
- * workspace holds) and "plan_density_pct_f<k>" / "plan_density_pct_b<k>" (percentage of the MACs issued by forward /
+ * workspace holds), "grad_workspace_domains" (subdomains per wave of the last gnnb_score_grad(_device): the tape arena holds
+ * at least that many; 0 when no term was active), "grad_bad_terms" (out-of-range terms of the last gnnb_score_grad_device) and "plan_density_pct_f<k>" / "plan_density_pct_b<k>" (percentage of the MACs issued by forward /
  * backward propagation plan k that are useful); it returns -1 for an unknown key. */
 int gnnb_set_option(gnnb_ctx* ctx, const char* key, int64_t value);
 int64_t gnnb_get_option(gnnb_ctx* ctx, const char* key);
@@ -200,13 +203,30 @@ int gnnb_babsr(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t sparsest_layer, f
  *     loss = sum_i term_coeff[i] * score[term_domain[i]][term_index[i]]
  * (term_index = flat index into the concatenated hidden layers) into d loss / d parameter for all 52 tensors.  The
  * reference's loss is the two terms (+1, argmax index), (-1, index of the KW decision); `improvement` is a constant and
- * has no gradient.  term_* are HOST arrays; term_scores [n_terms] (HOST, may be NULL) receives the terms' fp32 scores.
- * Frontier pointers live in `in->mem`; `in->mask` is not read.  Returns after the gradients are complete. */
+ * has no gradient.  term_* are HOST arrays, checked on the host (a term out of range fails with GNNB_ERR_INVALID);
+ * term_scores [n_terms] (HOST, may be NULL) receives the terms' fp32 scores.  Frontier pointers live in `in->mem`; `in->mask`
+ * is not read.  Copies the terms in and runs gnnb_score_grad_device; returns after the gradients are complete. */
 int gnnb_score_grad(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t n_terms, const int32_t* term_domain,
                     const int32_t* term_index, const float* term_coeff, float* term_scores, void* stream);
 
+/* The same gradient with the terms on the device, for a branch-and-bound loop whose terms are computed on the GPU.
+ * term_domain, term_index, term_coeff and term_scores [n_terms] are DEVICE arrays; frontier pointers live in `in->mem`.
+ *   - A term with term_domain < 0 is inactive: it adds nothing, so a caller can pass a fixed-size list without reading a count.
+ *   - A term with term_domain >= B or term_index outside [0, n_hidden) is never dereferenced: it is treated as inactive and
+ *     counted, gnnb_get_option("grad_bad_terms").
+ *   - term_scores of an inactive or out-of-range term is NaN.
+ * Only the subdomains that carry an active term are run: they are listed on the device, and their count is read back (one
+ * 8-byte device -> host copy and one synchronise of `stream`).  Forward with tape and backward then run over that list in
+ * waves of at most option "grad_chunk" subdomains, each gathered into staging rows first; the gradients of the waves add up.
+ * Everything after the read-back is only enqueued on `stream` (HOST frontiers: the call returns after the pass).  Argument
+ * errors (null pointers, B < 1, n_terms < 1, weights or network not set, a network with zero-tap positions) are reported
+ * before anything is enqueued, as in gnnb_score_grad. */
+int gnnb_score_grad_device(gnnb_ctx* ctx, const gnnb_frontier* in, int32_t n_terms, const int32_t* term_domain,
+                           const int32_t* term_index, const float* term_coeff, float* term_scores, void* stream);
+
 /* Copy the gradients of the last gnnb_score_grad (the reference's `p.grad`) / the current parameters (the reference's
- * `model.state_dict()`) into 52 HOST tensors in the order of gnnb_set_gnn_weights. */
+ * `model.state_dict()`) into 52 tensors in the order of gnnb_set_gnn_weights, HOST or DEVICE memory (each pointer's memory
+ * space is taken from its address).  Synchronises the device. */
 int gnnb_get_gradients(gnnb_ctx* ctx, float* const* tensors, const int64_t* numels, int n_tensors);
 int gnnb_get_gnn_weights(gnnb_ctx* ctx, float* const* tensors, const int64_t* numels, int n_tensors);
 
